@@ -19,6 +19,9 @@ N > 1:     ONE C3 problem sharded over the N ranks behind the C ABI (library-own
 ``--impl reference`` times the reference's CPU algorithm for the same call on the host cores: the C++
 restatement in oracle/ (Julia is not installed in this image, so the reference itself cannot run; kind = "port",
 single-threaded because the reference is).
+
+``--dump-outputs DIR`` writes the split vectors the last timed step returned as ``DIR/<name>.npy`` (float64). The
+inputs come from seeded generators, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import gc
@@ -148,6 +151,22 @@ def rooflines(prof, step_ms_total, steps, key):
                     "algorithmic_bytes_per_launch": k["bytes"] / max(k["launches"], 1), "share_of_step": k["ms"] / max(step_ms_total, 1e-9),
                     "note": NOTES.get(nm, "")})
     return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, res):
+    """Writes what a caller of the timed call receives: the split vector ``spl`` of partition_stripe / pack_stripe, or
+    ``Pi_spl`` and ``Phi_spl`` of partition_plaid's (Pi, Phi).  float64 holds every 1-based index exactly."""
+    parts = [("Pi_spl", res[0]), ("Phi_spl", res[1])] if isinstance(res, tuple) else [("spl", res)]
+    arrays = {name: np.asarray(p.spl, dtype=np.float64) for name, p in parts}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def time_workload(cp, w, M, extra, steps, warmup, flush_l2, e2e_steps=None, pinned=False):
@@ -281,7 +300,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--configs", default=os.environ.get("CPB_BENCH_CONFIGS", "all"), help="all | none | comma list of C1,C2,C4a,C4b,C5 (N = 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the split vectors of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -307,14 +329,16 @@ def main():
             torch.cuda.set_device(local_rank)
         M, extra = W.make(SCALE, have_cuda)
         release_memory()
-        steps = max(1, min(args.steps, 3))
+        steps = args.steps
         t0 = time.perf_counter()
         secs = [0.0, 0.0]
         for _ in range(steps):
-            W.call(ref, M, extra)
+            res = W.call(ref, M, extra)
             secs[0] += ref.last_seconds[0]
             secs[1] += ref.last_seconds[1]
         per = (time.perf_counter() - t0) / steps
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res)
         v = 1.0 / per
         line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": 0,
                 "ms_per_step": per * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "int64", "data": "synthetic",
@@ -371,6 +395,8 @@ def main():
     sampler.active.clear()
     dev_ms, e2e_ms = t["dev_ms"], float(np.sum(t["e2e_samples"]))
     assert W.same(t["res"], t["res_e2e"])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, t["res"])
     value = args.steps / (dev_ms / 1e3)
     e2e_value = args.steps / (e2e_ms / 1e3)
     roofs = rooflines(t["prof"], dev_ms, args.steps, HEADLINE)
@@ -404,7 +430,7 @@ def main():
             cache[ck] = w.make(SCALE, True)
             release_memory()
         Mk, ek = cache[ck]
-        entry = {"config": key, **config_entry(cp, ref, key, Mk, ek, 3, flush_l2)}
+        entry = {"config": key, **config_entry(cp, ref, key, Mk, ek, args.steps, flush_l2)}
         if key == "C2":
             queries = query_throughput(cp, ref, Mk, AFF, rank)
             entry["oracle_queries"] = queries

@@ -80,8 +80,10 @@ def run_sharded(cp, dist, W, M, extra, args, rank, world, local_rank, barrier, f
     sampler.join(timeout=2)
     if rank != 0:
         return None
-    from bench import rooflines
+    from bench import dump_outputs, rooflines
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     roofs = rooflines(prof, dev_ms, args.steps, "C3")
     value = args.steps / (dev_ms_max / 1e3)
     return {"metric": metric, "value": value, "unit": unit, "n_gpus": world, "steps": args.steps, "warmup": warm,
