@@ -403,10 +403,11 @@ __global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
 // is `prev <= first position of the part`; written `prev < j` below.)
 // The reference streams cch[] = previous column of every nonzero and counts `cch[q] < j` for the
 // current part start j; a part ends where the running cost first exceeds c.  Here one 8-CTA cluster
-// per threshold streams the same link array in super-steps of 8 x 16384 elements: ballots turn
-// `prev < j` into bit masks, a block scan + a DSMEM exchange give the running count at every column
-// boundary inside the tile, and all boundaries of the tile are tested at once.  No dominance index is
-// needed for bisection at all.
+// per threshold streams the same link array in super-steps of register tiles: every lane stores its
+// `prev < j` flags as one byte per group, a block scan gives each CTA's running count, and two st.async
+// exchanges between the cluster's CTAs, completing on mbarriers, give the count at every column
+// boundary inside the tile and the feasible boundaries of the whole cluster; all boundaries of the tile
+// are tested at once.  No dominance index is needed for bisection at all.
 // ------------------------------------------------------------------------------------------------
 static constexpr int SP_THREADS = 1024;
 #ifndef CPB_SP_VEC
@@ -418,21 +419,8 @@ static constexpr int SP_NVMAX = SP_VEC * SP_SUB;       // 128-bit loads per thre
 static constexpr int SP_CE = SP_THREADS * SP_VEC * 4;  // 32768 elements per CTA per register tile
 static constexpr int SP_GROUPS = SP_NVMAX * 32;        // 128-element groups per CTA (one warp-wide uint4 load each) at most
 
-// `prev < j` count among the first x elements of this CTA's slice, from the per-group masks
-__device__ __forceinline__ u32 stream_prefix(const u32* s_mask, const u32* s_cum, u32 x) {
-  const u32 g = x >> 7, r = x & 127u;
-  u32 cnt = s_cum[g];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int nl = ((int)r - k + 3) >> 2;  // lanes l with 4 l + k < r
-    const u32 msk = nl >= 32 ? 0xffffffffu : (nl <= 0 ? 0u : ((1u << nl) - 1u));
-    cnt += __popc(s_mask[g * 4 + k] & msk);
-  }
-  return cnt;
-}
-
-// The same count when a group's flags are stored as one byte per lane (bit k of byte l = element 4 l + k of the group; 8 words
-// per group): what k_probe_stream writes since round 2 -- every thread stores the nibble of its own four compares, no
+// `prev < j` count among the first x elements of this CTA's slice, from the per-group flags stored as one byte per lane (bit k
+// of byte l = element 4 l + k of the group; 8 words per group): every thread stores the nibble of its own four compares, no
 // warp vote (VOTE runs on the SM's one address-divergence unit: 1024 votes per super-step were the tile phase's limiter).
 __device__ __forceinline__ u32 stream_prefix_nib(const u32* s_mask, const u32* s_cum, u32 x) {
   const u32 g = x >> 7, r = x & 127u;
@@ -453,7 +441,6 @@ struct DevStream {
   const u32* colq;    // [ceil(Ne / LS_COLQ) + 1] 0-based column of every LS_COLQ-th element (LinkStream::colq)
   const u32* P;       // element offsets of the column boundaries, 1 <= x <= n+1
   const u32* Wt;      // prefix of the pin-like term, 1 <= x <= n+1
-  const u32* chunk_col;  // [ceil(Ne / LS_CHUNK) + 1] column of the first element of every LS_CHUNK-element chunk (ring probes)
   u32 Ne, n;
   int same_w;         // Wt == P
   double cf[4];
@@ -468,7 +455,7 @@ template <class T> __device__ __forceinline__ T stream_cost(const DevStream& s, 
   return C::get(s, 0) + (T)nv * C::get(s, 1) + (T)w * C::get(s, 2) + (T)g * C::get(s, 3);
 }
 
-// ---- cluster exchange / bulk copy primitives (PTX) ----
+// ---- cluster exchange primitives (PTX) ----
 __device__ __forceinline__ u32 smem_addr(const void* p) { return (u32)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ u32 map_peer(u32 addr, u32 rank) {
   u32 r;
@@ -481,9 +468,9 @@ __device__ __forceinline__ void mbar_expect_tx(u32 bar, u32 bytes) {
 }
 // A wait that never completes -- a protocol bug -- traps after ~2 s instead of hanging the GPU, after leaving a record
 // (which wait, where) in a host-mapped buffer that bisect_advance appends to the error message.
-__device__ unsigned long long* g_ring_dbg = nullptr;
-__device__ __noinline__ void ring_wait_failed(u32 tag, u32 a, u32 b, u32 c, u32 d) {
-  unsigned long long* g = g_ring_dbg;
+__device__ unsigned long long* g_probe_dbg = nullptr;
+__device__ __noinline__ void probe_wait_failed(u32 tag, u32 a, u32 b, u32 c, u32 d) {
+  unsigned long long* g = g_probe_dbg;
   if (g) {
     unsigned cr;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(cr));
@@ -502,17 +489,6 @@ __device__ __noinline__ void ring_wait_failed(u32 tag, u32 a, u32 b, u32 c, u32 
   }
   __trap();
 }
-__device__ __forceinline__ void mbar_wait(u32 bar, u32 parity, u32 tag = 0, u32 a = 0, u32 b = 0, u32 c = 0, u32 d = 0) {  // this CTA's bulk copies
-  u32 ok = 0;
-  long long t0 = 0;
-  while (true) {
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n" : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    if (ok) break;
-    const long long t = clock64();
-    if (t0 == 0) t0 = t;
-    else if (t - t0 > 4000000000ll) ring_wait_failed(tag, a, b, c, d);
-  }
-}
 __device__ __forceinline__ void mbar_wait_cluster(u32 bar, u32 parity, u32 tag = 0, u32 a = 0, u32 b = 0, u32 c = 0, u32 d = 0) {  // peers' st.async
   u32 ok = 0;
   long long t0 = 0;
@@ -521,7 +497,7 @@ __device__ __forceinline__ void mbar_wait_cluster(u32 bar, u32 parity, u32 tag =
     if (ok) break;
     const long long t = clock64();
     if (t0 == 0) t0 = t;
-    else if (t - t0 > 4000000000ll) ring_wait_failed(tag, a, b, c, d);
+    else if (t - t0 > 4000000000ll) probe_wait_failed(tag, a, b, c, d);
   }
 }
 __device__ __forceinline__ void st_async_u32(u32 remote_addr, u32 v, u32 remote_bar) {
@@ -530,10 +506,6 @@ __device__ __forceinline__ void st_async_u32(u32 remote_addr, u32 v, u32 remote_
 __device__ __forceinline__ void st_async_v4(u32 remote_addr, u32 a, u32 b, u32 c, u32 d, u32 remote_bar) {
   asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(remote_addr), "r"(a), "r"(b),
                "r"(c), "r"(d), "r"(remote_bar) : "memory");
-}
-__device__ __forceinline__ void bulk_load(u32 dst, const void* src, u32 bytes, u32 bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
 }
 
 #ifdef CPB_PROBE_TIMING
@@ -567,11 +539,10 @@ __device__ __forceinline__ void stream_cols_of(const DevStream& s, bool use1, u3
   c2 = lo2;
 }
 
-// AX: the two exchanges of a super-step as remote st.async stores that complete a transaction count on every peer's
-// mbarrier (no barrier.cluster, no fence in front of it, no L1 invalidation); !AX: DSMEM stores + cluster barriers.
-// CL: CTAs per cluster (8, or 16 = the non-portable size; set by the launch attribute)
-template <class T, bool AX, int CL>
-__global__ void __launch_bounds__(SP_THREADS, 1)
+// The two exchanges of a super-step are remote st.async stores that complete a transaction count on every peer's mbarrier
+// (no barrier.cluster, no fence in front of it, no L1 invalidation).
+template <class T>
+__global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(SP_THREADS, 1)
     k_probe_stream(const __grid_constant__ DevStream s, int K, double eps1, const BisectState* __restrict__ st,
                    int* __restrict__ node_spl, int* __restrict__ node_res, double* __restrict__ node_c,
                    const int* __restrict__ node_ids, int node_base) {
@@ -579,10 +550,9 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
   __shared__ u32 s_cum[SP_GROUPS + 1];
   __shared__ double s_c;
   __shared__ int s_valid;
-  __shared__ u32 s_xa[2][CL];     // per-CTA `prev < j` totals of the tile
-  __shared__ u32 s_xb[2][4][CL];  // per-CTA (feasible boundaries, boundaries, P and Wt at the last feasible one)
-  __shared__ __align__(16) u32 s_xv[2][CL][4];  // the same, one 16-byte record per CTA (AX)
-  __shared__ __align__(8) unsigned long long s_mb[2][2];  // [exchange][super-step parity] (AX)
+  __shared__ u32 s_xa[2][BS_CLUSTER];  // per-CTA `prev < j` totals of the tile
+  __shared__ __align__(16) u32 s_xv[2][BS_CLUSTER][4];  // per CTA (feasible boundaries, boundaries, P and Wt at the last feasible one)
+  __shared__ __align__(8) unsigned long long s_mb[2][2];  // [exchange][super-step parity]
   __shared__ u32 s_pj[2 * SP_THREADS];    // (P, Wt) of every thread's boundary candidate, pass 1 | pass 2
   __shared__ u32 s_w[2 * SP_THREADS];
   __shared__ u32 s_wtot[32];              // per-warp `prev < j` totals of the tile
@@ -590,24 +560,22 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
   cg::cluster_group cluster = cg::this_cluster();
   const unsigned crank = cluster.block_rank();
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int node = node_base + blockIdx.x / CL;
+  const int node = node_base + blockIdx.x / BS_CLUSTER;
   const bool writer = crank == 0 && tid == 0;
   if (tid == 0) {
     s_valid = node_threshold(st, eps1, node_ids[node], &s_c);
     for (int k = 0; k < 8; ++k) s_mask[SP_GROUPS * 8 + k] = 0;
     for (int k = 0; k < 4; ++k) { s_red[0][k] = 0; s_red[1][k] = 0; }
-    if (AX) {
-      for (int x = 0; x < 2; ++x)
-        for (int p = 0; p < 2; ++p) mbar_init(smem_addr(&s_mb[x][p]), 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    for (int x = 0; x < 2; ++x)
+      for (int p = 0; p < 2; ++p) mbar_init(smem_addr(&s_mb[x][p]), 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
   if (!s_valid) {
     if (writer) node_res[node] = 0;
     return;
   }
-  if (AX) cluster.sync();  // every CTA's mbarriers exist before a peer's st.async can reach them
+  cluster.sync();  // every CTA's mbarriers exist before a peer's st.async can reach them
   u32 sstep = 0;
 #ifdef CPB_PROBE_TIMING
   __shared__ unsigned long long s_pt[16];
@@ -640,7 +608,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
     PT(10);
     for (u32 e_tile = e0 & ~3u;;) {  // 16-byte aligned tiles; elements left of e0 are masked out
       const u32 CE = (u32)SP_THREADS * 4u * nv;  // elements of this CTA in this super-step
-      const u32 TE = CE * CL;
+      const u32 TE = CE * BS_CLUSTER;
       const u32 ngroups = nv * 32u;
 #ifdef CPB_PROBE_TIMING
       PT(6);  // between the super-steps (part bookkeeping)
@@ -722,7 +690,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
       __syncthreads();
       PT(1);
       // ---- every warp adds the totals of the warps before it to its own groups' prefixes; warp 0 also forms the CTA
-      //      total.  The cluster barrier below orders these writes for the boundary phase. ----
+      //      total.  The __syncthreads below orders these writes for the boundary phase. ----
       u32 tot_c = 0;
       {
         const u32 t = s_wtot[lane];
@@ -740,13 +708,8 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
       }
       PT(2);
       const u32 xpar = (sstep >> 1) & 1u;
-      if (AX) {
-        if (tid == 0) { mbar_expect_tx(smem_addr(&s_mb[0][ph]), 4u * CL); mbar_expect_tx(smem_addr(&s_mb[1][ph]), 16u * CL); }
-        if (tid < CL) st_async_u32(map_peer(smem_addr(&s_xa[ph][crank]), tid), tot_c, map_peer(smem_addr(&s_mb[0][ph]), tid));
-      } else {
-        if (tid < CL) *cluster.map_shared_rank(&s_xa[ph][crank], tid) = tot_c;
-        cluster.barrier_arrive();  // split barrier: the boundary offsets below are fetched while the totals travel
-      }
+      if (tid == 0) { mbar_expect_tx(smem_addr(&s_mb[0][ph]), 4u * BS_CLUSTER); mbar_expect_tx(smem_addr(&s_mb[1][ph]), 16u * BS_CLUSTER); }
+      if (tid < BS_CLUSTER) st_async_u32(map_peer(smem_addr(&s_xa[ph][crank]), tid), tot_c, map_peer(smem_addr(&s_mb[0][ph]), tid));
       const u32 nb = (jb >= ja) ? jb - ja + 1 : 0;
       // thread t owns the (at most 4) consecutive boundaries [t * per, (t + 1) * per) when the CTA has at most 4096 of
       // them: all loaded up front (one memory latency), before the barrier completes
@@ -761,16 +724,12 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
           pjv[i] = __ldg(s.P + ja + b0 + i);
           wv[i] = s.same_w ? pjv[i] : __ldg(s.Wt + ja + b0 + i);
         }
-      if (AX) {
-        __syncthreads();  // s_cum (every warp added its base) is complete for the boundary phase
-        mbar_wait_cluster(smem_addr(&s_mb[0][ph]), xpar, 5u, sstep, nv, e0, e_tile);
-      } else {
-        cluster.barrier_wait();  // also orders s_cum for the boundary phase
-      }
+      __syncthreads();  // s_cum (every warp added its base) is complete for the boundary phase
+      mbar_wait_cluster(smem_addr(&s_mb[0][ph]), xpar, 5u, sstep, nv, e0, e_tile);
       PT(3);
       u32 base_c = 0, tile_tot = 0;
 #pragma unroll
-      for (int p = 0; p < CL; ++p) {
+      for (int p = 0; p < BS_CLUSTER; ++p) {
         const u32 v = s_xa[ph][p];
         if (p < (int)crank) base_c += v;
         tile_tot += v;
@@ -851,35 +810,17 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
       }
       PT(4);
       u32 feas = 0, nbs = 0;
-      if (AX) {
-        if (tid < CL) st_async_v4(map_peer(smem_addr(&s_xv[ph][crank][0]), tid), cnt, nb, lastp, lastw, map_peer(smem_addr(&s_mb[1][ph]), tid));
-        mbar_wait_cluster(smem_addr(&s_mb[1][ph]), xpar, 6u, sstep, nv, e0, e_tile);
-        PT(5);
+      if (tid < BS_CLUSTER) st_async_v4(map_peer(smem_addr(&s_xv[ph][crank][0]), tid), cnt, nb, lastp, lastw, map_peer(smem_addr(&s_mb[1][ph]), tid));
+      mbar_wait_cluster(smem_addr(&s_mb[1][ph]), xpar, 6u, sstep, nv, e0, e_tile);
+      PT(5);
 #pragma unroll
-        for (int p = 0; p < CL; ++p) {
-          const uint4 q = *reinterpret_cast<const uint4*>(&s_xv[ph][p][0]);
-          feas += q.x;
-          nbs += q.y;
-          if (q.x > 0) { pcur = q.z; wcur = q.w; }  // the last CTA with a feasible boundary wins
-        }
-        PT(7);
-      } else {
-        if (tid < CL) {
-          *cluster.map_shared_rank(&s_xb[ph][0][crank], tid) = cnt;
-          *cluster.map_shared_rank(&s_xb[ph][1][crank], tid) = nb;
-          *cluster.map_shared_rank(&s_xb[ph][2][crank], tid) = lastp;
-          *cluster.map_shared_rank(&s_xb[ph][3][crank], tid) = lastw;
-        }
-        cluster.sync();
-        PT(5);
-#pragma unroll
-        for (int p = 0; p < CL; ++p) {
-          const u32 cp = s_xb[ph][0][p];
-          feas += cp;
-          nbs += s_xb[ph][1][p];
-          if (cp > 0) { pcur = s_xb[ph][2][p]; wcur = s_xb[ph][3][p]; }  // the last CTA with a feasible boundary wins
-        }
+      for (int p = 0; p < BS_CLUSTER; ++p) {
+        const uint4 q = *reinterpret_cast<const uint4*>(&s_xv[ph][p][0]);
+        feas += q.x;
+        nbs += q.y;
+        if (q.x > 0) { pcur = q.z; wcur = q.w; }  // the last CTA with a feasible boundary wins
       }
+      PT(7);
       ++sstep;
       ph ^= 1;
       first = false;
@@ -894,7 +835,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
     {  // size the next part's first tile from this part (+1/8 slack); a miss (second super-step needed) resets
        // the estimate to the full tile, from where it shrinks by one vector load per part at most
       const u32 elems = pcur - e0;
-      const u32 want = (elems + (elems >> 3) + 3u) / ((u32)SP_THREADS * 4u * CL) + 1u;
+      const u32 want = (elems + (elems >> 3) + 3u) / ((u32)SP_THREADS * 4u * BS_CLUSTER) + 1u;
       nv_est = missed ? (u32)SP_NVMAX : max(min(max(want, 2u), (u32)SP_NVMAX), nv_est > 2u ? nv_est - 1u : 2u);
       nv = nv_est;
     }
@@ -925,370 +866,6 @@ __global__ void __launch_bounds__(SP_THREADS, 1)
 #endif
   }
   cluster.sync();
-}
-
-// ------------------------------------------------------------------------------------------------
-// Streaming probe, ring form (kernel "probe_ring").  Same algorithm and results as k_probe_stream; what changes is how
-// the latency chain of a part is built:
-//   * the link array is consumed (almost always) left to right by every threshold, so it is staged AHEAD of the search:
-//     the cluster's 8 CTAs own the 32 KB chunks of the array round-robin (chunk g belongs to CTA g mod 8) and each keeps
-//     its next PR_S chunks in a shared-memory ring filled by 1-D bulk copies (cp.async.bulk + mbarrier complete_tx).
-//     Only the compare `prev <= first position of the part` depends on the part start, so a part's tile is already on
-//     chip when its start becomes known.  (A part can end far behind the window that detected its end -- a giant column
-//     in between -- and the next part then starts behind the ring: the ring is drained and refilled from there.)
-//   * warp specialisation: warps 0..30 turn chunks into bit masks; warp 31 owns everything asynchronous -- it arms the
-//     exchange barriers, keeps the ring full, resolves the chunks' column ranges, waits for the peers' chunk totals and
-//     turns them into per-chunk bases -- off the consumers' instruction stream (an mbarrier / bulk-copy instruction
-//     costs ~150 cycles on the issuing thread: measured, profiles/r02_ring.md);
-//   * the two exchanges of a super-step (per-chunk `prev < j` totals; per-CTA feasible-boundary counts) are remote
-//     st.async stores that carry their payload into every peer's shared memory and complete a transaction count on the
-//     peer's mbarrier -- no barrier.cluster, no fence in front of it, no L1 invalidation; each store is issued by a
-//     different warp (the per-lane cost of remote stores is serial inside one instruction);
-//   * chunk boundaries (first / last column of a chunk) come from a per-chunk table built once with the links; the
-//     crossing is found by 1024-way search rounds over the CTA's boundary candidates.
-// A super-step covers the chunks [g_win, g_win + 8 W) (W <= PR_WMAX per CTA, sized from the previous part).
-// ------------------------------------------------------------------------------------------------
-static constexpr int PR_THREADS = 1024;
-static constexpr u32 PR_C = LS_CHUNK;  // elements per chunk (32 KB)
-static constexpr int PR_S = 6;         // ring slots per CTA (192 KB)
-static constexpr int PR_WMAX = 3;      // chunks per CTA per super-step
-static constexpr int PR_G = 64;        // 128-element groups per chunk
-static constexpr int PR_CW = 31;       // consumer warps; warp 31 is the producer / coordinator
-static constexpr size_t PR_RING_BYTES = (size_t)PR_S * PR_C * sizeof(u32);
-static_assert(PR_C == 8192, "PR_G groups of 128 elements per chunk");
-
-#ifdef CPB_PROBE_TIMING
-__device__ unsigned long long g_ring_t[16];
-__device__ unsigned long long g_ring_n[8];  // super-steps, parts, search rounds, rewinds, empty steps, sum of W
-#define RT(i) do { if (node == 0 && crank == 0 && tid == 0) { unsigned long long _t = clock64(); g_ring_t[i] += _t - rt_last; rt_last = _t; } } while (0)
-#define RN(i, v) do { if (node == 0 && crank == 0 && tid == 0) g_ring_n[i] += (v); } while (0)
-#else
-#define RT(i) do {} while (0)
-#define RN(i, v) do {} while (0)
-#endif
-
-struct PrShared {
-  alignas(16) u32 mask[PR_WMAX][PR_G + 1][4];  // `prev < j` bit masks of every group; [.][64] = zero sentinel (offset == chunk size)
-  u32 cnt[PR_WMAX][PR_G];                      // set bits per group
-  u32 cum[PR_WMAX][PR_G + 1];                  // exclusive prefix of cnt inside the chunk; [.][64] = chunk total
-  u32 cb[2][PR_WMAX][2];                       // (first boundary, number of boundaries) of this CTA's chunks, per super-step parity
-  u32 base[2][PR_WMAX + 1];                    // `prev < j` elements of the window in front of each of this CTA's chunks; [.][WMAX] = window total
-  alignas(16) u32 x1[2][8 * PR_WMAX];          // exchange 1: chunk totals of the whole window, window order
-  alignas(16) u32 x2[2][8][4];                 // exchange 2: per CTA (feasible boundaries, boundaries, P and Wt at its last feasible one)
-  u32 pj[PR_THREADS];                          // (P, Wt) of the boundary candidates of the current search round
-  u32 w[PR_THREADS];
-  alignas(8) unsigned long long mb_full[PR_S];
-  alignas(8) unsigned long long mb_x1[2];
-  alignas(8) unsigned long long mb_x2[2];
-  double c;
-  int valid;
-};
-
-template <class T>
-__global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(PR_THREADS, 1)
-    k_probe_ring(const __grid_constant__ DevStream s, int K, double eps1, const BisectState* __restrict__ st, int* __restrict__ node_spl,
-                 int* __restrict__ node_res, double* __restrict__ node_c, const int* __restrict__ node_ids, int node_base) {
-  extern __shared__ __align__(128) unsigned char pr_ring_raw[];
-  u32* const ring = reinterpret_cast<u32*>(pr_ring_raw);  // [PR_S][PR_C]
-  __shared__ PrShared sh;
-  cg::cluster_group cluster = cg::this_cluster();
-  const u32 crank = cluster.block_rank();
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const bool producer = warp == PR_CW;
-  const int node = node_base + blockIdx.x / BS_CLUSTER;
-  const bool writer = crank == 0 && tid == 0;
-  if (tid == 0) {
-    sh.valid = node_threshold(st, eps1, node_ids[node], &sh.c);
-    for (int t = 0; t < PR_S; ++t) mbar_init(smem_addr(&sh.mb_full[t]), 1);
-    for (int t = 0; t < 2; ++t) { mbar_init(smem_addr(&sh.mb_x1[t]), 1); mbar_init(smem_addr(&sh.mb_x2[t]), 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (tid < PR_WMAX * 4) sh.mask[tid >> 2][PR_G][tid & 3] = 0;
-  __syncthreads();
-  if (!sh.valid) {  // uniform over the cluster: every CTA derives it from the same state
-    if (writer) node_res[node] = 0;
-    return;
-  }
-  cluster.sync();  // every CTA's mbarriers are initialised before a peer's st.async can reach them
-  const double c = sh.c;
-  const u32 n1 = s.n + 1;
-  const u32 Ne = s.Ne;
-  int* spl = node_spl + (size_t)node * (K + 2);
-  if (writer) { spl[1] = 1; spl[K + 1] = (int)n1; }
-  // this CTA's local chunk l is the global chunk 8 l + crank; l_end = its first chunk that starts at or behind Ne
-  const u32 nchunks = (Ne + PR_C - 1) / PR_C;
-  const u32 l_end = nchunks > crank ? (nchunks - crank + 7u) >> 3 : 0u;
-  u32 W = PR_WMAX, w_est = PR_WMAX;
-  u32 sstep = 0;        // super-steps so far (selects the exchange buffers / mbarrier parities)
-  u32 fill_hi = 0;      // the ring holds (or has requested) the local chunks [fill_hi - PR_S, fill_hi), chunk l in slot l mod PR_S
-  u32 pmask = (1u << PR_S) - 1u;  // bit t: parity of the most recent bulk copy into slot t (first copy: phase 0)
-  u32 ver_hi = 0;       // (consumer warps) chunks below ver_hi are known to have landed
-  u32 j = 1;
-  bool broke = false, feasible = false;
-  u32 pcur = __ldg(s.P + 1), wcur = __ldg(s.Wt + 1);
-  const u32 x1_base = smem_addr(&sh.x1[0][0]), x2_base = smem_addr(&sh.x2[0][0][0]);
-  const u32 bar_x1 = smem_addr(&sh.mb_x1[0]), bar_x2 = smem_addr(&sh.mb_x2[0]);
-  // slots [a, b) of the ring as a PR_S-bit mask (b - a <= PR_S)
-  auto slot_bits = [](u32 a, u32 b) -> u32 {
-    const u32 len = b - a;
-    u32 m = ((1u << len) - 1u) << (a % PR_S);
-    return (m | (m >> PR_S)) & ((1u << PR_S) - 1u);
-  };
-  for (int k = 1; k <= K; ++k) {
-    if (!cost_leq(stream_cost<T>(s, 0, 0, 0), c)) { broke = true; break; }  // even the empty part exceeds c
-    const u32 e0 = pcur;
-    const i64 wj = (i64)wcur;
-    u32 jlast = j, grun = 0;
-    bool first = true, missed = false;
-    RN(1, 1);
-    for (u32 g_win = e0 / PR_C;;) {
-#ifdef CPB_PROBE_TIMING
-      unsigned long long rt_last = clock64();
-#endif
-      RN(0, 1);
-      RN(5, W);
-      const u32 ph = sstep & 1u, xpar = (sstep >> 1) & 1u;
-      const u32 l0 = (g_win + 7u - crank) >> 3;              // first local chunk of this CTA inside the window
-      const u32 p0 = (crank - g_win) & 7u;                   // its position in window order; the others follow at +8
-      // ---- ring bookkeeping, replicated in every thread: which chunks get requested now, the slots' new parities ----
-      const bool rewind = l0 + PR_S < fill_hi;               // the part starts behind the ring
-      const u32 req_lo = rewind ? l0 : max(fill_hi, l0);
-      const u32 req_hi = l0 + PR_S;
-      const u32 iss_lo = min(req_lo, l_end), iss_hi = min(req_hi, l_end);  // chunks that exist (start in front of Ne)
-      const u32 old_lo = fill_hi > (u32)PR_S ? fill_hi - PR_S : 0u;       // (rewind) what was in flight before
-      const u32 old_hi = min(fill_hi, l_end), old_pmask = pmask;
-      if (iss_hi > iss_lo) pmask ^= slot_bits(iss_lo, iss_hi);
-      if (rewind) { ver_hi = l0; RN(3, 1); }
-      fill_hi = req_hi;
-      if (producer) {
-        // ---- warp 31: arm this super-step's exchange barriers, keep the ring full, resolve the chunks' column ranges ----
-        if (lane == 0) {
-          mbar_expect_tx(bar_x1 + 8u * ph, 32u * W);
-          mbar_expect_tx(bar_x2 + 8u * ph, 128u);
-          if (rewind)  // every copy still in flight lands before its slot is armed again
-            for (u32 l = old_lo; l < old_hi; ++l) mbar_wait(smem_addr(&sh.mb_full[l % PR_S]), (old_pmask >> (l % PR_S)) & 1u, 4u, l, sstep, fill_hi, 1u);
-          if (iss_hi > iss_lo) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the slots' last readers were generic-proxy loads
-            for (u32 l = iss_lo; l < iss_hi; ++l) {
-              const u64 x0 = ((u64)l * 8u + crank) * PR_C;
-              const u32 slot = l % PR_S;
-              const u32 bar = smem_addr(&sh.mb_full[slot]);
-              mbar_expect_tx(bar, PR_C * 4u);
-              bulk_load(smem_addr(ring + (size_t)slot * PR_C), s.prev + x0, PR_C * 4u, bar);
-            }
-          }
-        }
-        // chunk [x0, x0 + C) owns the column boundaries r with x0 < P[r] <= x0 + C
-        if (lane < (int)W) {
-          const u32 g = (l0 + lane) * 8u + crank;
-          const u64 x0 = (u64)g * PR_C;
-          const bool head = first && g == g_win;  // the chunk holding the part's first element: candidates start right after j
-          u32 ja, jb;
-          if (head) ja = j + 1;
-          else ja = (x0 < Ne) ? __ldg(s.chunk_col + g) + 2 : n1 + 1;
-          if (x0 >= Ne && !head) jb = 0;
-          else jb = (x0 + PR_C >= Ne) ? n1 : __ldg(s.chunk_col + g + 1) + 1;
-          sh.cb[ph][lane][0] = ja;
-          sh.cb[ph][lane][1] = (jb >= ja) ? jb - ja + 1 : 0;
-        }
-      } else {
-        // ---- warps 0..30: bit masks of `prev < j`; the 64 W groups of the window are dealt round-robin to the warps ----
-        for (u32 l = max(ver_hi, l0); l < min(l0 + W, l_end); ++l)  // chunks of the window this warp has not seen land yet
-          mbar_wait(smem_addr(&sh.mb_full[l % PR_S]), (pmask >> (l % PR_S)) & 1u, 1u, l, sstep, e0, W);
-        ver_hi = max(ver_hi, l0 + W);
-        for (u32 G = (u32)warp; G < (u32)PR_G * W; G += PR_CW) {
-          const u32 v = G >> 6, gi = G & 63u;
-          const u32 l = l0 + v;
-          const u64 gbase = ((u64)l * 8u + crank) * PR_C + gi * 128u;
-          unsigned m0 = 0, m1 = 0, m2 = 0, m3 = 0;
-          if (gbase < Ne && gbase + 128u > e0) {  // (warp-uniform) the group holds elements of [e0, Ne)
-            const uint4 pv = *reinterpret_cast<const uint4*>(ring + (size_t)(l % PR_S) * PR_C + gi * 128u + lane * 4);
-            if (gbase >= e0 && gbase + 128u <= Ne) {
-              m0 = __ballot_sync(0xffffffffu, pv.x <= e0);
-              m1 = __ballot_sync(0xffffffffu, pv.y <= e0);
-              m2 = __ballot_sync(0xffffffffu, pv.z <= e0);
-              m3 = __ballot_sync(0xffffffffu, pv.w <= e0);
-            } else {  // the part's first group / the array's last group: mask what lies outside [e0, Ne)
-              const u64 idx = gbase + (u32)lane * 4u;
-              m0 = __ballot_sync(0xffffffffu, pv.x <= e0 && idx + 0 >= e0 && idx + 0 < Ne);
-              m1 = __ballot_sync(0xffffffffu, pv.y <= e0 && idx + 1 >= e0 && idx + 1 < Ne);
-              m2 = __ballot_sync(0xffffffffu, pv.z <= e0 && idx + 2 >= e0 && idx + 2 < Ne);
-              m3 = __ballot_sync(0xffffffffu, pv.w <= e0 && idx + 3 >= e0 && idx + 3 < Ne);
-            }
-          }
-          if (lane == 0) {
-            *reinterpret_cast<uint4*>(&sh.mask[v][gi][0]) = make_uint4(m0, m1, m2, m3);
-            sh.cnt[v][gi] = __popc(m0) + __popc(m1) + __popc(m2) + __popc(m3);
-          }
-        }
-      }
-      RT(0);
-      __syncthreads();  // B1: masks, counts, column ranges
-      RT(1);
-      // ---- warp v < W scans chunk v (two groups per lane) ----
-      if (warp < (int)W) {
-        const u32 t0 = sh.cnt[warp][2 * lane], t1 = sh.cnt[warp][2 * lane + 1];
-        u32 inc = t0 + t1;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const u32 y = __shfl_up_sync(0xffffffffu, inc, o);
-          if (lane >= o) inc += y;
-        }
-        const u32 ex = inc - t0 - t1;
-        sh.cum[warp][2 * lane] = ex;
-        sh.cum[warp][2 * lane + 1] = ex + t0;
-        if (lane == 31) sh.cum[warp][PR_G] = inc;
-      }
-      // ---- this CTA's boundary candidates, flat over its W chunks ----
-      u32 cn[PR_WMAX + 1], cja[PR_WMAX];
-      cn[0] = 0;
-#pragma unroll
-      for (int v = 0; v < PR_WMAX; ++v) {
-        const bool on = v < (int)W;
-        cja[v] = on ? sh.cb[ph][v][0] : 0u;
-        cn[v + 1] = cn[v] + (on ? sh.cb[ph][v][1] : 0u);
-      }
-      const u32 nb = cn[PR_WMAX];
-      auto locate = [&](u32 b, u32& r, u32& v) {  // flat candidate index -> (boundary, local chunk)
-        v = (b >= cn[1] ? 1u : 0u) + (b >= cn[2] ? 1u : 0u);
-        const u32 cv = v == 0 ? cn[0] : (v == 1 ? cn[1] : cn[2]);
-        const u32 jv = v == 0 ? cja[0] : (v == 1 ? cja[1] : cja[2]);
-        r = jv + (b - cv);
-      };
-      // round 1 of the search: thread t owns the candidates [t stride, (t + 1) stride) and tests the LAST one; its
-      // offsets are fetched while the chunk totals travel
-      u32 lo = 0, hi = nb;  // candidates [0, lo) feasible, [hi, nb) not
-      u32 stride = (nb + PR_THREADS - 1) / PR_THREADS;
-      bool live = nb > 0 && (u64)tid * stride < nb;
-      u32 r = 0, v = 0, pj = 0, w = 0;
-      if (live) {
-        locate((u32)min((u64)(tid + 1) * stride - 1, (u64)nb - 1), r, v);
-        pj = __ldg(s.P + r);
-        w = s.same_w ? pj : __ldg(s.Wt + r);
-      }
-      __syncthreads();  // B2: chunk prefixes and totals
-      RT(2);
-      // ---- exchange 1: warp 8 v + p pushes the total of chunk v to CTA p (one remote store per warp) ----
-      if (warp < 8 * (int)W && lane == 0) {
-        const u32 cv = (u32)warp >> 3, peer = (u32)warp & 7u;
-        const u32 dst = x1_base + 4u * (ph * 8u * PR_WMAX + cv * 8u + p0);
-        st_async_u32(map_peer(dst, peer), sh.cum[cv][PR_G], map_peer(bar_x1 + 8u * ph, peer));
-      }
-      if (producer) {
-        // warp 31 turns the window's chunk totals (window order: position q belongs to CTA (g_win + q) mod 8) into the
-        // base of each of this CTA's chunks
-        mbar_wait_cluster(bar_x1 + 8u * ph, xpar, 2u, sstep, W, e0, g_win);
-        const u32 nwin = 8u * W;  // <= 24
-        const u32 t = (u32)lane < nwin ? sh.x1[ph][lane] : 0u;
-        u32 inc = t;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const u32 y = __shfl_up_sync(0xffffffffu, inc, o);
-          if (lane >= o) inc += y;
-        }
-        if ((u32)lane < nwin && ((u32)lane & 7u) == p0) sh.base[ph][lane >> 3] = inc - t;
-        if (lane == 31) sh.base[ph][PR_WMAX] = inc;
-      }
-      RT(3);
-      __syncthreads();  // B3: bases
-      RT(4);
-      const u32 tile_tot = sh.base[ph][PR_WMAX];
-      // count of `prev < j` among the part's elements left of offset pj, pj inside (or at the end of) local chunk v
-      auto count_at = [&](u32 pj_, u32 v_) -> u32 {
-        const u32 x = pj_ - (u32)((((u64)(l0 + v_)) * 8u + crank) * PR_C);  // 0 <= x <= C
-        const u32 g = x >> 7, rr = x & 127u;
-        u32 cnt = grun + sh.base[ph][v_] + sh.cum[v_][g];
-        const uint4 mk = *reinterpret_cast<const uint4*>(&sh.mask[v_][g][0]);
-        const u32 mm[4] = {mk.x, mk.y, mk.z, mk.w};
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const int nl = ((int)rr - t + 3) >> 2;  // lanes l with 4 l + t < rr
-          const u32 msk = nl >= 32 ? 0xffffffffu : (nl <= 0 ? 0u : ((1u << nl) - 1u));
-          cnt += __popc(mm[t] & msk);
-        }
-        return cnt;
-      };
-      u32 cnt = 0, lastp = 0, lastw = 0;
-      if (nb == 0) RN(4, 1);
-      while (lo < hi) {  // (uniform over the CTA)
-        RN(2, 1);
-        bool ok = false;
-        if (live) {
-          sh.pj[tid] = pj;
-          sh.w[tid] = w;
-          ok = cost_leq(stream_cost<T>(s, (i64)r - (i64)j, (i64)w - wj, (i64)count_at(pj, v)), c);
-        }
-        const int ct = __syncthreads_count(ok);  // monotone costs: threads 0 .. ct-1 hold feasible candidates
-        if (ct > 0) { lastp = sh.pj[ct - 1]; lastw = sh.w[ct - 1]; }
-        const u32 nlo = (u32)min((u64)lo + (u64)ct * stride, (u64)hi);
-        const u32 nhi = (u32)min((u64)hi, (u64)lo + (u64)(ct + 1) * stride - 1);  // thread ct's last candidate failed
-        lo = nlo;
-        hi = max(nhi, nlo);
-        if (stride == 1 || lo >= hi) break;
-        __syncthreads();  // sh.pj / sh.w are rewritten by the next round
-        const u32 span = hi - lo;
-        stride = (span + PR_THREADS - 1) / PR_THREADS;
-        live = (u64)lo + (u64)tid * stride < hi;
-        if (live) {
-          locate((u32)min((u64)lo + (u64)(tid + 1) * stride - 1, (u64)hi - 1), r, v);
-          pj = __ldg(s.P + r);
-          w = s.same_w ? pj : __ldg(s.Wt + r);
-        }
-      }
-      cnt = lo;
-      RT(5);
-      // ---- exchange 2: (feasible boundaries, boundaries, P and Wt at the last feasible one), warp p pushes to CTA p ----
-      if (warp < BS_CLUSTER && lane == 0) {
-        const u32 dst = x2_base + 16u * (ph * 8u + crank);
-        st_async_v4(map_peer(dst, (u32)warp), cnt, nb, lastp, lastw, map_peer(bar_x2 + 8u * ph, (u32)warp));
-      }
-      RT(6);
-      mbar_wait_cluster(bar_x2 + 8u * ph, xpar, 3u, sstep, W, e0, g_win);
-      RT(7);
-      u32 feas = 0, nbs = 0, bestp = 0;
-      bool any = false;
-#pragma unroll
-      for (int p = 0; p < BS_CLUSTER; ++p) {
-        const uint4 q = *reinterpret_cast<const uint4*>(&sh.x2[ph][p][0]);
-        feas += q.x;
-        nbs += q.y;
-        if (q.x > 0 && (!any || q.z >= bestp)) { any = true; bestp = q.z; pcur = q.z; wcur = q.w; }  // the furthest feasible boundary wins
-      }
-      ++sstep;
-      first = false;
-      jlast += feas;
-      if (feas < nbs) break;                                     // the cost crossed c inside this window
-      if (((u64)g_win + 8u * W) * PR_C >= Ne) break;             // streamed to the end: jlast == n + 1
-      grun += tile_tot;
-      g_win += 8u * W;
-      W = PR_WMAX;                                               // the part is longer than estimated
-      missed = true;
-    }
-    {  // size the next part's window from this part (+1/8 slack, + the misaligned start)
-      const u32 elems = pcur - e0;
-      const u32 want = (elems + (elems >> 3) + 9u * PR_C - 1u) / (PR_C * BS_CLUSTER);
-      w_est = missed ? (u32)PR_WMAX : max(min(want, (u32)PR_WMAX), w_est > 1u ? w_est - 1u : 1u);
-      W = w_est;
-    }
-    if (k == K) { feasible = (jlast == n1); break; }
-    if (jlast == n1) {
-      if (writer)
-        for (int t = k + 1; t <= K; ++t) spl[t] = (int)n1;
-      feasible = true;
-      break;
-    }
-    if (writer) spl[k + 1] = (int)jlast;
-    j = jlast;
-  }
-  if (writer) {
-    node_c[node] = c;
-    node_res[node] = (!broke && feasible) ? 2 : 1;
-  }
-  if (producer && lane == 0) {  // the ring runs ahead of the search: wait for the bulk copies still in flight into this CTA's shared memory
-    const u32 a = fill_hi > (u32)PR_S ? fill_hi - PR_S : 0u;
-    for (u32 l = a; l < min(fill_hi, l_end); ++l) mbar_wait(smem_addr(&sh.mb_full[l % PR_S]), (pmask >> (l % PR_S)) & 1u, 4u, l, sstep, fill_hi, 0u);
-  }
-  cluster.sync();  // no CTA may exit while peers can still write into its shared memory
 }
 
 __global__ void k_count_zero(const u32* __restrict__ v, size_t n, u32* __restrict__ out) {
@@ -1739,7 +1316,6 @@ static void stream_view(Oracle& f, DevStream& ds) {
   const Matrix& A = *f.A;
   ds.prev = f.ls->prev.get();
   ds.colq = f.ls->colq.get();
-  ds.chunk_col = f.ls->chunk_col.get();
   ds.P = f.ls->P;
   ds.Wt = (f.dev.kind == CPB_MODEL_MONOSYM) ? f.overpos.get() - 1 : A.pos.get() - 1;
   ds.Ne = (u32)f.ls->Ne;
@@ -1974,38 +1550,26 @@ BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int*
   return run.release();
 }
 
-// CPB_PROBE_RING=0 selects the register-tile probes (k_probe_stream) instead of the shared-memory ring form
-static unsigned long long* g_ring_dbg_host = nullptr;
-static std::string ring_debug_string() {
-  if (!g_ring_dbg_host || g_ring_dbg_host[0] == 0) return "";
-  const unsigned long long w0 = g_ring_dbg_host[0], w1 = g_ring_dbg_host[1], w2 = g_ring_dbg_host[2];
+static unsigned long long* g_probe_dbg_host = nullptr;
+static std::string probe_debug_string() {
+  if (!g_probe_dbg_host || g_probe_dbg_host[0] == 0) return "";
+  const unsigned long long w0 = g_probe_dbg_host[0], w1 = g_probe_dbg_host[1], w2 = g_probe_dbg_host[2];
   char buf[256];
   std::snprintf(buf, sizeof(buf), " [probe wait timed out: tag=%llu crank=%llu block=%llu tid=%llu a=%llu b=%llu c=%llu d=%llu]", (w0 >> 4) & 15, (w0 >> 8) & 15,
                 (w0 >> 12) & 0xffff, (w0 >> 28) & 0xfff, w1 >> 32, w1 & 0xffffffffull, w2 >> 32, w2 & 0xffffffffull);
   return buf;
 }
-// the host-mapped record a timed-out wait leaves (see ring_wait_failed)
-static void ring_debug_arm() {
-  if (g_ring_dbg_host) return;
+// the host-mapped record a timed-out wait leaves (see probe_wait_failed)
+static void probe_debug_arm() {
+  if (g_probe_dbg_host) return;
   unsigned long long* d = nullptr;
-  CPB_CUDA(cudaHostAlloc((void**)&g_ring_dbg_host, 128, cudaHostAllocMapped));
-  std::memset(g_ring_dbg_host, 0, 128);
-  CPB_CUDA(cudaHostGetDevicePointer((void**)&d, g_ring_dbg_host, 0));
-  CPB_CUDA(cudaMemcpyToSymbol(g_ring_dbg, &d, sizeof(d)));
+  CPB_CUDA(cudaHostAlloc((void**)&g_probe_dbg_host, 128, cudaHostAllocMapped));
+  std::memset(g_probe_dbg_host, 0, 128);
+  CPB_CUDA(cudaHostGetDevicePointer((void**)&d, g_probe_dbg_host, 0));
+  CPB_CUDA(cudaMemcpyToSymbol(g_probe_dbg, &d, sizeof(d)));
 }
 static void check_probes(cudaError_t e) {
-  if (e != cudaSuccess) throw Error(CPB_ERR_CUDA, std::string("CUDA error: ") + cudaGetErrorString(e) + " in the bisection probes" + ring_debug_string());
-}
-static bool probe_ring_enabled() {
-  static bool attr_set = false;
-  if (env_int("CPB_PROBE_RING", 0) == 0) return false;
-  if (!attr_set) {
-    ring_debug_arm();
-    CPB_CUDA(cudaFuncSetAttribute(k_probe_ring<i64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PR_RING_BYTES));
-    CPB_CUDA(cudaFuncSetAttribute(k_probe_ring<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PR_RING_BYTES));
-    attr_set = true;
-  }
-  return true;
+  if (e != cudaSuccess) throw Error(CPB_ERR_CUDA, std::string("CUDA error: ") + cudaGetErrorString(e) + " in the bisection probes" + probe_debug_string());
 }
 
 // probes the nodes [node_lo, node_hi) of the current round's speculation tree
@@ -2019,47 +1583,14 @@ void bisect_probe(BisectRun& run, int node_lo, int node_hi) {
   for (int t = node_lo; t < node_hi; ++t) run.speculated += run.h_ids[t] >= 0;
   for (int base = node_lo; base < node_hi; base += (1 << BS_LOCAL_DEPTH)) {
     const int cnt = std::min(node_hi - base, 1 << BS_LOCAL_DEPTH);
-    if (run.stream && probe_ring_enabled()) {
-      // algorithmic bytes of one fused pass over the links for the thresholds of this launch (SURVEY.md 8d, G4)
-      ProfScope pk("k_probe_ring", (double)(f.ls->Ne + f.A->n + 1) * 4.0 + (double)cnt * (K + 1) * 8.0);
-      if (f.dev.is_float)
-        CPB_LAUNCH(k_probe_ring<double>, cnt * BS_CLUSTER, PR_THREADS, PR_RING_BYTES, run.ds, K, run.eps1, run.st.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
-      else
-        CPB_LAUNCH(k_probe_ring<i64>, cnt * BS_CLUSTER, PR_THREADS, PR_RING_BYTES, run.ds, K, run.eps1, run.st.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
-    } else if (run.stream) {
+    if (run.stream) {
       // algorithmic bytes of one fused pass over the links for the thresholds of this launch (SURVEY.md 8d, G4)
       ProfScope pk("k_probe_stream", (double)(f.ls->Ne + f.A->n + 1) * 4.0 + (double)cnt * (K + 1) * 8.0);
-      const bool ax = env_int("CPB_PROBE_ASYNC", 1) != 0;  // exchanges by st.async + mbarrier (0: DSMEM stores + cluster barriers)
-      const int cl = env_int("CPB_PROBE_CLUSTER", 8) == 16 ? 16 : 8;  // CTAs per threshold (16: the non-portable cluster size)
-      ring_debug_arm();
-      auto launch = [&](auto kern, int CLv) {
-        static bool attr16_set = false;
-        if (CLv == 16) CPB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        (void)attr16_set;
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)(cnt * CLv), 1, 1);
-        cfg.blockDim = dim3(SP_THREADS, 1, 1);
-        cfg.dynamicSmemBytes = 0;
-        cfg.stream = ctx().stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)CLv;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        CPB_CUDA(cudaLaunchKernelEx(&cfg, kern, run.ds, K, run.eps1, (const BisectState*)run.st.get(), run.node_spl, run.node_res, run.node_c, (const int*)run.ids.get(), base));
-        ctx().launches += 1;
-      };
-      if (f.dev.is_float) {
-        if (cl == 16) launch(k_probe_stream<double, true, 16>, 16);
-        else if (ax) launch(k_probe_stream<double, true, 8>, 8);
-        else launch(k_probe_stream<double, false, 8>, 8);
-      } else {
-        if (cl == 16) launch(k_probe_stream<i64, true, 16>, 16);
-        else if (ax) launch(k_probe_stream<i64, true, 8>, 8);
-        else launch(k_probe_stream<i64, false, 8>, 8);
-      }
+      probe_debug_arm();
+      if (f.dev.is_float)
+        CPB_LAUNCH(k_probe_stream<double>, cnt * BS_CLUSTER, SP_THREADS, 0, run.ds, K, run.eps1, run.st.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
+      else
+        CPB_LAUNCH(k_probe_stream<i64>, cnt * BS_CLUSTER, SP_THREADS, 0, run.ds, K, run.eps1, run.st.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
     } else if (f.dev.is_float) {
       CPB_LAUNCH(k_bisect_round<double>, cnt * BS_CLUSTER, BS_THREADS, 0, f.dev, K, run.eps1, run.st.get(), run.hint_lo.get(), run.hint_hi.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
     } else {
@@ -2105,22 +1636,6 @@ void bisect_finish(BisectRun* run_ptr, int64_t* h_spl_out) {
 }
 
 #ifdef CPB_PROBE_TIMING
-void ring_timing_dump() {
-  unsigned long long t[16], n[8];
-  cudaMemcpyFromSymbol(t, g_ring_t, sizeof(t));
-  cudaMemcpyFromSymbol(n, g_ring_n, sizeof(n));
-  const char* names[11] = {"fill|ballots (to B1)", "sync B1", "scan+candidates (to B2)", "push x1|wait x1+bases", "sync B3", "search rounds", "push x2", "wait x2",
-                           "-", "-", "-"};
-  const double ss = (double)std::max<unsigned long long>(n[0], 1);
-  double tot = 0;
-  for (int i = 0; i < 11; ++i) tot += (double)t[i];
-  for (int i = 0; i < 11; ++i) std::printf("ring_timing %-22s %8.1f cycles/super-step\n", names[i], (double)t[i] / ss);
-  std::printf("ring_timing total %.1f cycles/super-step; super-steps %llu parts %llu search rounds %llu rewinds %llu empty %llu mean W %.2f\n", tot / ss, n[0], n[1], n[2], n[3], n[4],
-              (double)n[5] / ss);
-  unsigned long long z[16] = {0};
-  cudaMemcpyToSymbol(g_ring_t, z, sizeof(t));
-  cudaMemcpyToSymbol(g_ring_n, z, sizeof(n));
-}
 void probe_timing_dump() {
   unsigned long long t[16], n;
   cudaMemcpyFromSymbol(t, g_probe_t, sizeof(t));
@@ -2158,11 +1673,7 @@ int probe_cluster_capacity(bool stream) {
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   int n = 0;
-  if (stream && probe_ring_enabled()) {
-    cfg.blockDim = dim3(PR_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = PR_RING_BYTES;
-    CPB_CUDA(cudaOccupancyMaxActiveClusters(&n, k_probe_ring<i64>, &cfg));
-  } else if (stream) CPB_CUDA(cudaOccupancyMaxActiveClusters(&n, (k_probe_stream<i64, true, 8>), &cfg));
+  if (stream) CPB_CUDA(cudaOccupancyMaxActiveClusters(&n, k_probe_stream<i64>, &cfg));
   else CPB_CUDA(cudaOccupancyMaxActiveClusters(&n, k_bisect_round<i64>, &cfg));
   return n;
 }
@@ -2250,13 +1761,10 @@ void solve_bisect(Oracle& f, bool lazy, double eps, i64 K, int64_t* h_spl_out) {
     delete run;
     throw;
   }
-#ifdef CPB_PROBE_TIMING
-  const bool run_was_ring = run->stream && probe_ring_enabled();
-#endif
   bisect_finish(run, h_spl_out);
   trace_mark("finish");
 #ifdef CPB_PROBE_TIMING
-  if (env_int("CPB_PROBE_TIMING_DUMP", 0)) { if (run_was_ring) ring_timing_dump(); else probe_timing_dump(); }
+  if (env_int("CPB_PROBE_TIMING_DUMP", 0)) probe_timing_dump();
 #endif
 }
 

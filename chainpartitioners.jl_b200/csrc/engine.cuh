@@ -44,7 +44,6 @@ struct LinkStream {
                      //      streams with position-valued links do not build it (1 GB and 0.65 ms at config 3)
   DBuf<u32> colq;    // [ceil(Ne / LS_COLQ) + 1] 0-based column of every LS_COLQ-th element: what the streaming probes need to find the
                      //      columns of a tile's two ends (a short cooperative search on P from there)
-  DBuf<u32> chunk_col;  // [ceil(Ne / LS_CHUNK) + 1] column of the first element of every LS_CHUNK-element chunk (ring probes)
   DBuf<u32> P_own;   // own prefix array (diagonal-augmented variant)
   DBuf<u32> first_count;  // [2] number of links equal to 0 (= non-empty rows); max row degree seen by the row-segment form
   bool speculative = false;   // the row-segment kernels were launched before that degree was checked (see compute_prev_links)
@@ -53,11 +52,11 @@ struct LinkStream {
   size_t Ne = 0;
 };
 struct Matrix;
-static constexpr u32 LS_CHUNK = 8192;   // chunk of the link array the ring probes stage at a time; `prev` is allocated in whole chunks
-static constexpr u32 LS_COLQ = 128;     // granularity of LinkStream::colq (LS_CHUNK is a multiple of it): 128 elements rarely span more than 32 columns
+static constexpr u32 LS_COLQ = 128;     // granularity of LinkStream::colq: 128 elements rarely span more than 32 columns
 static constexpr u32 LT_MAX_DEG = 128;  // largest row degree handled by the row-segment link construction (links.cu)
 std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row_lo = 0, i64 row_hi = ((i64)1 << 62), bool defer_check = false,
                                               bool force_sort = false, bool as_pos = false);
+void fill_colq(LinkStream& ls, u32 n);  // LinkStream::colq from P and Ne
 
 // SparseColorArrays.jl: NetCount :103-118, dianetcount! :72-99, SelfNetCount :177-229, SelfPinCount :281-318
 enum { RANK_NET = 1, RANK_DIANET = 2, RANK_SELFNET = 3, RANK_SELFPIN = 4 };

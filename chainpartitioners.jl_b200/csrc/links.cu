@@ -232,23 +232,11 @@ __global__ void k_colq(const u32* __restrict__ P, u32 n, size_t Ne, u32* __restr
   }
   colq[g] = c;
 }
-// chunk_col[g] = column of element g * LS_CHUNK for every chunk that starts inside the array (0 behind it)
-__global__ void k_chunk_cols(const u32* __restrict__ colq, size_t Ne, u32* __restrict__ chunk_col, u32 nchunks) {
-  const u32 g = blockIdx.x * blockDim.x + threadIdx.x;
-  if (g > nchunks) return;
-  const size_t x = (size_t)g * LS_CHUNK;
-  chunk_col[g] = x < Ne ? colq[x / LS_COLQ] : 0u;
-}
-static void fill_chunk_cols(LinkStream& ls, u32 n) {
+void fill_colq(LinkStream& ls, u32 n) {
   const u32 G = (u32)((ls.Ne + LS_COLQ - 1) / LS_COLQ);
   ls.colq.alloc((size_t)G + 2);
   CPB_LAUNCH(k_colq, (G + 1) / 256 + 1, 256, 0, ls.P, n, ls.Ne, ls.colq.get(), G + 1);
-  const u32 nchunks = (u32)((ls.Ne + LS_CHUNK - 1) / LS_CHUNK);
-  ls.chunk_col.alloc((size_t)nchunks + 1);
-  CPB_LAUNCH(k_chunk_cols, nchunks / 256 + 1, 256, 0, ls.colq.get(), ls.Ne, ls.chunk_col.get(), nchunks);
 }
-void fill_chunk_cols_public(LinkStream& ls, u32 n) { fill_chunk_cols(ls, n); }
-static size_t padded_links(size_t Ne) { return (Ne + LS_CHUNK - 1) / LS_CHUNK * LS_CHUNK + LS_CHUNK; }  // whole chunks (bulk copies read them whole)
 
 static u32 read_u32(const u32* d) {
   u32 h = 0;
@@ -373,13 +361,13 @@ std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row
   const u32 n = (u32)A.n, m = (u32)A.m;
   if (!dia) {
     ls->Ne = N;
-    ls->prev.alloc(padded_links(N));
+    ls->prev.alloc(N);
     if (!as_pos) ls->colidx.alloc(N);
     ls->first_count.alloc(2);
     ls->speculative = compute_prev_links(A.pos.get(), A.row.get(), m, n, N, ls->prev.get(), as_pos ? nullptr : ls->colidx.get(), ls->first_count.get(), row_lo,
                                          row_hi, defer_check, force_sort, as_pos, &A.max_row_deg);
     ls->P = A.pos.get() - 1;  // P[x] = pos[x-1]
-    fill_chunk_cols(*ls, n);
+    fill_colq(*ls, n);
     return ls;
   }
   CPB_REQUIRE(A.m >= A.n, "dianetcount needs m >= n");
@@ -398,13 +386,13 @@ std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row
   if (n) CPB_LAUNCH(k_aug_diag, grid_for(n), 256, 0, pos2, add.get(), n, row2.get());
   i64 heavy_hint = A.max_row_deg > (i64)LT_MAX_DEG ? A.max_row_deg : -1;  // A + I only adds entries: a heavy row of A stays heavy
   ls->Ne = N2;
-  ls->prev.alloc(padded_links(N2));
+  ls->prev.alloc(N2);
   if (!as_pos) ls->colidx.alloc(N2);
   ls->first_count.alloc(2);
   ls->speculative = compute_prev_links(pos2, row2.get(), m, n, N2, ls->prev.get(), as_pos ? nullptr : ls->colidx.get(), ls->first_count.get(), row_lo, row_hi,
                                        defer_check, force_sort, as_pos, &heavy_hint);
   ls->P = ls->P_own.get();  // P[x] = pos2[x-1]
-  fill_chunk_cols(*ls, n);
+  fill_colq(*ls, n);
   return ls;
 }
 

@@ -185,8 +185,6 @@ __global__ void k_carry_pick(const u32* __restrict__ all, size_t m, int rank, u3
 
 static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-void fill_chunk_cols_public(LinkStream& ls, u32 n);  // links.cu
-
 // run heads of the packed (row << 32 | local position) pairs: as k_shard_heads
 __global__ void k_shard_heads_pairs(const u64* __restrict__ sorted, size_t cnt, const u32* __restrict__ carry, u32* __restrict__ prev_blk,
                                     u32* __restrict__ first_count) {
@@ -259,11 +257,11 @@ static std::unique_ptr<LinkStream> new_link_stream(const Matrix& A, size_t min_e
   auto ls = std::make_unique<LinkStream>();
   ls->pos_links = true;
   ls->Ne = N;
-  ls->prev.alloc(std::max<size_t>((N + LS_CHUNK - 1) / LS_CHUNK * LS_CHUNK + LS_CHUNK, min_entries + LS_CHUNK));
+  ls->prev.alloc(std::max<size_t>(N, min_entries));
   ls->first_count.alloc(2);
   CPB_CUDA(cudaMemsetAsync(ls->first_count.get(), 0, 2 * sizeof(u32), ctx().stream));
   ls->P = A.pos.get() - 1;
-  fill_chunk_cols_public(*ls, (u32)A.n);
+  fill_colq(*ls, (u32)A.n);
   ls->speculative = false;
   return ls;
 }

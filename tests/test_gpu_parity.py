@@ -295,11 +295,10 @@ def test_speculation_depth_does_not_change_result(ref, monkeypatch):
         assert np.array_equal(cp.partition_stripe(A, 16, mtd).spl, exp), depth
 
 
-def test_probe_ring_and_register_tile_forms(ref, monkeypatch):
-    """The two streaming-probe kernels (k_probe_ring: shared-memory ring + st.async exchanges, the default; k_probe_stream:
-    register tiles + cluster barriers, CPB_PROBE_RING=0) against the CPU oracle on inputs that span many 4096-element chunks
-    per part, many parts per chunk, long runs of empty columns (more than 4096 boundary candidates per window), the
-    diagonal-augmented stream and Float64 costs."""
+def test_streaming_probe_tiles(ref):
+    """The streaming-probe kernel (k_probe_stream: register tiles, st.async exchanges between the cluster's CTAs) against the
+    CPU oracle on inputs whose parts span several super-steps, super-steps that hold many parts, long runs of empty columns
+    (more than 4096 boundary candidates per CTA and super-step), the diagonal-augmented stream and Float64 costs."""
     rng = np.random.default_rng(77)
     n_sparse = 300_000
     cols = np.sort(rng.choice(n_sparse, 4000, replace=False))
@@ -318,11 +317,8 @@ def test_probe_ring_and_register_tile_forms(ref, monkeypatch):
         for K in Ks:
             for mtd in (cp.LazyBisectCostBottleneckSplitter(f, eps), cp.BisectCostBottleneckSplitter(f, eps)):
                 exp = ref.partition_stripe(A, K, mtd).spl
-                for ring in ("1", "0"):
-                    monkeypatch.setenv("CPB_PROBE_RING", ring)
-                    got = cp.partition_stripe(dA, K, mtd).spl
-                    assert np.array_equal(got, exp), (A.n, K, type(mtd).__name__, "ring=" + ring)
-        monkeypatch.delenv("CPB_PROBE_RING", raising=False)
+                got = cp.partition_stripe(dA, K, mtd).spl
+                assert np.array_equal(got, exp), (A.n, K, type(mtd).__name__)
         dA.close()
 
 
