@@ -21,6 +21,7 @@ __all__ = [
     "pack_stripe", "partition_plaid", "pack_plaid", "bottleneck_value", "total_value", "pincount", "netcount",
     "dianetcount", "selfnetcount", "selfpincount", "PrefixMatrix", "dominancecount", "dominancesum", "rookcount", "rooksum", "profile_enable", "profile_reset", "profile_get",
     "Communicator", "ShardedMatrix", "partition_stripe_sharded", "partition_stripe_sharded_emulated", "sharded_stats", "shard_range",
+    "partition_plaid_sharded", "partition_plaid_sharded_emulated", "adjointpattern_sharded_emulated",
     "launch_count", "probe_cluster_capacity", "bisect_stats", "bisect_plan", "bisect_prewalk", "timer_start", "timer_stop", "StepwiseBisection", "StripeOracle", "init", "synchronize", "trim_memory", "library_path", "load_library", "CpbError",
 ]
 
@@ -38,6 +39,7 @@ ABI_SYMBOLS = [
     "cpb_bisect_begin", "cpb_bisect_probe", "cpb_bisect_advance", "cpb_bisect_finish", "cpb_bisect_stats", "cpb_bisect_plan", "cpb_bisect_prewalk", "cpb_probe_cluster_capacity",
     "cpb_comm_unique_id", "cpb_comm_init", "cpb_comm_destroy", "cpb_comm_info", "cpb_shard_range", "cpb_sharded_matrix_create", "cpb_sharded_matrix_destroy",
     "cpb_partition_stripe_sharded", "cpb_partition_stripe_sharded_emulated", "cpb_sharded_stats",
+    "cpb_sharded_adjointpattern", "cpb_adjointpattern_sharded_emulated", "cpb_sharded_matrix_get",
     "cpb_links_partial", "cpb_oracle_set_links", "cpb_prefix_create", "cpb_prefix_query", "cpb_prefix_destroy", "cpb_matrix_permute", "cpb_trim_memory", "cpb_matrix_create_i32",
 ]
 
@@ -99,6 +101,9 @@ def load_library():
         lib.cpb_partition_stripe_sharded.argtypes = [vp, ctypes.POINTER(T.CModel), i32, dbl, i64, vp]
         lib.cpb_partition_stripe_sharded_emulated.argtypes = [vp, ctypes.POINTER(T.CModel), i32, dbl, i64, i32, vp]
         lib.cpb_sharded_stats.argtypes = [vp]
+        lib.cpb_sharded_adjointpattern.argtypes = [vp, ctypes.POINTER(vp)]
+        lib.cpb_adjointpattern_sharded_emulated.argtypes = [vp, i32, ctypes.POINTER(vp)]
+        lib.cpb_sharded_matrix_get.argtypes = [vp, vp, vp, ctypes.POINTER(i64), ctypes.POINTER(i64)]
         _lib = lib
     return _lib
 
@@ -686,6 +691,30 @@ class ShardedMatrix:
         self._h = ctypes.c_void_p()
         _check(load_library().cpb_sharded_matrix_create(self.m, self.n, self.nnz, _p(A.colptr), _p(A.rowval), 0, ctypes.byref(self._h)))
 
+    @classmethod
+    def _adopt(cls, h, m, n, nnz, comm):
+        S = cls.__new__(cls)
+        S.m, S.n, S.nnz, S.comm, S._h = int(m), int(n), int(nnz), comm, h
+        return S
+
+    def adjointpattern(self) -> "ShardedMatrix":
+        """``adjointpattern`` of the sharded pattern (``cpb_sharded_adjointpattern``; collective): a ``ShardedMatrix`` of the
+        transpose with the same blocks of CSC positions."""
+        h = ctypes.c_void_p()
+        _check(load_library().cpb_sharded_adjointpattern(self._h, ctypes.byref(h)))
+        return ShardedMatrix._adopt(h, self.n, self.m, self.nnz, self.comm)
+
+    def to_host_block(self):
+        """-> ``(colptr, rowval_block, q_lo, q_hi)``: the complete 1-based column offsets, the 1-based row indices of this
+        rank's CSC positions ``[q_lo, q_hi)`` (0-based, half-open, as ``shard_range``)."""
+        lib = load_library()
+        lo, hi = ctypes.c_int64(), ctypes.c_int64()
+        _check(lib.cpb_sharded_matrix_get(self._h, None, None, ctypes.byref(lo), ctypes.byref(hi)))
+        colptr = np.empty(self.n + 1, dtype=I64)
+        rowval = np.empty(hi.value - lo.value, dtype=I64)
+        _check(lib.cpb_sharded_matrix_get(self._h, _p(colptr), _p(rowval) if rowval.size else None, None, None))
+        return colptr, rowval, lo.value, hi.value
+
     def close(self):
         if self._h is not None and _lib is not None:
             _lib.cpb_sharded_matrix_destroy(self._h)
@@ -702,15 +731,16 @@ def _sharded_args(method):
     code, spec, eps = T.split_method_code(method)
     f, con = T.split_constrained(spec)
     if con.enabled:
-        raise TypeError("sharded solves take an unconstrained AffineConnectivityModel")
+        raise TypeError("sharded solves take an unconstrained AffineConnectivityModel or AffineMonotonizedSymmetricConnectivityModel")
     cm, keep = f.to_c()
     return code, cm, keep, eps
 
 
 def partition_stripe_sharded(A, K, method, comm: Optional[Communicator] = None) -> T.SplitPartition:
-    """``partition_stripe(A, K, BisectCost/LazyBisectCost(AffineConnectivityModel, eps))`` as ONE solve over all ranks of the
-    communicator (collective; every rank gets the same ``SplitPartition``).  ``A``: a ``ShardedMatrix`` (resident) or a host
-    matrix (every rank uploads its block inside the call)."""
+    """``partition_stripe(A, K, BisectCost/LazyBisectCost(f, eps))`` as ONE solve over all ranks of the communicator
+    (collective; every rank gets the same ``SplitPartition``), ``f`` an ``AffineConnectivityModel`` or an
+    ``AffineMonotonizedSymmetricConnectivityModel`` (square ``A``).  ``A``: a ``ShardedMatrix`` (resident) or a host matrix
+    (every rank uploads its block inside the call)."""
     K = int(K)
     code, cm, keep, eps = _sharded_args(method)
     own = not isinstance(A, ShardedMatrix)
@@ -740,7 +770,114 @@ def sharded_stats() -> dict:
     _check(load_library().cpb_sharded_stats(out))
     return {"world": int(out[0]), "host_ms_until_links_queued": out[1], "bisection_ms_incl_links_wait": out[2], "rounds": int(out[3]),
             "link_allgather_bytes": out[4], "carry_bytes_per_hop": out[5], "threshold_allgather_bytes": out[6], "thresholds_per_round": int(out[7]),
-            "limiting_collective": "in-place ncclAllGather of the link array (nnz x 4 bytes on every rank)"}
+            "transpose_pair_bytes_received": out[8], "transpose_histogram_allgather_bytes": out[9],
+            "limiting_collective": "in-place gather of the link array (nnz x 4 bytes on every rank; nnz of A + I for the monotonized symmetric model)"}
+
+
+def adjointpattern_sharded_emulated(A, world: int):
+    """``adjointpattern`` built as ``ShardedMatrix.adjointpattern`` would build it over ``world`` ranks, the ranks played one
+    after the other on this GPU (tests).  Host matrix in -> host matrix out; DeviceMatrix in -> DeviceMatrix out."""
+    with _Scoped(A) as dm:
+        h = ctypes.c_void_p()
+        _check(load_library().cpb_adjointpattern_sharded_emulated(dm._h, int(world), ctypes.byref(h)))
+        out = DeviceMatrix(h, dm.n, dm.m, dm.nnz)
+        if isinstance(A, DeviceMatrix):
+            return out
+        res = out.to_host()
+        out.close()
+        return res
+
+
+def _plaid_sharded_methods(method):
+    """The stripe methods of a plaid partitioner, each checked for the sharded solve (before any collective starts)."""
+    if isinstance(method, T.DisjointPartitioner):
+        mtds = [method.mtd, method.mtd2]
+    elif isinstance(method, (T.AlternatingPartitioner, T.SymmetricPartitioner)):
+        mtds = list(method.mtds)
+    else:
+        raise TypeError(f"partition_plaid_sharded: unsupported method {type(method).__name__}")
+    if not mtds:
+        raise TypeError("partition_plaid_sharded: no stripe methods")
+    for mtd in mtds:
+        code, spec, _ = T.split_method_code(mtd)
+        if code not in (T.SPLIT_BISECT_COST, T.SPLIT_LAZY_BISECT_COST):
+            raise TypeError(f"partition_plaid_sharded: {type(mtd).__name__} has no sharded form (BisectCost / LazyBisectCost splitters only)")
+        f, con = T.split_constrained(spec)
+        if con.enabled or getattr(f, "kind", None) not in (T.MODEL_CONNECTIVITY, T.MODEL_MONOSYM):
+            raise TypeError("partition_plaid_sharded: the stripe methods must use an unconstrained AffineConnectivityModel or "
+                            f"AffineMonotonizedSymmetricConnectivityModel, not {type(f).__name__}")
+    return mtds
+
+
+def _plaid_walk(method, mtds, solve, on_A, on_T):
+    """partition_plaid's alternation (AlternatingPartitioner.jl:6-88) over a stripe solve ``solve(side, K, mtd)``."""
+    if isinstance(method, T.DisjointPartitioner):
+        Phi = solve(on_A(), mtds[0])
+        return solve(on_T(), mtds[1]), Phi
+    if isinstance(method, T.AlternatingPartitioner):
+        Phi = solve(on_A(), mtds[0])
+        Pi = solve(on_T(), mtds[1])
+        for i, mtd in enumerate(mtds[2:], start=1):
+            if i % 2 == 1:
+                Phi = solve(on_A(), mtd)
+            else:
+                Pi = solve(on_T(), mtd)
+        return Pi, Phi
+    Pi = solve(on_A(), mtds[0])  # SymmetricPartitioner
+    for i, mtd in enumerate(mtds[1:], start=1):
+        Pi = solve(on_A() if i % 2 == 1 else on_T(), mtd)
+    return Pi, Pi
+
+
+def partition_plaid_sharded(A, K, method, comm: Optional[Communicator] = None, adj_A=None):
+    """``partition_plaid(A, K, method)`` with every stripe solve sharded over the ranks of the communicator (collective; every
+    rank gets the same ``(Pi, Phi)``).  ``method``: an Alternating / Symmetric / Disjoint partitioner whose stripe methods are
+    BisectCost / LazyBisectCost over the connectivity or the monotonized symmetric model; anything else raises TypeError
+    before any collective starts.  ``A``: a ``ShardedMatrix`` or a host matrix; ``adj_A``: the transpose as either, or None
+    (built once per call with ``ShardedMatrix.adjointpattern`` and shared by the alternations, as on one GPU)."""
+    K = int(K)
+    mtds = _plaid_sharded_methods(method)
+    own = not isinstance(A, ShardedMatrix)
+    sA = ShardedMatrix(A, comm) if own else A
+    held = {}
+
+    def on_T():
+        if "T" not in held:
+            if adj_A is None:
+                held["T"], held["own"] = sA.adjointpattern(), True
+            elif isinstance(adj_A, ShardedMatrix):
+                held["T"], held["own"] = adj_A, False
+            else:
+                held["T"], held["own"] = ShardedMatrix(adj_A, comm), True
+        return held["T"]
+
+    try:
+        return _plaid_walk(method, mtds, lambda S, mtd: partition_stripe_sharded(S, K, mtd), lambda: sA, on_T)
+    finally:
+        if held.get("own"):
+            held["T"].close()
+        if own:
+            sA.close()
+
+
+def partition_plaid_sharded_emulated(A, K, method, world: int):
+    """``partition_plaid_sharded`` with ``world`` ranks played one after the other on this GPU: the emulated sharded transpose
+    and the emulated sharded stripe solves (tests)."""
+    K = int(K)
+    mtds = _plaid_sharded_methods(method)
+    with _Scoped(A) as dA:
+        held = {}
+
+        def on_T():
+            if "T" not in held:
+                held["T"] = adjointpattern_sharded_emulated(dA, world)
+            return held["T"]
+
+        try:
+            return _plaid_walk(method, mtds, lambda M, mtd: partition_stripe_sharded_emulated(M, K, mtd, world), lambda: dA, on_T)
+        finally:
+            if "T" in held:
+                held["T"].close()
 
 
 class StepwiseBisection:

@@ -707,6 +707,10 @@ void sharded_destroy(ShardedMatrix* S);
 void solve_sharded(ShardedMatrix& S, const cpb_model* mdl, int method, double eps, i64 K, int64_t* h_spl_out);
 void solve_sharded_emulated(Matrix& A, const cpb_model* mdl, int method, double eps, i64 K, int world, int64_t* h_spl_out);
 void sharded_stats(double out[16]);
+ShardedMatrix* sharded_adjointpattern(const ShardedMatrix& S);
+std::unique_ptr<Matrix> adjoint_pattern_sharded_emulated(const Matrix& A, int world);
+void sharded_dims(const ShardedMatrix& S, i64* m, i64* n, i64* nnz, i64* q_lo, i64* q_hi);
+void sharded_get(const ShardedMatrix& S, i64* h_colptr, i64* h_rowval_blk);
 }  // namespace cpb
 }  // extern "C++"
 
@@ -770,6 +774,35 @@ int cpb_partition_stripe_sharded_emulated(cpb_matrix* A, const cpb_model* mdl, i
   CPB_REQUIRE(A && mdl && spl_out, "NULL argument");
   CPB_REQUIRE(K >= 1, "K must be >= 1");
   solve_sharded_emulated(A->M, mdl, method, eps, K, world, spl_out);
+  CPB_API_END
+}
+int cpb_sharded_adjointpattern(cpb_sharded* A, cpb_sharded** out) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(A && out, "NULL argument");
+  *out = reinterpret_cast<cpb_sharded*>(sharded_adjointpattern(*reinterpret_cast<ShardedMatrix*>(A)));
+  CPB_API_END
+}
+int cpb_adjointpattern_sharded_emulated(cpb_matrix* A, int world, cpb_matrix** out) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(A && out, "NULL argument");
+  auto B = adjoint_pattern_sharded_emulated(A->M, world);
+  auto h = std::make_unique<cpb_matrix>();
+  h->M = std::move(*B);
+  *out = h.release();
+  CPB_API_END
+}
+int cpb_sharded_matrix_get(const cpb_sharded* A, int64_t* colptr_out, int64_t* rowval_block_out, int64_t* q_lo, int64_t* q_hi) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(A, "NULL argument");
+  const ShardedMatrix& S = *reinterpret_cast<const ShardedMatrix*>(A);
+  i64 lo = 0, hi = 0;
+  sharded_dims(S, nullptr, nullptr, nullptr, &lo, &hi);
+  if (q_lo) *q_lo = lo;
+  if (q_hi) *q_hi = hi;
+  if (colptr_out || rowval_block_out) sharded_get(S, (i64*)colptr_out, (i64*)rowval_block_out);
   CPB_API_END
 }
 int cpb_sharded_stats(double out[16]) {

@@ -9,7 +9,9 @@
 //     block the predecessor lies in an earlier block: the per-row "last position seen" array (m * 4 bytes) travels down
 //     the ranks once (rank r receives the running array from r - 1, fixes its run heads, merges its own last positions,
 //     sends on), exactly the reference's hst[] carried across column blocks.  One in-place all-gather then gives every
-//     rank the whole link array (N * 4 bytes) for the probes.
+//     rank the whole link array (N * 4 bytes) for the probes.  The monotonized symmetric model streams the links of A + I:
+//     the same construction on each rank's block of A + I positions (see "A + I" below), gathered by per-rank broadcasts.
+//   * adjointpattern of a sharded matrix (the alternation's second solve runs on the transpose): see below.
 //   * bisection: the speculation tree of a round holds world x 15 thresholds; rank r probes slots [15 r, 15 (r + 1)) and
 //     the per-slot results (feasible?, threshold, split vector) are all-gathered; every rank walks the same tree, so all
 //     ranks end with the same state and the same split vector -- the reference's threshold sequence, hence its result.
@@ -32,6 +34,7 @@ struct NcclApi {
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*Broadcast)(const void*, void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*GroupStart)() = nullptr;
@@ -69,6 +72,7 @@ static void load_nccl() {
   g_nccl.CommDestroy = (decltype(g_nccl.CommDestroy))sym("ncclCommDestroy");
   g_nccl.AllGather = (decltype(g_nccl.AllGather))sym("ncclAllGather");
   g_nccl.AllReduce = (decltype(g_nccl.AllReduce))sym("ncclAllReduce");
+  g_nccl.Broadcast = (decltype(g_nccl.Broadcast))sym("ncclBroadcast");
   g_nccl.Send = (decltype(g_nccl.Send))sym("ncclSend");
   g_nccl.Recv = (decltype(g_nccl.Recv))sym("ncclRecv");
   g_nccl.GroupStart = (decltype(g_nccl.GroupStart))sym("ncclGroupStart");
@@ -252,27 +256,155 @@ static void block_heads(const BlockWork& w, const u32* carry_in, u32 q_lo, u32* 
   else CPB_LAUNCH(k_shard_heads, grid_for(w.cntL), 256, 0, w.sk, w.sq, w.cntL, carry_in, prev_full + q_lo, first_count);
 }
 
-static std::unique_ptr<LinkStream> new_link_stream(const Matrix& A, size_t min_entries) {
-  const size_t N = (size_t)A.N;
+// ---- A + I: the monotonized symmetric model streams the links of A + I (links.cu, build_link_stream(dia = true)) ----------
+// A virtual diagonal (j, j) is appended to every column j that lacks one (SparseColorArrays.jl:87-91).  Position q of A moves
+// to img(q) = q + addscan[c(q)] in A + I, c(q) the column holding q.  Rank r's block of A + I is [img(q_lo), img(q_hi)) with
+// img(N) = N2 and rank 0 starting at 0: a virtual diagonal goes with the last real element of its column, and the diagonals
+// of leading empty columns go to rank 0.  The blocks are contiguous, ordered and cover [0, N2); every rank computes all.
+
+// the column holding element q < pos[n]: the largest c < n with pos[c] <= q (a non-empty column)
+__device__ __forceinline__ u32 column_of(const u32* __restrict__ pos, u32 n, u32 q) {
+  u32 lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const u32 mid = lo + ((hi - lo + 1) >> 1);
+    if (__ldg(pos + mid) <= q) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// present[j] = 1 if the part of column j inside the block [q_lo, q_hi) holds row j (the binary search of k_diag_missing on
+// that part; rows ascend inside a column).  Flags of several blocks combine with MAX.
+__global__ void k_shard_diag_present(const u32* __restrict__ pos, const u32* __restrict__ row_blk, u32 n, u32 q_lo, u32 q_hi,
+                                     unsigned char* __restrict__ present) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += stride) {
+    u32 lo = max(__ldg(pos + j), q_lo), hi = min(__ldg(pos + j + 1), q_hi);
+    if (lo >= hi) continue;
+    const u32 end = hi;
+    while (lo < hi) {
+      const u32 mid = lo + ((hi - lo) >> 1);
+      if (row_blk[mid - q_lo] < (u32)j) lo = mid + 1; else hi = mid;
+    }
+    if (lo < end && row_blk[lo - q_lo] == (u32)j) present[j] = 1;
+  }
+}
+__global__ void k_shard_dia_add(const unsigned char* __restrict__ present, u32 n, u32* __restrict__ add) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j <= n; j += stride) add[j] = (j < n && !present[j]) ? 1u : 0u;
+}
+// P_own[0] = 0, P_own[j + 1] = pos[j] + addscan[j]: the A + I column offsets as LinkStream::P (P[x] = pos2[x - 1])
+__global__ void k_shard_dia_pos(const u32* __restrict__ pos, const u32* __restrict__ addscan, u32 n, u32* __restrict__ P_own) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j <= n; j += stride) {
+    if (j == 0) P_own[0] = 0;
+    P_own[j + 1] = pos[j] + addscan[j];
+  }
+}
+// bnd[r] = first A + I position of rank r's block, r = 0..world (bnd[world] = N2)
+__global__ void k_shard_dia_bounds(const u32* __restrict__ pos, const u32* __restrict__ addscan, u32 n, u32 N, u32 cnt, int world, u32* __restrict__ bnd) {
+  const int r = threadIdx.x;
+  if (r > world) return;
+  const u64 q = min((u64)N, (u64)r * cnt);
+  u32 b;
+  if (r == 0) b = 0;
+  else if (q >= N) b = N + addscan[n];
+  else b = (u32)q + addscan[column_of(pos, n, (u32)q)];
+  bnd[r] = b;
+}
+// the block's real rows at their A + I positions, then its virtual diagonals
+__global__ void k_shard_dia_rows(const u32* __restrict__ pos, const u32* __restrict__ addscan, u32 n, const u32* __restrict__ row_blk, u32 q_lo,
+                                 size_t cntL, u32 b_lo, u32* __restrict__ row2) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cntL; p += stride) {
+    const u32 q = q_lo + (u32)p;
+    row2[q + __ldg(addscan + column_of(pos, n, q)) - b_lo] = row_blk[p];
+  }
+}
+__global__ void k_shard_dia_diag(const u32* __restrict__ P_own, const u32* __restrict__ add, u32 n, u32 b_lo, u32 b_hi, u32* __restrict__ row2) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += stride) {
+    if (!add[j]) continue;
+    const u32 d = P_own[j + 2] - 1;  // pos2[j + 1] - 1: the end of column j (k_aug_diag)
+    if (d >= b_lo && d < b_hi) row2[d - b_lo] = (u32)j;
+  }
+}
+
+struct DiaLayout {
+  DBuf<u32> add, addscan, P_own;
+  std::vector<u32> bnd;  // [world + 1] A + I block boundaries
+  size_t N2 = 0;
+};
+// from the combined "diagonal present" flags: addscan, the A + I column offsets and every rank's A + I block
+static void dia_layout(const Matrix& A, const unsigned char* present, int world, i64 cnt, DiaLayout& L) {
+  const u32 n = (u32)A.n;
+  L.add.alloc((size_t)n + 1);
+  L.addscan.alloc((size_t)n + 1);
+  L.P_own.alloc((size_t)n + 2);
+  CPB_LAUNCH(k_shard_dia_add, grid_for((size_t)n + 1), 256, 0, present, n, L.add.get());
+  exclusive_scan_u32(L.add.get(), L.addscan.get(), (size_t)n + 1);
+  CPB_LAUNCH(k_shard_dia_pos, grid_for((size_t)n + 1), 256, 0, A.pos.get(), L.addscan.get(), n, L.P_own.get());
+  DBuf<u32> bnd((size_t)world + 1);
+  CPB_LAUNCH(k_shard_dia_bounds, 1, 32, 0, A.pos.get(), L.addscan.get(), n, (u32)A.N, (u32)cnt, world, bnd.get());
+  L.bnd.assign((size_t)world + 1, 0u);
+  CPB_CUDA(cudaMemcpyAsync(L.bnd.data(), bnd.get(), ((size_t)world + 1) * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
+  CPB_CUDA(cudaStreamSynchronize(ctx().stream));
+  L.N2 = L.bnd[world];
+}
+// rank r's rows of A + I (rows of its A block [q_lo, q_lo + cntL) plus the virtual diagonals that fall into its A + I block)
+static void dia_block_rows(const Matrix& A, const DiaLayout& L, const u32* P_own, const u32* row_blk, i64 q_lo, size_t cntL, int r, DBuf<u32>& out) {
+  const u32 n = (u32)A.n, b_lo = L.bnd[r], b_hi = L.bnd[r + 1];
+  out.alloc(std::max<size_t>(b_hi - b_lo, 1));
+  if (cntL) CPB_LAUNCH(k_shard_dia_rows, grid_for(cntL), 256, 0, A.pos.get(), L.addscan.get(), n, row_blk, (u32)q_lo, cntL, b_lo, out.get());
+  if (n && b_hi > b_lo) CPB_LAUNCH(k_shard_dia_diag, grid_for(n), 256, 0, P_own, L.add.get(), n, b_lo, b_hi, out.get());
+}
+
+// link stream of A (dia = nullptr: P = A.pos) or of A + I (P = the layout's offsets, taken over)
+static std::unique_ptr<LinkStream> new_link_stream(const Matrix& A, size_t min_entries, DiaLayout* dia) {
+  const size_t Ne = dia ? dia->N2 : (size_t)A.N;
   auto ls = std::make_unique<LinkStream>();
   ls->pos_links = true;
-  ls->Ne = N;
-  ls->prev.alloc(std::max<size_t>(N, min_entries));
+  ls->Ne = Ne;
+  ls->prev.alloc(std::max<size_t>(Ne, min_entries));
   ls->first_count.alloc(2);
   CPB_CUDA(cudaMemsetAsync(ls->first_count.get(), 0, 2 * sizeof(u32), ctx().stream));
-  ls->P = A.pos.get() - 1;
+  if (dia) {
+    ls->P_own = std::move(dia->P_own);
+    ls->P = ls->P_own.get();
+  } else {
+    ls->P = A.pos.get() - 1;
+  }
   fill_colq(*ls, (u32)A.n);
   ls->speculative = false;
   return ls;
 }
 
-// the complete link stream of the sharded matrix on every rank
-static std::unique_ptr<LinkStream> sharded_link_stream(const ShardedMatrix& S) {
+// the complete link stream of the sharded matrix (dia: of A + I) on every rank
+static std::unique_ptr<LinkStream> sharded_link_stream(const ShardedMatrix& S, bool dia) {
   const Matrix& A = S.M;
   const size_t m = (size_t)A.m;
-  auto ls = new_link_stream(A, (size_t)S.cnt * S.world);
+  const u32 n = (u32)A.n;
+  const u32* rows = S.row_blk.get();
+  size_t cntL = (size_t)(S.q_hi - S.q_lo);
+  u32 off = (u32)S.q_lo;
+  DiaLayout L;
+  DBuf<u32> rows2;
+  if (dia) {
+    ProfScope pk("shard_dia", (double)n);
+    DBuf<unsigned char> present(std::max<size_t>(n, 1));
+    present.zero();
+    if (n) CPB_LAUNCH(k_shard_diag_present, grid_for(n), 256, 0, A.pos.get(), rows, n, (u32)S.q_lo, (u32)S.q_hi, present.get());
+    if (S.world > 1 && n) CPB_NCCL(g_nccl.AllReduce(present.get(), present.get(), n, ncclUint8, ncclMax, g_comm, ctx().stream));
+    dia_layout(A, present.get(), S.world, S.cnt, L);  // (synchronises: `present` is free afterwards)
+  }
+  auto ls = new_link_stream(A, dia ? 0 : (size_t)S.cnt * S.world, dia ? &L : nullptr);
+  if (dia) {
+    dia_block_rows(A, L, ls->P_own.get(), rows, S.q_lo, cntL, S.rank, rows2);
+    rows = rows2.get();
+    off = L.bnd[S.rank];
+    cntL = L.bnd[S.rank + 1] - L.bnd[S.rank];
+  }
   BlockWork w;
-  block_local_links(S.row_blk.get(), (size_t)(S.q_hi - S.q_lo), (u32)S.q_lo, m, ls->prev.get(), w);
+  block_local_links(rows, cntL, off, m, ls->prev.get(), w);
   DBuf<u32> carry(std::max<size_t>(m, 1));
   const bool has_in = S.rank > 0 && S.world > 1;
   if (S.world > 2 && std::getenv("CPB_SHARD_CHAIN") == nullptr) {
@@ -283,7 +415,7 @@ static std::unique_ptr<LinkStream> sharded_link_stream(const ShardedMatrix& S) {
     DBuf<u32> all(std::max<size_t>(m, 1) * S.world);
     CPB_NCCL(g_nccl.AllGather(w.last_local.get(), all.get(), m, ncclUint32, g_comm, ctx().stream));
     if (has_in) CPB_LAUNCH(k_carry_pick, grid_for(m), 256, 0, all.get(), m, S.rank, carry.get());
-    block_heads(w, has_in ? carry.get() : nullptr, (u32)S.q_lo, ls->prev.get(), ls->first_count.get());
+    block_heads(w, has_in ? carry.get() : nullptr, off, ls->prev.get(), ls->first_count.get());
     CPB_CUDA(cudaStreamSynchronize(ctx().stream));  // `all` is released at the end of this scope
   } else {
     // two ranks (or CPB_SHARD_CHAIN=1): the "last seen" array travels down the ranks once, m * 4 bytes per hop
@@ -295,12 +427,21 @@ static std::unique_ptr<LinkStream> sharded_link_stream(const ShardedMatrix& S) {
       CPB_NCCL(g_nccl.Send(out.get(), m, ncclUint32, S.rank + 1, g_comm, ctx().stream));
       CPB_CUDA(cudaStreamSynchronize(ctx().stream));  // `out` is released at the end of this scope
     }
-    block_heads(w, has_in ? carry.get() : nullptr, (u32)S.q_lo, ls->prev.get(), ls->first_count.get());
+    block_heads(w, has_in ? carry.get() : nullptr, off, ls->prev.get(), ls->first_count.get());
   }
   if (S.world > 1) {
-    ProfScope pk("shard_allgather", (double)S.cnt * S.world * 4.0);
+    ProfScope pk("shard_allgather", (double)(dia ? L.N2 : (size_t)S.cnt * S.world) * 4.0);
     CPB_NCCL(g_nccl.GroupStart());
-    CPB_NCCL(g_nccl.AllGather(ls->prev.get() + (size_t)S.rank * S.cnt, ls->prev.get(), (size_t)S.cnt, ncclUint32, g_comm, ctx().stream));
+    if (dia) {
+      // the A + I blocks differ in size by their virtual diagonals: one in-place broadcast per rank at its offset
+      for (int r = 0; r < S.world; ++r) {
+        const size_t len = L.bnd[r + 1] - L.bnd[r];
+        u32* const p = ls->prev.get() + L.bnd[r];
+        if (len) CPB_NCCL(g_nccl.Broadcast(p, p, len, ncclUint32, r, g_comm, ctx().stream));
+      }
+    } else {
+      CPB_NCCL(g_nccl.AllGather(ls->prev.get() + (size_t)S.rank * S.cnt, ls->prev.get(), (size_t)S.cnt, ncclUint32, g_comm, ctx().stream));
+    }
     CPB_NCCL(g_nccl.AllReduce(ls->first_count.get(), ls->first_count.get(), 1, ncclUint32, ncclSum, g_comm, ctx().stream));
     CPB_NCCL(g_nccl.GroupEnd());
   }
@@ -308,39 +449,69 @@ static std::unique_ptr<LinkStream> sharded_link_stream(const ShardedMatrix& S) {
 }
 
 // The same construction with the ranks played one after the other on this GPU (tests: the block kernels and the carry rule
-// without NCCL).  A holds the complete pattern.
-std::unique_ptr<LinkStream> emulated_sharded_link_stream(const Matrix& A, int world) {
+// without NCCL).  A holds the complete pattern; dia: the link stream of A + I with the blocks of sharded_link_stream.
+std::unique_ptr<LinkStream> emulated_sharded_link_stream(const Matrix& A, int world, bool dia) {
   const size_t m = (size_t)A.m;
+  const u32 n = (u32)A.n;
   i64 cnt = 0;
   shard_range(A.N, 0, world, &cnt, nullptr, nullptr);
-  auto ls = new_link_stream(A, (size_t)cnt * world);
+  DiaLayout L;
+  if (dia) {
+    DBuf<unsigned char> present(std::max<size_t>(n, 1));
+    present.zero();
+    for (int r = 0; r < world && n; ++r) {
+      i64 lo = 0, hi = 0;
+      shard_range(A.N, r, world, nullptr, &lo, &hi);
+      if (hi > lo) CPB_LAUNCH(k_shard_diag_present, grid_for(n), 256, 0, A.pos.get(), A.row.get() + lo, n, (u32)lo, (u32)hi, present.get());
+    }
+    dia_layout(A, present.get(), world, cnt, L);
+  }
+  auto ls = new_link_stream(A, dia ? 0 : (size_t)cnt * world, dia ? &L : nullptr);
+  // rank r's rows and their first (A or A + I) position
+  auto block = [&](int r, DBuf<u32>& tmp, const u32*& rows, size_t& len, u32& off) {
+    i64 lo = 0, hi = 0;
+    shard_range(A.N, r, world, nullptr, &lo, &hi);
+    rows = A.row.get() + lo;
+    len = (size_t)(hi - lo);
+    off = (u32)lo;
+    if (dia) {
+      dia_block_rows(A, L, ls->P_own.get(), rows, lo, len, r, tmp);
+      rows = tmp.get();
+      off = L.bnd[r];
+      len = L.bnd[r + 1] - L.bnd[r];
+    }
+  };
   DBuf<u32> carry(std::max<size_t>(m, 1)), next(std::max<size_t>(m, 1));
   const bool pick = world > 2 && std::getenv("CPB_SHARD_CHAIN") == nullptr;  // the same two carry forms as the real ranks
   if (pick) {
     // pass 1: every block's local links and last positions; pass 2: heads from the nearest non-empty entry below
     DBuf<u32> all(std::max<size_t>(m, 1) * world);
     std::vector<BlockWork> ws(world);
+    std::vector<u32> offs(world);
     for (int r = 0; r < world; ++r) {
-      i64 lo = 0, hi = 0;
-      shard_range(A.N, r, world, nullptr, &lo, &hi);
-      block_local_links(A.row.get() + lo, (size_t)(hi - lo), (u32)lo, m, ls->prev.get(), ws[r]);
+      DBuf<u32> tmp;
+      const u32* rows = nullptr;
+      size_t len = 0;
+      block(r, tmp, rows, len, offs[r]);
+      block_local_links(rows, len, offs[r], m, ls->prev.get(), ws[r]);
       if (m) CPB_CUDA(cudaMemcpyAsync(all.get() + (size_t)r * m, ws[r].last_local.get(), m * sizeof(u32), cudaMemcpyDeviceToDevice, ctx().stream));
     }
     for (int r = 0; r < world; ++r) {
-      i64 lo = 0;
-      shard_range(A.N, r, world, nullptr, &lo, nullptr);
       if (r > 0) CPB_LAUNCH(k_carry_pick, grid_for(m), 256, 0, all.get(), m, r, carry.get());
-      block_heads(ws[r], r > 0 ? carry.get() : nullptr, (u32)lo, ls->prev.get(), ls->first_count.get());
+      block_heads(ws[r], r > 0 ? carry.get() : nullptr, offs[r], ls->prev.get(), ls->first_count.get());
     }
     CPB_CUDA(cudaStreamSynchronize(ctx().stream));  // the blocks' buffers are released here
     return ls;
   }
   for (int r = 0; r < world; ++r) {
-    i64 lo = 0, hi = 0;
-    shard_range(A.N, r, world, nullptr, &lo, &hi);
+    DBuf<u32> tmp;
+    const u32* rows = nullptr;
+    size_t len = 0;
+    u32 off = 0;
+    block(r, tmp, rows, len, off);
     BlockWork w;
-    block_local_links(A.row.get() + lo, (size_t)(hi - lo), (u32)lo, m, ls->prev.get(), w);
-    block_heads(w, r > 0 ? carry.get() : nullptr, (u32)lo, ls->prev.get(), ls->first_count.get());
+    block_local_links(rows, len, off, m, ls->prev.get(), w);
+    block_heads(w, r > 0 ? carry.get() : nullptr, off, ls->prev.get(), ls->first_count.get());
     CPB_LAUNCH(k_carry_merge, grid_for(m), 256, 0, w.last_local.get(), r > 0 ? carry.get() : nullptr, next.get(), m);
     std::swap(carry, next);
     CPB_CUDA(cudaStreamSynchronize(ctx().stream));  // the block's buffers are released here
@@ -398,13 +569,16 @@ void sharded_dims(const ShardedMatrix& S, i64* m, i64* n, i64* nnz, i64* q_lo, i
 void bisect_node_buffers(BisectRun& run, int** res, double** c, int** spl, int* P);  // bisect.cu
 bool bisect_is_done(BisectRun& run);
 
+static bool sharded_model(const cpb_model* mdl) { return mdl && (mdl->kind == CPB_MODEL_CONNECTIVITY || mdl->kind == CPB_MODEL_MONOSYM); }
+
 void solve_sharded(ShardedMatrix& S, const cpb_model* mdl, int method, double eps, i64 K, int64_t* h_spl_out) {
   CPB_REQUIRE(method == CPB_SPLIT_BISECT_COST || method == CPB_SPLIT_LAZY_BISECT_COST, "sharded solves: BisectCost / LazyBisectCost splitters");
-  CPB_REQUIRE(mdl && mdl->kind == CPB_MODEL_CONNECTIVITY, "sharded solves: AffineConnectivityModel (the streaming link form)");
+  CPB_REQUIRE(sharded_model(mdl), "sharded solves: AffineConnectivityModel or AffineMonotonizedSymmetricConnectivityModel (the streaming link forms)");
   CPB_REQUIRE(S.world == g_world && S.rank == g_rank, "the sharded matrix was created under another communicator");
   const double t0 = now_ms();
-  auto f = oracle_create(S.M, mdl, nullptr, 0);
-  f->ls = sharded_link_stream(S);
+  auto f = oracle_create(S.M, mdl, nullptr, 0);  // (the monotonized symmetric model checks that A is square, on every rank alike)
+  const bool dia = mdl->kind == CPB_MODEL_MONOSYM;
+  f->ls = sharded_link_stream(S, dia);
   f->ls_complete = true;
   const double t1 = now_ms();
   const int cap = std::min(probe_cluster_capacity(true), 15);
@@ -448,7 +622,7 @@ void solve_sharded(ShardedMatrix& S, const cpb_model* mdl, int method, double ep
   g_shard_stats[1] = t1 - t0;                      // link construction incl. carry + all-gather, host clock (asynchronous part excluded)
   g_shard_stats[2] = t2 - t1;                      // bisection (includes waiting for the construction queued before it)
   g_shard_stats[3] = rounds;
-  g_shard_stats[4] = (double)S.cnt * S.world * 4.0; // link all-gather bytes (whole array)
+  g_shard_stats[4] = (double)(dia ? f->ls->Ne : (size_t)S.cnt * S.world) * 4.0;  // link gather bytes (whole array; A + I for dia)
   g_shard_stats[5] = (double)S.M.m * 4.0;          // carry bytes per hop
   g_shard_stats[6] = coll_bytes;                   // threshold all-gather bytes
   g_shard_stats[7] = nodes;
@@ -457,10 +631,10 @@ void solve_sharded(ShardedMatrix& S, const cpb_model* mdl, int method, double ep
 // single-GPU stand-in for `world` ranks: emulated block construction, every threshold slot probed here (tests)
 void solve_sharded_emulated(Matrix& A, const cpb_model* mdl, int method, double eps, i64 K, int world, int64_t* h_spl_out) {
   CPB_REQUIRE(method == CPB_SPLIT_BISECT_COST || method == CPB_SPLIT_LAZY_BISECT_COST, "sharded solves: BisectCost / LazyBisectCost splitters");
-  CPB_REQUIRE(mdl && mdl->kind == CPB_MODEL_CONNECTIVITY, "sharded solves: AffineConnectivityModel (the streaming link form)");
+  CPB_REQUIRE(sharded_model(mdl), "sharded solves: AffineConnectivityModel or AffineMonotonizedSymmetricConnectivityModel (the streaming link forms)");
   CPB_REQUIRE(world >= 1 && world <= 16, "1..16 emulated ranks");
   auto f = oracle_create(A, mdl, nullptr, 0);
-  f->ls = emulated_sharded_link_stream(A, world);
+  f->ls = emulated_sharded_link_stream(A, world, mdl->kind == CPB_MODEL_MONOSYM);
   f->ls_complete = true;
   const int cap = std::min(probe_cluster_capacity(true), 15);
   const int per = std::max(1, std::min(cap, 255 / world));
@@ -477,6 +651,227 @@ void solve_sharded_emulated(Matrix& A, const cpb_model* mdl, int method, double 
     throw;
   }
   bisect_finish(run, h_spl_out);
+}
+
+// ---- adjointpattern of a sharded matrix ---------------------------------------------------------------------------------
+// Aᵀ has the same nnz, so the same shard_range blocks.  Rank r sorts its block by row (stable: columns ascend inside a row);
+// the per-block row histograms (m x 4 bytes each) are all-gathered, which gives every rank colptrᵀ (their sum) and
+// below[i] (the sum over the lower ranks).  The Aᵀ position of the block's k-th entry of row i is
+// colptrᵀ[i] + below[i] + k.  Those positions increase along the sorted block, so each destination rank receives one
+// contiguous slice: (column << 32 | position) pairs, 8 bytes per nonzero, grouped ncclSend / ncclRecv, scattered there.
+__global__ void k_tr_hist(const u32* __restrict__ rows, size_t cnt, u32* __restrict__ hist) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cnt; p += stride) atomicAdd(&hist[rows[p]], 1u);
+}
+// tot[i] = entries of row i over all blocks, below[i] = over the blocks of the ranks below `rank`
+__global__ void k_tr_combine(const u32* __restrict__ all, size_t m, int world, int rank, u32* __restrict__ tot, u32* __restrict__ below) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride) {
+    u32 t = 0, b = 0;
+    for (int r = 0; r < world; ++r) {
+      if (r == rank) b = t;
+      t += all[(size_t)r * m + i];
+    }
+    tot[i] = t;
+    below[i] = b;
+  }
+}
+// the sorted block (packed pairs of the one-sweep sort, or keys / values) -> (column << 32 | Aᵀ position) in sorted order
+__global__ void k_tr_pairs(const u64* __restrict__ sorted, const u32* __restrict__ sk, const u32* __restrict__ sq, size_t cntL, u32 q_lo,
+                           const u32* __restrict__ pos, u32 n, const u32* __restrict__ colptrT, const u32* __restrict__ below,
+                           const u32* __restrict__ lstart, u64* __restrict__ out) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cntL; p += stride) {
+    u32 i, lp;
+    if (sorted) {
+      const u64 v = sorted[p];
+      i = (u32)(v >> 32);
+      lp = (u32)v;
+    } else {
+      i = sk[p];
+      lp = sq[p];
+    }
+    const u32 dst = colptrT[i] + below[i] + ((u32)p - lstart[i]);
+    out[p] = ((u64)column_of(pos, n, q_lo + lp) << 32) | dst;
+  }
+}
+// off[d] = first pair bound for rank d's block or a later one (d = 0..world); counts[d] = off[d + 1] - off[d]
+__global__ void k_tr_slices(const u64* __restrict__ pairs, size_t cntL, u64 cnt, u64 N, int world, u32* __restrict__ off, u32* __restrict__ counts) {
+  __shared__ u32 s[33];
+  const int d = threadIdx.x;
+  if (d <= world) {
+    const u64 t = min(N, (u64)d * cnt);
+    size_t lo = 0, hi = cntL;
+    while (lo < hi) {
+      const size_t mid = lo + ((hi - lo) >> 1);
+      if ((u64)(u32)pairs[mid] < t) lo = mid + 1; else hi = mid;
+    }
+    s[d] = (u32)lo;
+    off[d] = (u32)lo;
+  }
+  __syncthreads();
+  if (d < world && counts) counts[d] = s[d + 1] - s[d];
+}
+__global__ void k_tr_scatter(const u64* __restrict__ pairs, size_t cnt, u32 q_lo, u32* __restrict__ row_blk) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cnt; p += stride) {
+    const u64 v = pairs[p];
+    row_blk[(u32)v - q_lo] = (u32)(v >> 32);
+  }
+}
+
+struct TrBlock {
+  DBuf<u32> k0, v0, k1, v1;
+  DBuf<u64> a, b;
+  const u64* sorted = nullptr;
+  const u32 *sk = nullptr, *sq = nullptr;
+};
+// stable sort of a block by row: the one-sweep passes block_local_links runs, or the tile-histogram sort
+static void tr_sort(const u32* rows, size_t cntL, size_t m, TrBlock& t) {
+  if (!cntL) return;
+  const char* os_env = std::getenv("CPB_ONESWEEP");
+  if (onesweep_supported(cntL) && !(os_env && os_env[0] == '0')) {
+    t.a.alloc(cntL);
+    t.b.alloc(cntL);
+    t.sorted = onesweep_sort_iota(rows, cntL, bits_for(m ? m - 1 : 0), t.a.get(), t.b.get());
+    return;
+  }
+  t.k0.alloc(cntL); t.v0.alloc(cntL); t.k1.alloc(cntL); t.v1.alloc(cntL);
+  const int which = radix_sort_pairs_iota(rows, t.k0.get(), t.v0.get(), t.k1.get(), t.v1.get(), cntL, bits_for(m ? m - 1 : 0));
+  t.sk = which ? t.k1.get() : t.k0.get();
+  t.sq = which ? t.v1.get() : t.v0.get();
+}
+// colptrᵀ (m + 1, 0-based) and the routed pairs of rank `rank`'s sorted block, from every rank's row histogram (all: world x m)
+static void tr_pairs(const Matrix& A, const u32* all, int world, int rank, const TrBlock& t, size_t cntL, u32 q_lo, u32* colptrT, DBuf<u64>& pairs) {
+  const size_t m = (size_t)A.m;
+  DBuf<u32> tot(m + 1), below(std::max<size_t>(m, 1)), lstart(std::max<size_t>(m, 1));
+  tot.zero();
+  if (m) {
+    CPB_LAUNCH(k_tr_combine, grid_for(m), 256, 0, all, m, world, rank, tot.get(), below.get());
+    exclusive_scan_u32(all + (size_t)rank * m, lstart.get(), m);
+  }
+  exclusive_scan_u32(tot.get(), colptrT, m + 1);
+  pairs.alloc(std::max<size_t>(cntL, 1));
+  if (cntL) CPB_LAUNCH(k_tr_pairs, grid_for(cntL), 256, 0, t.sorted, t.sk, t.sq, cntL, q_lo, A.pos.get(), (u32)A.n, colptrT, below.get(), lstart.get(), pairs.get());
+}
+
+ShardedMatrix* sharded_adjointpattern(const ShardedMatrix& S) {
+  CPB_REQUIRE(S.world == g_world && S.rank == g_rank, "the sharded matrix was created under another communicator");
+  const Matrix& A = S.M;
+  const size_t m = (size_t)A.m, cntL = (size_t)(S.q_hi - S.q_lo);
+  const int world = S.world, rank = S.rank;
+  ProfScope prof("shard_adjointpattern", (double)cntL * 16.0 + (double)m * 4.0 * world);
+  auto T = std::make_unique<ShardedMatrix>();
+  T->rank = rank;
+  T->world = world;
+  T->M.m = A.n; T->M.n = A.m; T->M.N = A.N;
+  T->cnt = S.cnt; T->q_lo = S.q_lo; T->q_hi = S.q_hi;
+  T->M.pos.alloc(m + 1);
+  T->row_blk.alloc(std::max<size_t>(cntL, 1));
+  DBuf<u32> all(std::max<size_t>(m, 1) * world);
+  all.zero();
+  u32* const mine = all.get() + (size_t)rank * m;
+  if (cntL) CPB_LAUNCH(k_tr_hist, grid_for(cntL), 256, 0, S.row_blk.get(), cntL, mine);
+  if (world > 1 && m) CPB_NCCL(g_nccl.AllGather(mine, all.get(), m, ncclUint32, g_comm, ctx().stream));
+  TrBlock t;
+  tr_sort(S.row_blk.get(), cntL, m, t);
+  DBuf<u64> pairs;
+  tr_pairs(A, all.get(), world, rank, t, cntL, (u32)S.q_lo, T->M.pos.get(), pairs);
+  if (world == 1) {
+    if (cntL) CPB_LAUNCH(k_tr_scatter, grid_for(cntL), 256, 0, pairs.get(), cntL, 0u, T->row_blk.get());
+    CPB_CUDA(cudaStreamSynchronize(ctx().stream));
+    return T.release();
+  }
+  // world x world pair counts: row s = what rank s sends to every rank
+  DBuf<u32> off((size_t)world + 1), counts((size_t)world * world);
+  CPB_LAUNCH(k_tr_slices, 1, 32, 0, pairs.get(), cntL, (u64)S.cnt, (u64)A.N, world, off.get(), counts.get() + (size_t)rank * world);
+  CPB_NCCL(g_nccl.AllGather(counts.get() + (size_t)rank * world, counts.get(), (size_t)world, ncclUint32, g_comm, ctx().stream));
+  std::vector<u32> h_off((size_t)world + 1), h_cnt((size_t)world * world);
+  CPB_CUDA(cudaMemcpyAsync(h_off.data(), off.get(), h_off.size() * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
+  CPB_CUDA(cudaMemcpyAsync(h_cnt.data(), counts.get(), h_cnt.size() * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
+  CPB_CUDA(cudaStreamSynchronize(ctx().stream));
+  std::vector<size_t> recv_off((size_t)world + 1, 0);
+  for (int s = 0; s < world; ++s) recv_off[s + 1] = recv_off[s] + h_cnt[(size_t)s * world + rank];
+  CPB_REQUIRE(recv_off[world] == cntL, "sharded adjointpattern: the routed slices do not cover this rank's block");
+  DBuf<u64> recv(std::max<size_t>(cntL, 1));
+  {
+    ProfScope pk("shard_transpose_exchange", (double)cntL * 8.0);
+    CPB_NCCL(g_nccl.GroupStart());
+    for (int d = 0; d < world; ++d) {
+      const size_t c = h_cnt[(size_t)rank * world + d];
+      if (d != rank && c) CPB_NCCL(g_nccl.Send(pairs.get() + h_off[d], c, ncclUint64, d, g_comm, ctx().stream));
+    }
+    for (int s = 0; s < world; ++s) {
+      const size_t c = h_cnt[(size_t)s * world + rank];
+      if (s != rank && c) CPB_NCCL(g_nccl.Recv(recv.get() + recv_off[s], c, ncclUint64, s, g_comm, ctx().stream));
+    }
+    CPB_NCCL(g_nccl.GroupEnd());
+  }
+  const size_t self = h_cnt[(size_t)rank * world + rank];
+  if (self)
+    CPB_CUDA(cudaMemcpyAsync(recv.get() + recv_off[rank], pairs.get() + h_off[rank], self * sizeof(u64), cudaMemcpyDeviceToDevice, ctx().stream));
+  if (cntL) CPB_LAUNCH(k_tr_scatter, grid_for(cntL), 256, 0, recv.get(), cntL, (u32)S.q_lo, T->row_blk.get());
+  CPB_CUDA(cudaStreamSynchronize(ctx().stream));  // the exchange buffers are released at the end of this scope
+  g_shard_stats[8] = (double)(cntL - self) * 8.0;  // transpose pairs received from other ranks (bytes, this rank)
+  g_shard_stats[9] = (double)m * 4.0 * world;      // histogram all-gather bytes
+  return T.release();
+}
+
+// The same with the ranks played one after the other on this GPU; assembles the whole Aᵀ (tests)
+std::unique_ptr<Matrix> adjoint_pattern_sharded_emulated(const Matrix& A, int world) {
+  CPB_REQUIRE(world >= 1 && world <= 16, "1..16 emulated ranks");
+  const size_t m = (size_t)A.m, N = (size_t)A.N;
+  i64 cnt = 0;
+  shard_range(A.N, 0, world, &cnt, nullptr, nullptr);
+  auto B = std::make_unique<Matrix>();
+  B->m = A.n; B->n = A.m; B->N = A.N;
+  B->pos.alloc(m + 1);
+  B->row.alloc(N);
+  DBuf<u32> all(std::max<size_t>(m, 1) * world);
+  all.zero();
+  for (int r = 0; r < world; ++r) {
+    i64 lo = 0, hi = 0;
+    shard_range(A.N, r, world, nullptr, &lo, &hi);
+    if (hi > lo) CPB_LAUNCH(k_tr_hist, grid_for((size_t)(hi - lo)), 256, 0, A.row.get() + lo, (size_t)(hi - lo), all.get() + (size_t)r * m);
+  }
+  DBuf<u32> colptrT(m + 1), off((size_t)world + 1);
+  for (int r = 0; r < world; ++r) {
+    i64 lo = 0, hi = 0;
+    shard_range(A.N, r, world, nullptr, &lo, &hi);
+    const size_t cntL = (size_t)(hi - lo);
+    TrBlock t;
+    tr_sort(A.row.get() + lo, cntL, m, t);
+    DBuf<u64> pairs;
+    tr_pairs(A, all.get(), world, r, t, cntL, (u32)lo, r == 0 ? B->pos.get() : colptrT.get(), pairs);
+    // the slices as the destination ranks would receive them
+    CPB_LAUNCH(k_tr_slices, 1, 32, 0, pairs.get(), cntL, (u64)cnt, (u64)N, world, off.get(), (u32*)nullptr);
+    std::vector<u32> h_off((size_t)world + 1);
+    CPB_CUDA(cudaMemcpyAsync(h_off.data(), off.get(), h_off.size() * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
+    CPB_CUDA(cudaStreamSynchronize(ctx().stream));
+    for (int d = 0; d < world; ++d) {
+      i64 dlo = 0;
+      shard_range(A.N, d, world, nullptr, &dlo, nullptr);
+      const size_t c = h_off[d + 1] - h_off[d];
+      if (c) CPB_LAUNCH(k_tr_scatter, grid_for(c), 256, 0, pairs.get() + h_off[d], c, (u32)dlo, B->row.get() + dlo);
+    }
+    CPB_CUDA(cudaStreamSynchronize(ctx().stream));
+  }
+  return B;
+}
+
+// colptr (n + 1) and this rank's block of rowval, both 1-based
+void sharded_get(const ShardedMatrix& S, i64* h_colptr, i64* h_rowval_blk) {
+  const size_t n = (size_t)S.M.n, cntL = (size_t)(S.q_hi - S.q_lo);
+  DBuf<i64> dc(n + 1), dr(std::max<size_t>(cntL, 1));
+  if (h_colptr) {
+    widen_plus(S.M.pos.get(), dc.get(), n + 1, 1);
+    CPB_CUDA(cudaMemcpyAsync(h_colptr, dc.get(), (n + 1) * sizeof(i64), cudaMemcpyDeviceToHost, ctx().stream));
+  }
+  if (h_rowval_blk && cntL) {
+    widen_plus(S.row_blk.get(), dr.get(), cntL, 1);
+    CPB_CUDA(cudaMemcpyAsync(h_rowval_blk, dr.get(), cntL * sizeof(i64), cudaMemcpyDeviceToHost, ctx().stream));
+  }
+  CPB_CUDA(cudaStreamSynchronize(ctx().stream));
 }
 
 void sharded_stats(double out[16]) {

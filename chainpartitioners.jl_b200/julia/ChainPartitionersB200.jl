@@ -301,21 +301,77 @@ end
 init(device::Integer) = check(ccall((:cpb_init, lib), Cint, (Cint,), device))
 comm_init(id::Vector{UInt8}, rank::Integer, world::Integer) = check(ccall((:cpb_comm_init, lib), Cint, (Ptr{UInt8}, Cint, Cint), id, rank, world))
 comm_destroy() = check(ccall((:cpb_comm_destroy, lib), Cint, ()))
-# collective: every rank calls it with the same A; each uploads only its block of rowval
-function partition_stripe_sharded(A::SparseMatrixCSC{Tv, Int64}, K, method::OnB200{<:Union{BisectCostBottleneckSplitter, LazyBisectCostBottleneckSplitter}}) where {Tv}
+# A pattern spread over the ranks (cpb_sharded): the column offsets on every rank, each rank's block of rowval.  Collective:
+# every rank calls it with the same A; each uploads only its block of rowval.  Free it with close_sharded on every rank.
+mutable struct ShardedMatrix
+    h::Ptr{Cvoid}
+    m::Int64
+    n::Int64
+end
+function ShardedMatrix(A::SparseMatrixCSC{Tv, Int64}) where {Tv}
     (m, n) = size(A)
     h = Ref{Ptr{Cvoid}}(C_NULL)
     GC.@preserve A check(ccall((:cpb_sharded_matrix_create, lib), Cint, (Int64, Int64, Int64, Ptr{Int64}, Ptr{Int64}, Cint, Ref{Ptr{Cvoid}}),
                                m, n, nnz(A), A.colptr, A.rowval, 0, h))
+    return ShardedMatrix(h[], m, n)
+end
+function close_sharded(S::ShardedMatrix)
+    S.h == C_NULL || ccall((:cpb_sharded_matrix_destroy, lib), Cvoid, (Ptr{Cvoid},), S.h)
+    S.h = C_NULL
+end
+# adjointpattern of the sharded pattern (collective): the transpose with the same blocks of CSC positions
+function adjointpattern(S::ShardedMatrix)
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:cpb_sharded_adjointpattern, lib), Cint, (Ptr{Cvoid}, Ref{Ptr{Cvoid}}), S.h, h))
+    return ShardedMatrix(h[], S.n, S.m)
+end
+# (colptr, this rank's block of rowval, q_lo, q_hi): 1-based indices, 0-based half-open block of CSC positions
+function host_block(S::ShardedMatrix)
+    lo, hi = Ref{Int64}(0), Ref{Int64}(0)
+    check(ccall((:cpb_sharded_matrix_get, lib), Cint, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}, Ref{Int64}, Ref{Int64}), S.h, C_NULL, C_NULL, lo, hi))
+    colptr, rowval = Vector{Int64}(undef, S.n + 1), Vector{Int64}(undef, hi[] - lo[])
+    check(ccall((:cpb_sharded_matrix_get, lib), Cint, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}, Ptr{Int64}, Ptr{Int64}), S.h, colptr,
+                isempty(rowval) ? C_NULL : pointer(rowval), C_NULL, C_NULL))
+    return (colptr, rowval, lo[], hi[])
+end
+const ShardedSplitter = OnB200{<:Union{BisectCostBottleneckSplitter, LazyBisectCostBottleneckSplitter}}
+# collective: ONE stripe solve over all ranks, AffineConnectivityModel or AffineMonotonizedSymmetricConnectivityModel (square
+# A); the library refuses any other model on every rank alike
+function partition_stripe_sharded(S::ShardedMatrix, K, method::ShardedSplitter, args...)
     (code, ϵ) = split_code(method.mtd)
     (cm, keep) = cmodel(method.mtd.f, 0, 0)
     spl = Vector{Int64}(undef, K + 1)
-    try
-        GC.@preserve keep check(ccall((:cpb_partition_stripe_sharded, lib), Cint, (Ptr{Cvoid}, Ref{CModel}, Cint, Float64, Int64, Ptr{Int64}), h[], cm, code, ϵ, K, spl))
-    finally
-        ccall((:cpb_sharded_matrix_destroy, lib), Cvoid, (Ptr{Cvoid},), h[])
-    end
+    GC.@preserve keep check(ccall((:cpb_partition_stripe_sharded, lib), Cint, (Ptr{Cvoid}, Ref{CModel}, Cint, Float64, Int64, Ptr{Int64}), S.h, cm, code, ϵ, K, spl))
     return SplitPartition{Int64}(K, spl)
+end
+function partition_stripe_sharded(A::SparseMatrixCSC{Tv, Int64}, K, method::ShardedSplitter) where {Tv}
+    S = ShardedMatrix(A)
+    try
+        return partition_stripe_sharded(S, K, method)
+    finally
+        close_sharded(S)
+    end
+end
+# partition_plaid(A, K, AlternatingPartitioner(...)) (src/AlternatingPartitioner.jl:18-32) with every stripe solve sharded
+# over the ranks; the transpose is built once (cpb_sharded_adjointpattern) unless adj_A is given.  Collective.
+function partition_plaid_sharded(A::Union{SparseMatrixCSC, ShardedMatrix}, K, method::AlternatingPartitioner{<:Tuple{Vararg{ShardedSplitter}}}; adj_A = nothing)
+    S = A isa ShardedMatrix ? A : ShardedMatrix(A)
+    T = adj_A === nothing ? adjointpattern(S) : (adj_A isa ShardedMatrix ? adj_A : ShardedMatrix(adj_A))
+    try
+        Φ = partition_stripe_sharded(S, K, method.mtds[1])
+        Π = partition_stripe_sharded(T, K, method.mtds[2])
+        for (i, mtd) in enumerate(method.mtds[3:end])
+            if isodd(i)
+                Φ = partition_stripe_sharded(S, K, mtd)
+            else
+                Π = partition_stripe_sharded(T, K, mtd)
+            end
+        end
+        return (Π, Φ)
+    finally
+        T === adj_A || close_sharded(T)
+        S === A || close_sharded(S)
+    end
 end
 
 function partition_stripe(A::SparseMatrixCSC{Tv, Int64}, K, method::OnB200, args...; kwargs...) where {Tv}

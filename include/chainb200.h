@@ -252,15 +252,27 @@ int cpb_bisect_stats(double out[8]);
  * cpb_sharded_matrix_create: every rank passes the complete colptr; of rowval only the rank's block of CSC positions
  * [q_lo, q_hi) (cpb_shard_range) is read and uploaded -- pass the whole array (rowval_is_block = 0) or just the block
  * (rowval_is_block = 1, rowval[0] = entry q_lo).
- * cpb_partition_stripe_sharded: BisectCost / LazyBisectCost with the AffineConnectivityModel.  Link construction by
- * blocks of CSC positions: local stable sort by row, the per-row "last position" array (m x 4 bytes) carried down the ranks
- * once (ncclSend/Recv), one in-place all-gather of the link shards (nnz x 4 bytes); bisection rounds of world x 15
- * thresholds, rank r probing its 15, one all-gather of the per-threshold results per round.  Every rank returns the same
- * split vector -- the single-GPU (and the reference's) one.
+ * cpb_partition_stripe_sharded: BisectCost / LazyBisectCost with the AffineConnectivityModel or the
+ * AffineMonotonizedSymmetricConnectivityModel (square A).  Link construction by blocks of CSC positions: local stable sort
+ * by row, the per-row "last position" array (m x 4 bytes) carried down the ranks once (ncclSend/Recv), one in-place
+ * all-gather of the link shards (nnz x 4 bytes); bisection rounds of world x 15 thresholds, rank r probing its 15, one
+ * all-gather of the per-threshold results per round.  Every rank returns the same split vector -- the single-GPU (and the
+ * reference's) one.  The monotonized symmetric model streams the links of A + I: the ranks combine their "diagonal present"
+ * flags (one n-byte MAX all-reduce), every rank's block becomes [img(q_lo), img(q_hi)) of A + I positions (a virtual diagonal
+ * goes with the last element of its column, rank 0 starts at 0), and one in-place broadcast per rank gathers the blocks.
  * cpb_partition_stripe_sharded_emulated plays `world` ranks one after the other on this GPU (tests; no NCCL).
+ * cpb_sharded_adjointpattern: adjointpattern (util.jl:67-95) of a sharded matrix, collective; the result holds the complete
+ * colptr of the transpose and this rank's block of its rowval (the same cpb_shard_range blocks: nnz is unchanged).  Row
+ * histograms of the blocks are all-gathered (m x 4 bytes per rank), each entry is routed to the rank owning its position in
+ * the transpose with grouped ncclSend/Recv (8 bytes per nonzero).  Rectangular patterns are fine.
+ * cpb_adjointpattern_sharded_emulated: the same construction with `world` ranks played on this GPU, assembled into one
+ * whole matrix (tests).
+ * cpb_sharded_matrix_get: the 1-based colptr (n + 1 entries) and this rank's block of rowval (q_hi - q_lo entries, 1-based),
+ * and the 0-based half-open block [q_lo, q_hi) of CSC positions; any output may be NULL.
  * cpb_sharded_stats: out[0] = world, [1] = host ms until the construction was queued, [2] = ms of the bisection (incl.
- * waiting for the construction), [3] = bisection rounds, [4] = link all-gather bytes, [5] = carry bytes per hop,
- * [6] = threshold all-gather bytes, [7] = thresholds per round. */
+ * waiting for the construction), [3] = bisection rounds, [4] = link gather bytes (of A + I for the monotonized symmetric
+ * model), [5] = carry bytes per hop, [6] = threshold all-gather bytes, [7] = thresholds per round, [8] = bytes of transpose
+ * pairs this rank received from other ranks in its last cpb_sharded_adjointpattern, [9] = its histogram all-gather bytes. */
 typedef struct cpb_sharded cpb_sharded;
 int cpb_comm_unique_id(char id_out[128]);
 int cpb_comm_init(const char id[128], int rank, int world);
@@ -273,6 +285,9 @@ void cpb_sharded_matrix_destroy(cpb_sharded* A);
 int cpb_partition_stripe_sharded(cpb_sharded* A, const cpb_model* mdl, int method, double eps, int64_t K, int64_t* spl_out);
 int cpb_partition_stripe_sharded_emulated(cpb_matrix* A, const cpb_model* mdl, int method, double eps, int64_t K, int world,
                                           int64_t* spl_out);
+int cpb_sharded_adjointpattern(cpb_sharded* A, cpb_sharded** out);
+int cpb_adjointpattern_sharded_emulated(cpb_matrix* A, int world, cpb_matrix** out);
+int cpb_sharded_matrix_get(const cpb_sharded* A, int64_t* colptr_out, int64_t* rowval_block_out, int64_t* q_lo, int64_t* q_hi);
 int cpb_sharded_stats(double out[16]);
 
 /* ---- pack_stripe ------------------------------------------------------------------------- */
