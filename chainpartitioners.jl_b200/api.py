@@ -22,7 +22,7 @@ __all__ = [
     "dianetcount", "selfnetcount", "selfpincount", "PrefixMatrix", "dominancecount", "dominancesum", "rookcount", "rooksum", "profile_enable", "profile_reset", "profile_get",
     "Communicator", "ShardedMatrix", "partition_stripe_sharded", "partition_stripe_sharded_emulated", "sharded_stats", "shard_range",
     "partition_plaid_sharded", "partition_plaid_sharded_emulated", "adjointpattern_sharded_emulated",
-    "launch_count", "probe_cluster_capacity", "bisect_stats", "bisect_plan", "bisect_prewalk", "timer_start", "timer_stop", "StepwiseBisection", "StripeOracle", "init", "synchronize", "trim_memory", "library_path", "load_library", "CpbError",
+    "weight_windows", "launch_count", "probe_cluster_capacity", "bisect_stats", "bisect_plan", "bisect_prewalk", "timer_start", "timer_stop", "StepwiseBisection", "StripeOracle", "init", "synchronize", "trim_memory", "library_path", "load_library", "CpbError",
 ]
 
 I64 = np.int64
@@ -41,6 +41,7 @@ ABI_SYMBOLS = [
     "cpb_partition_stripe_sharded", "cpb_partition_stripe_sharded_emulated", "cpb_sharded_stats",
     "cpb_sharded_adjointpattern", "cpb_adjointpattern_sharded_emulated", "cpb_sharded_matrix_get",
     "cpb_links_partial", "cpb_oracle_set_links", "cpb_prefix_create", "cpb_prefix_query", "cpb_prefix_destroy", "cpb_matrix_permute", "cpb_trim_memory", "cpb_matrix_create_i32",
+    "cpb_partition_stripe_weighted", "cpb_weight_windows",
 ]
 
 
@@ -83,6 +84,8 @@ def load_library():
         lib.cpb_bound_stripe.argtypes = [vp, i64, ctypes.POINTER(dbl)]
         lib.cpb_objective.argtypes = [vp, i32, i64, vp, ctypes.POINTER(dbl)]
         lib.cpb_partition_stripe.argtypes = [vp, i32, ctypes.POINTER(T.CConstraint), dbl, i64, vp]
+        lib.cpb_partition_stripe_weighted.argtypes = [vp, i32, vp, i64, dbl, i64, vp]
+        lib.cpb_weight_windows.argtypes = [vp, i64, vp, vp]
         lib.cpb_pack_stripe.argtypes = [vp, vp, i32, ctypes.POINTER(T.CConstraint), dbl, i64, vp, ctypes.POINTER(i64), vp]
         lib.cpb_profile_get.argtypes = [i32, vp, vp, vp, vp]
         lib.cpb_bisect_begin.argtypes = [vp, i32, dbl, i64, i32, vp, vp, vp, ctypes.POINTER(vp)]
@@ -336,12 +339,24 @@ def _pi(Pi):
 
 
 class StripeOracle:
-    """``oracle_stripe(hint, mdl, A[, Pi])``: callable ``ocl(j, j'[, k])``; arrays are batched on the GPU."""
+    """``oracle_stripe(hint, mdl, A[, Pi])``: callable ``ocl(j, j'[, k])``; arrays are batched on the GPU.  For
+    ``ConstrainedCost(f, w, w_max)`` with a count weight ``w`` (``ConstrainedCost.count_weight``), ``weight`` is a second
+    oracle: ``w``'s own, on the same device matrix (its own wavelet index)."""
 
     def __init__(self, mdl, A, Pi=None, hint=None, w_tab=None):
-        f, con = T.split_constrained(mdl)
+        self.weight, self.w_max = None, None
+        wmdl = mdl.count_weight() if isinstance(mdl, T.ConstrainedCost) else None
+        if wmdl is not None:
+            f, con = mdl.f, T.CConstraint()
+            self.w_max = int(mdl.w_max)
+        else:
+            f, con = T.split_constrained(mdl)
         self.model, self.constraint = f, con
+        self._h = None
         if Pi is not None and not isinstance(Pi, T.SplitPartition):
+            if wmdl is not None and wmdl.kind == T.MODEL_MONOSYM:
+                # the rows are renamed part by part below: the diagonal the weight counts would move
+                raise TypeError("a monotonized-symmetric weight needs a SplitPartition of the rows (renaming the rows moves the diagonal)")
             # oracle_stripe converts any row partition to a MapPartition (PrimaryConnectivityCosts.jl:56-67); the device
             # structures want contiguous row parts, and the counts depend on a row only through its part: rename the rows
             row_new, Pi = _rows_by_part(Pi, A.m)
@@ -359,6 +374,8 @@ class StripeOracle:
         spl, pK = _pi(Pi)
         self._h = ctypes.c_void_p()
         _check(load_library().cpb_oracle_create(self.dm._h, ctypes.byref(cm), _p(spl), pK, ctypes.byref(self._h)))
+        if wmdl is not None:
+            self.weight = StripeOracle(wmdl, self.dm)
 
     def query(self, j, jp, k=None) -> np.ndarray:
         j, jp = _arr(np.atleast_1d(j)), _arr(np.atleast_1d(jp))
@@ -375,7 +392,17 @@ class StripeOracle:
                 dm_pos = self.dm.to_host().colptr
                 width = width + (dm_pos[jp - 1] - dm_pos[j - 1]) * w[2]
             out = np.where(width <= self.constraint.w_max, out, np.inf)
+        if self.weight is not None:  # the same with the weight model's own oracle
+            out = np.where(self.weight.query(j, jp) <= self.w_max, out, np.inf)
         return out
+
+    def weight_windows(self):
+        """``(first_fit, reach)`` of the count weight, 1-based, ``n + 1`` entries each (index ``c - 1`` is column ``c``):
+        ``first_fit[j'-1]`` = smallest ``j <= j'`` with ``j == j'`` or ``w(j, j') <= w_max``, ``reach[j-1]`` = largest
+        ``j' >= j`` with ``j' == j`` or ``w(j, j') <= w_max``."""
+        if self.weight is None:
+            raise TypeError("weight_windows needs a ConstrainedCost with a count weight")
+        return weight_windows(self.weight, self.w_max)
 
     def links_partial(self, row_lo: int, row_hi: int, d_prev: int) -> int:
         """Multi-GPU link construction: links of the nonzeros with row in [row_lo, row_hi) into the device buffer
@@ -399,10 +426,13 @@ class StripeOracle:
         return r
 
     def close(self):
-        if self._h is not None and _lib is not None:
+        if getattr(self, "weight", None) is not None:
+            self.weight.close()
+            self.weight = None
+        if getattr(self, "_h", None) is not None and _lib is not None:
             _lib.cpb_oracle_destroy(self._h)
         self._h = None
-        if self._own is not None:
+        if getattr(self, "_own", None) is not None:
             self._own.__exit__()
             self._own = None
 
@@ -411,6 +441,14 @@ class StripeOracle:
             self.close()
         except Exception:
             pass
+
+
+def weight_windows(w: StripeOracle, w_max: int):
+    """``cpb_weight_windows``: the windows of the weight oracle ``w`` under ``w_max`` (see ``StripeOracle.weight_windows``)."""
+    n1 = w.dm.n + 1
+    first_fit, reach = np.empty(n1, dtype=I64), np.empty(n1, dtype=I64)
+    _check(load_library().cpb_weight_windows(w._h, int(w_max), _p(first_fit), _p(reach)))
+    return first_fit, reach
 
 
 def oracle_stripe(*args, **kwargs) -> StripeOracle:
@@ -533,7 +571,10 @@ def partition_stripe(A, K, method, Pi=None, **kwargs) -> T.SplitPartition:
             spec = T.AffineWorkModel(0, 0, 0)
         ocl = StripeOracle(spec, dm, Pi)
         try:
-            _check(load_library().cpb_partition_stripe(ocl._h, code, ctypes.byref(ocl.constraint), eps, K, _p(spl)))
+            if ocl.weight is not None:  # ConstrainedCost with a count weight
+                _check(load_library().cpb_partition_stripe_weighted(ocl._h, code, ocl.weight._h, ocl.w_max, eps, K, _p(spl)))
+            else:
+                _check(load_library().cpb_partition_stripe(ocl._h, code, ctypes.byref(ocl.constraint), eps, K, _p(spl)))
         finally:
             ocl.close()
     return T.SplitPartition(K, spl)
@@ -553,6 +594,9 @@ def _scratch(name: str, count: int) -> np.ndarray:
 def pack_stripe(A, method, Pi=None, n_nets=None, **kwargs) -> T.SplitPartition:
     """``pack_stripe(A, method[, Pi]; kwargs...)`` -> ``SplitPartition(K, spl)`` with a free number of chunks."""
     code, spec, rho, w_max = T.pack_method_code(method)
+    if isinstance(spec, T.ConstrainedCost) and spec.count_weight() is not None:
+        raise TypeError("pack_stripe takes VertexCount() or an integer AffineWorkModel as the weight: count weights "
+                        "(AffineConnectivityModel / AffineMonotonizedSymmetricConnectivityModel) are not built for the chunkers")
     with _Scoped(A) as dm:
         # the ABI wants room for the worst case (n + 1 boundaries): reuse one scratch array across calls instead of
         # faulting in tens of megabytes per call

@@ -581,13 +581,8 @@ int cpb_objective(cpb_oracle* f, int total, int64_t K, const int64_t* spl, doubl
   CPB_API_END
 }
 
-int cpb_partition_stripe(cpb_oracle* f, int method, const cpb_constraint* con, double eps, int64_t K, int64_t* spl_out) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(f && spl_out, "NULL argument");
-  CPB_REQUIRE(K >= 1, "K must be >= 1");
-  trace_mark("enter");
-  struct TraceEnd { ~TraceEnd() { trace_mark("exit"); trace_flush("partition_stripe"); } } trace_end;
+// partition_stripe's method dispatch (the caller holds the library lock)
+static void partition_stripe_impl(cpb_oracle* f, int method, const cpb_constraint* con, double eps, int64_t K, int64_t* spl_out) {
   if ((method == CPB_SPLIT_DYNAMIC_BOTTLENECK_CHUNKER || method == CPB_SPLIT_DYNAMIC_TOTAL_CHUNKER) && f->O->mdl.kind >= CPB_MODEL_PRIMCONN &&
       f->O->mdl.kind <= CPB_MODEL_SECEDGE)
     // the chunker-form K-DP calls f(j, j') without a part index (DynamicSplitter.jl:62-71, 290-301): a MethodError for the
@@ -610,6 +605,67 @@ int cpb_partition_stripe(cpb_oracle* f, int method, const cpb_constraint* con, d
       break;
     }
     default: throw Error(CPB_ERR_UNSUPPORTED, "unsupported partition_stripe method");
+  }
+}
+
+int cpb_partition_stripe(cpb_oracle* f, int method, const cpb_constraint* con, double eps, int64_t K, int64_t* spl_out) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(f && spl_out, "NULL argument");
+  CPB_REQUIRE(K >= 1, "K must be >= 1");
+  trace_mark("enter");
+  struct TraceEnd { ~TraceEnd() { trace_mark("exit"); trace_flush("partition_stripe"); } } trace_end;
+  partition_stripe_impl(f, method, con, eps, K, spl_out);
+  CPB_API_END
+}
+
+int cpb_partition_stripe_weighted(cpb_oracle* f, int method, cpb_oracle* w, int64_t w_max, double eps, int64_t K, int64_t* spl_out) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(f && w && spl_out, "NULL argument");
+  CPB_REQUIRE(K >= 1, "K must be >= 1");
+  CPB_REQUIRE(f->O->A == w->O->A, "the weight oracle must be built on the same cpb_matrix as the cost oracle");
+  trace_mark("enter");
+  struct TraceEnd { ~TraceEnd() { trace_mark("exit"); trace_flush("partition_stripe_weighted"); } } trace_end;
+  if (method != CPB_SPLIT_DYNAMIC_BOTTLENECK && method != CPB_SPLIT_DYNAMIC_TOTAL && method != CPB_SPLIT_DYNAMIC_BOTTLENECK_CHUNKER &&
+      method != CPB_SPLIT_DYNAMIC_TOTAL_CHUNKER && method != CPB_SPLIT_CONVEX_TOTAL && method != CPB_SPLIT_CONCAVE_TOTAL)
+    throw Error(CPB_ERR_UNSUPPORTED, "a weight constraint is taken by the Dynamic, Convex and Concave total splitters only");
+  weight_check(*w->O);
+  if (w->O->mdl.kind == CPB_MODEL_WORK) {  // an affine work weight: the cpb_constraint path, one implementation of its windows
+    cpb_constraint con{};
+    con.enabled = 1;
+    for (int t = 0; t < 3; ++t) con.w_coef[t] = (int64_t)w->O->mdl.coef[t];
+    con.w_max = w_max;
+    partition_stripe_impl(f, method, &con, eps, K, spl_out);
+    return CPB_OK;
+  }
+  if ((method == CPB_SPLIT_DYNAMIC_BOTTLENECK_CHUNKER || method == CPB_SPLIT_DYNAMIC_TOTAL_CHUNKER) && f->O->mdl.kind >= CPB_MODEL_PRIMCONN &&
+      f->O->mdl.kind <= CPB_MODEL_SECEDGE)
+    throw Error(CPB_ERR_UNSUPPORTED, "the chunker-form K-DP has no method for the row-partition-aware cost models (the reference calls f(j, j') without k)");
+  switch (method) {
+    case CPB_SPLIT_DYNAMIC_BOTTLENECK: case CPB_SPLIT_DYNAMIC_BOTTLENECK_CHUNKER: solve_dynamic_weighted(*f->O, false, *w->O, w_max, K, spl_out); break;
+    case CPB_SPLIT_DYNAMIC_TOTAL: case CPB_SPLIT_DYNAMIC_TOTAL_CHUNKER: solve_dynamic_weighted(*f->O, true, *w->O, w_max, K, spl_out); break;
+    case CPB_SPLIT_CONVEX_TOTAL: solve_convex_weighted(*f->O, *w->O, w_max, K, spl_out); break;
+    case CPB_SPLIT_CONCAVE_TOTAL: solve_concave_weighted(*f->O, *w->O, w_max, K, spl_out); break;
+    default: throw Error(CPB_ERR_UNSUPPORTED, "a weight constraint is taken by the Dynamic, Convex and Concave total splitters only");
+  }
+  CPB_API_END
+}
+
+int cpb_weight_windows(cpb_oracle* w, int64_t w_max, int64_t* first_fit_out, int64_t* reach_out) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(w && first_fit_out && reach_out, "NULL argument");
+  DBuf<u32> ff, rc;
+  weight_windows(*w->O, w_max, ff, &rc);
+  const size_t n1 = (size_t)w->O->A->n + 1;
+  std::vector<u32> h(2 * n1);
+  CPB_CUDA(cudaMemcpyAsync(h.data(), ff.get() + 1, n1 * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
+  CPB_CUDA(cudaMemcpyAsync(h.data() + n1, rc.get() + 1, n1 * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
+  CPB_CUDA(cudaStreamSynchronize(ctx().stream));
+  for (size_t c = 0; c < n1; ++c) {
+    first_fit_out[c] = h[c];
+    reach_out[c] = h[n1 + c];
   }
   CPB_API_END
 }

@@ -161,51 +161,16 @@ __global__ void k_concave_unravel(const u32* __restrict__ ptr, u32 n2, int K, u3
 }
 
 // partition_stripe(A, K, ConcaveTotalSplitter(f)) (:26-55) and its ConstrainedCost form (:143-181)
-template <class T> static void concave_splitter_T(Oracle& f, const cpb_constraint* con, i64 K, int64_t* h_spl_out) {
+template <class T> static void concave_splitter_T(Oracle& f, const Windows* win, i64 K, int64_t* h_spl_out) {
   const Matrix& A = *f.A;
   const i64 n = A.n;
   const u32 n1 = (u32)n + 1, n2 = n1 + 1;
   std::vector<i64> lo(K + 1, 1), hi(K + 1, n + 1);
-  const bool windowed = con && con->enabled;
+  const bool windowed = win != nullptr;
   if (windowed) {
-    if (!(con->w_coef[1] >= 0 && con->w_coef[2] >= 0 && con->w_coef[1] + con->w_coef[2] >= 1 && con->w_coef[0] >= 0))
-      throw Error(CPB_ERR_UNSUPPORTED, "constrained splitters on the device need a weight that grows with the part (VertexCount or "
-                                       "AffineWorkModel(a >= 0, b_v >= 0, b_p >= 0) with b_v + b_p >= 1)");
-    const i64 wa = con->w_coef[0], wbv = con->w_coef[1], wbp = con->w_coef[2], w_max = con->w_max;
-    std::vector<u32> hpos;
-    if (wbp != 0) {
-      hpos.resize((size_t)n + 1);
-      CPB_CUDA(cudaMemcpyAsync(hpos.data(), A.pos.get(), ((size_t)n + 1) * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
-      CPB_CUDA(cudaStreamSynchronize(ctx().stream));
-    }
-    auto fits = [&](i64 j, i64 jp) {
-      i64 w = wa + (jp - j) * wbv;
-      if (wbp != 0) w += ((i64)hpos[jp - 1] - (i64)hpos[j - 1]) * wbp;
-      return w <= w_max;
-    };
-    // column_constraints (DynamicSplitter.jl:144-173); the reference's linear walks are binary searches (w is monotone)
-    for (i64 k = K, jp = n + 1; k >= 1; --k) {
-      lo[k] = jp;
-      i64 a = 1, b = jp;
-      while (a < b) {
-        const i64 mid = a + (b - a) / 2;
-        if (fits(mid, jp)) b = mid; else a = mid + 1;
-      }
-      jp = a;
-    }
-    for (i64 k = 1, j = 1; k <= K; ++k) {
-      i64 a = j, b = n + 1;
-      while (a < b) {
-        const i64 mid = a + (b - a + 1) / 2;
-        if (fits(j, mid)) a = mid; else b = mid - 1;
-      }
-      hi[k] = a;
-      j = a;
-    }
-    if (wa > w_max) { for (i64 k = 1; k <= K; ++k) hi[k] = 1; }
-    if (hi[K] < n + 1) {  // :153-158 infeasible -> degenerate partition
-      for (i64 k = 0; k < K; ++k) h_spl_out[k] = 1;
-      h_spl_out[K] = n + 1;
+    // column_constraints (DynamicSplitter.jl:144-173); the weight shapes nothing but the windows
+    if (!column_constraints(*win, n, K, lo, hi)) {  // :153-158 infeasible -> degenerate partition
+      degenerate_partition(n, K, h_spl_out);
       return;
     }
   } else if (K == 1) {  // :33-35
@@ -257,8 +222,19 @@ void solve_concave_chunker(Oracle& f, const cpb_constraint* con, int64_t* h_spl_
 void solve_concave_splitter(Oracle& f, const cpb_constraint* con, i64 K, int64_t* h_spl_out) {
   CPB_REQUIRE(K >= 1, "K must be >= 1");
   concave_check_model(f);
+  Windows win;
+  if (con && con->enabled) win = windows_affine(*f.A, con);
+  const Windows* pw = (con && con->enabled) ? &win : nullptr;
   oracle_ensure_ranks(f);
-  if (f.dev.is_float) concave_splitter_T<double>(f, con, K, h_spl_out); else concave_splitter_T<i64>(f, con, K, h_spl_out);
+  if (f.dev.is_float) concave_splitter_T<double>(f, pw, K, h_spl_out); else concave_splitter_T<i64>(f, pw, K, h_spl_out);
+}
+
+void solve_concave_weighted(Oracle& f, Oracle& w, i64 w_max, i64 K, int64_t* h_spl_out) {
+  CPB_REQUIRE(K >= 1, "K must be >= 1");
+  concave_check_model(f);
+  const Windows win = windows_weighted(w, w_max);
+  oracle_ensure_ranks(f);
+  if (f.dev.is_float) concave_splitter_T<double>(f, &win, K, h_spl_out); else concave_splitter_T<i64>(f, &win, K, h_spl_out);
 }
 
 }  // namespace cpb

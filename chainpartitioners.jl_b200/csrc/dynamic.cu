@@ -175,9 +175,11 @@ __global__ void __launch_bounds__(256) k_dp_total_dc(const __grid_constant__ Dev
 // weight-constrained layer (DynamicSplitter.jl:206-247) for weights w(j, j') = a + b_v (j' - j) + b_p (pos[j'] - pos[j])
 // with b_v, b_p >= 0: the feasible predecessors of j' are the window [max(lo_prev, j0(j')), min(j', hi_prev)], j0(j') the
 // smallest j with w(j, j') <= w_max (the reference advances j0 monotonically, :231-233; here a binary search, or
-// j' - W when there is no pin term); rightmost argmin (`<=`).
+// j' - W when there is no pin term); rightmost argmin (`<=`).  A count weight (weights.cu) hands j0(j') over as the window
+// array first_fit (nullptr: the affine weight).
 struct DevWeight {
   i64 a, bv, bp, w_max;
+  const u32* first_fit;
 };
 __device__ __forceinline__ bool weight_ok(const DevOracle& o, const DevWeight& w, u32 j, u32 jp) {
   return w.a + (i64)(jp - j) * w.bv + ((i64)__ldg(o.pos + (jp - 1)) - (i64)__ldg(o.pos + (j - 1))) * w.bp <= w.w_max;
@@ -196,7 +198,9 @@ __global__ void __launch_bounds__(256) k_dp_constrained(const __grid_constant__ 
     }
     u32 j0 = max(lo_p, jp > W ? jp - W : 1u);
     const u32 j1 = min(jp, hi_p);
-    if (wt.bp != 0) {  // smallest j in [j0, jp] with w(j, j') <= w_max (w shrinks as j grows)
+    if (wt.first_fit) {
+      j0 = max(j0, __ldg(wt.first_fit + jp));
+    } else if (wt.bp != 0) {  // smallest j in [j0, jp] with w(j, j') <= w_max (w shrinks as j grows)
       u32 a = j0, b = jp;
       while (a < b) {
         const u32 mid = a + ((b - a) >> 1);
@@ -228,7 +232,9 @@ __global__ void __launch_bounds__(256) k_dp_constrained_warp(const __grid_consta
     const u32 jp = (u32)t;
     u32 j0 = max(lo_p, jp > W ? jp - W : 1u);
     const u32 j1 = min(jp, hi_p);
-    if (wt.bp != 0) {
+    if (wt.first_fit) {
+      j0 = max(j0, __ldg(wt.first_fit + jp));
+    } else if (wt.bp != 0) {
       u32 a = j0, b = jp;
       while (a < b) {
         const u32 mid = a + ((b - a) >> 1);
@@ -315,53 +321,16 @@ template <class T, int TIE> static void dynamic_T(Oracle& f, bool total, i64 K, 
   CPB_CUDA(cudaStreamSynchronize(ctx().stream));
 }
 
-template <class T> static void dynamic_constrained_T(Oracle& f, bool total, const cpb_constraint* con, i64 K, int64_t* h_spl_out) {
+template <class T> static void dynamic_constrained_T(Oracle& f, bool total, const Windows& win, i64 K, int64_t* h_spl_out) {
   const Matrix& A = *f.A;
   const i64 n = A.n;
-  if (!(con->w_coef[1] >= 0 && con->w_coef[2] >= 0 && con->w_coef[1] + con->w_coef[2] >= 1 && con->w_coef[0] >= 0))
-    throw Error(CPB_ERR_UNSUPPORTED, "constrained dynamic splitters on the device need a weight that grows with the part (VertexCount or "
-                                     "AffineWorkModel(a >= 0, b_v >= 0, b_p >= 0) with b_v + b_p >= 1)");
-  const i64 wa = con->w_coef[0], wbv = con->w_coef[1], wbp = con->w_coef[2], w_max = con->w_max;
-  // widest part the vertex term alone allows (no pin term: exactly the window; with a pin term: an upper bound)
-  const i64 W = wbv > 0 ? (w_max - wa) / wbv : n;
-  // column_constraints (DynamicSplitter.jl:144-173): greedy chains from both ends.  The `while` loops of the reference
-  // are binary searches here because w is monotone in both arguments.
-  std::vector<u32> hpos;
-  if (wbp != 0) {
-    hpos.resize((size_t)n + 1);
-    CPB_CUDA(cudaMemcpyAsync(hpos.data(), A.pos.get(), ((size_t)n + 1) * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
-    CPB_CUDA(cudaStreamSynchronize(ctx().stream));
-  }
-  auto fits = [&](i64 j, i64 jp) {  // w(j, j') <= w_max, 1-based
-    i64 w = wa + (jp - j) * wbv;
-    if (wbp != 0) w += ((i64)hpos[jp - 1] - (i64)hpos[j - 1]) * wbp;
-    return w <= w_max;
-  };
-  std::vector<i64> lo(K + 1), hi(K + 1);
-  for (i64 k = K, jp = n + 1; k >= 1; --k) {
-    lo[k] = jp;
-    i64 a = 1, b = jp;  // smallest j in [1, jp] that fits (j = jp always "fits" in the reference's loop: it never tests it)
-    while (a < b) {
-      const i64 mid = a + (b - a) / 2;
-      if (fits(mid, jp)) b = mid; else a = mid + 1;
-    }
-    jp = a;
-  }
-  for (i64 k = 1, j = 1; k <= K; ++k) {
-    i64 a = j, b = n + 1;  // largest jp in [j, n + 1] that fits (jp = j is never tested by the reference either)
-    while (a < b) {
-      const i64 mid = a + (b - a + 1) / 2;
-      if (fits(j, mid)) a = mid; else b = mid - 1;
-    }
-    hi[k] = a;
-    j = a;
-  }
-  if (wa > w_max) { for (i64 k = 1; k <= K; ++k) hi[k] = 1; }  // not even the empty part is feasible
-  if (hi[K] < n + 1) {  // :217-222 infeasible -> degenerate partition
-    for (i64 k = 0; k < K; ++k) h_spl_out[k] = 1;
-    h_spl_out[K] = n + 1;
+  std::vector<i64> lo, hi;
+  if (!column_constraints(win, n, K, lo, hi)) {  // :217-222 infeasible -> degenerate partition
+    degenerate_partition(n, K, h_spl_out);
     return;
   }
+  const i64 W = win.W;
+  const DevWeight dw{win.a, win.bv, win.bp, win.w_max, win.first_fit.get()};
   const u32 n1 = (u32)n + 1, n2 = n1 + 1;
   ProfScope prof("dp_layer");
   DBuf<T> rowa(n2), rowb(n2);
@@ -377,11 +346,11 @@ template <class T> static void dynamic_constrained_T(Oracle& f, bool total, cons
     if (wide) {
       const unsigned wgrid = (unsigned)std::max<size_t>(1, std::min<size_t>((cnt * 32 + 255) / 256, (size_t)ctx().sm_count * 16));
       CPB_LAUNCH(k_dp_constrained_warp<T>, wgrid, 256, 0, f.dev, prev, cur, ptr.get() + (size_t)(k - 1) * n2, total ? 1 : 0, (u32)lo[k], (u32)hi[k],
-                 (u32)lo[k - 1], (u32)hi[k - 1], (u32)std::min<i64>(std::max<i64>(W, 0), n + 1), DevWeight{wa, wbv, wbp, w_max}, (u32)k);
+                 (u32)lo[k - 1], (u32)hi[k - 1], (u32)std::min<i64>(std::max<i64>(W, 0), n + 1), dw, (u32)k);
     } else {
       CPB_LAUNCH(k_dp_constrained<T>, grid, 256, 0, f.dev, prev, cur, ptr.get() + (size_t)(k - 1) * n2, total ? 1 : 0, (u32)lo[k], (u32)hi[k],
                  (u32)(k > 1 ? lo[k - 1] : 1), (u32)(k > 1 ? hi[k - 1] : 1), (u32)std::min<i64>(std::max<i64>(W, 0), n + 1), k == 1 ? 1 : 0,
-                 DevWeight{wa, wbv, wbp, w_max}, (u32)k);
+                 dw, (u32)k);
     }
     std::swap(prev, cur);
   }
@@ -431,7 +400,9 @@ __global__ void __launch_bounds__(256) k_dp_convex_constrained(const __grid_cons
       if (a > 0) {  // staircase pass: rightmost minimiser among the previous block's columns that still fit; replaces the initialisation
         u32 lo_j = __ldg(blk + a - 1) + 1;
         const u32 hi_j = min(j0, hi_p);
-        {
+        if (wt.first_fit) {  // the same smallest fitting j, read from the window array
+          lo_j = max(max(lo_j, __ldg(wt.first_fit + jp)), lo_p);
+        } else {
           u32 x = lo_j, y = j0;  // smallest j in [lo_j, j0] with w(j, j') <= w_max (j0 itself fits: j' lies in its block)
           while (x < y) {
             const u32 mid = x + ((y - x) >> 1);
@@ -480,58 +451,15 @@ __global__ void __launch_bounds__(256) k_dp_convex_constrained(const __grid_cons
   }
 }
 
-template <class T> static void convex_constrained_T(Oracle& f, const cpb_constraint* con, i64 K, int64_t* h_spl_out) {
+template <class T> static void convex_constrained_T(Oracle& f, const Windows& win, i64 K, int64_t* h_spl_out) {
   const Matrix& A = *f.A;
   const i64 n = A.n;
-  if (!(con->w_coef[1] >= 0 && con->w_coef[2] >= 0 && con->w_coef[1] + con->w_coef[2] >= 1 && con->w_coef[0] >= 0))
-    throw Error(CPB_ERR_UNSUPPORTED, "constrained splitters on the device need a weight that grows with the part (VertexCount or "
-                                     "AffineWorkModel(a >= 0, b_v >= 0, b_p >= 0) with b_v + b_p >= 1)");
-  const i64 wa = con->w_coef[0], wbv = con->w_coef[1], wbp = con->w_coef[2], w_max = con->w_max;
-  std::vector<u32> hpos;
-  if (wbp != 0) {
-    hpos.resize((size_t)n + 1);
-    CPB_CUDA(cudaMemcpyAsync(hpos.data(), A.pos.get(), ((size_t)n + 1) * sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
-    CPB_CUDA(cudaStreamSynchronize(ctx().stream));
-  }
-  auto fits = [&](i64 j, i64 jp) {
-    i64 w = wa + (jp - j) * wbv;
-    if (wbp != 0) w += ((i64)hpos[jp - 1] - (i64)hpos[j - 1]) * wbp;
-    return w <= w_max;
-  };
-  auto reach = [&](i64 j, i64 limit) {  // largest jp in [j + 1, limit] reached by the reference's `while w(j, jp + 1) <= w_max` from jp = j + 1
-    i64 a = std::min(j + 1, limit), b = limit;
-    while (a < b) {
-      const i64 mid = a + (b - a + 1) / 2;
-      if (fits(j, mid)) a = mid; else b = mid - 1;
-    }
-    return a;
-  };
-  // column_constraints (DynamicSplitter.jl:144-173), as in dynamic_constrained_T
-  std::vector<i64> lo(K + 1), hi(K + 1);
-  for (i64 k = K, jp = n + 1; k >= 1; --k) {
-    lo[k] = jp;
-    i64 a = 1, b = jp;
-    while (a < b) {
-      const i64 mid = a + (b - a) / 2;
-      if (fits(mid, jp)) b = mid; else a = mid + 1;
-    }
-    jp = a;
-  }
-  for (i64 k = 1, j = 1; k <= K; ++k) {
-    i64 a = j, b = n + 1;
-    while (a < b) {
-      const i64 mid = a + (b - a + 1) / 2;
-      if (fits(j, mid)) a = mid; else b = mid - 1;
-    }
-    hi[k] = a;
-    j = a;
-  }
-  if (wa > w_max) { for (i64 k = 1; k <= K; ++k) hi[k] = 1; }
-  if (hi[K] < n + 1) {  // ConvexTotalChunker.jl:184-189 infeasible -> degenerate partition
-    for (i64 k = 0; k < K; ++k) h_spl_out[k] = 1;
-    h_spl_out[K] = n + 1;
+  std::vector<i64> lo, hi;
+  if (!column_constraints(win, n, K, lo, hi)) {  // ConvexTotalChunker.jl:184-189 infeasible -> degenerate partition
+    degenerate_partition(n, K, h_spl_out);
     return;
   }
+  const DevWeight dw{win.a, win.bv, win.bp, win.w_max, win.first_fit.get()};
   const u32 n1 = (u32)n + 1, n2 = n1 + 1;
   ProfScope prof("dp_layer");
   DBuf<T> rowa(n2), rowb(n2);
@@ -545,14 +473,14 @@ template <class T> static void convex_constrained_T(Oracle& f, const cpb_constra
     const size_t cnt = (size_t)(hi[k] - lo[k] + 1);
     const unsigned grid = (unsigned)std::max<size_t>(1, std::min<size_t>((cnt + 255) / 256, (size_t)ctx().sm_count * 8));
     if (k == 1) {
-      CPB_LAUNCH(k_dp_constrained<T>, grid, 256, 0, f.dev, prev, cur, ptr.get(), 1, (u32)lo[1], (u32)hi[1], 1u, 1u, 0u, 1, DevWeight{wa, wbv, wbp, w_max}, 1u);
+      CPB_LAUNCH(k_dp_constrained<T>, grid, 256, 0, f.dev, prev, cur, ptr.get(), 1, (u32)lo[1], (u32)hi[1], 1u, 1u, 0u, 1, dw, 1u);
     } else {
       // the block chain of this layer: b_0 = j'_lo[k-1], b_1 = the reach of b_0 (at least b_0 + 1, :213-216), b_t+1 = the reach of b_t
       const i64 J0 = lo[k - 1], JP1 = hi[k];
       blk.clear();
       blk.push_back((u32)J0);
       for (i64 b = J0; b < JP1;) {
-        const i64 nx = std::max(reach(b, JP1), b + 1);
+        const i64 nx = std::max(win.reach(b, JP1), b + 1);
         blk.push_back((u32)nx);
         b = nx;
       }
@@ -560,7 +488,7 @@ template <class T> static void convex_constrained_T(Oracle& f, const cpb_constra
       CPB_CUDA(cudaStreamSynchronize(ctx().stream));  // blk is reused by the next layer
       const unsigned wgrid = (unsigned)std::max<size_t>(1, std::min<size_t>((cnt * 32 + 255) / 256, (size_t)ctx().sm_count * 16));
       CPB_LAUNCH(k_dp_convex_constrained<T>, wgrid, 256, 0, f.dev, prev, cur, ptr.get() + (size_t)(k - 1) * n2, (u32)lo[k], (u32)hi[k], (u32)lo[k - 1],
-                 (u32)hi[k - 1], DevWeight{wa, wbv, wbp, w_max}, (u32)k, dblk.get(), (u32)(blk.size() - 1));
+                 (u32)hi[k - 1], dw, (u32)k, dblk.get(), (u32)(blk.size() - 1));
     }
     std::swap(prev, cur);
   }
@@ -574,8 +502,9 @@ void solve_dynamic(Oracle& f, bool total, const cpb_constraint* con, i64 K, int6
   if (con && con->enabled) {
     if (f.dev.kind == CPB_MODEL_BLOCK || f.dev.kind == CPB_MODEL_COLBLOCK)
       throw Error(CPB_ERR_UNSUPPORTED, "dynamic splitters need an affine random-access oracle");
+    const Windows win = windows_affine(*f.A, con);
     oracle_ensure_ranks(f);
-    if (f.dev.is_float) dynamic_constrained_T<double>(f, total, con, K, h_spl_out); else dynamic_constrained_T<i64>(f, total, con, K, h_spl_out);
+    if (f.dev.is_float) dynamic_constrained_T<double>(f, total, win, K, h_spl_out); else dynamic_constrained_T<i64>(f, total, win, K, h_spl_out);
     return;
   }
   if (f.dev.kind == CPB_MODEL_BLOCK || f.dev.kind == CPB_MODEL_COLBLOCK)
@@ -592,6 +521,17 @@ void solve_dynamic(Oracle& f, bool total, const cpb_constraint* con, i64 K, int6
   if (f.dev.is_float) dynamic_T<double, TIE_RIGHT>(f, total, K, h_spl_out); else dynamic_T<i64, TIE_RIGHT>(f, total, K, h_spl_out);
 }
 
+// partition_stripe(A, K, DynamicBottleneck/TotalSplitter(ConstrainedCost(f, w, w_max))) with a count weight w: the same layers,
+// the windows from w's window array
+void solve_dynamic_weighted(Oracle& f, bool total, Oracle& w, i64 w_max, i64 K, int64_t* h_spl_out) {
+  CPB_REQUIRE(K >= 1, "K must be >= 1");
+  if (f.dev.kind == CPB_MODEL_BLOCK || f.dev.kind == CPB_MODEL_COLBLOCK)
+    throw Error(CPB_ERR_UNSUPPORTED, "dynamic splitters need an affine random-access oracle");
+  const Windows win = windows_weighted(w, w_max);
+  oracle_ensure_ranks(f);
+  if (f.dev.is_float) dynamic_constrained_T<double>(f, total, win, K, h_spl_out); else dynamic_constrained_T<i64>(f, total, win, K, h_spl_out);
+}
+
 // partition_stripe(A, K, ConvexTotalSplitter(f)) (ConvexTotalChunker.jl:26-55): the total-cost layers with the
 // stack algorithm's tie rule.  Only for cost models that obey the quadrangle inequality the algorithm assumes
 // (:121) -- work, connectivity and monotonized-symmetric models with non-negative coefficients; for anything else
@@ -602,8 +542,9 @@ void solve_convex_splitter(Oracle& f, const cpb_constraint* con, i64 K, int64_t*
   for (int t = 1; t <= 3; ++t) convex = convex && f.mdl.coef[t] >= 0;
   if (!convex) throw Error(CPB_ERR_UNSUPPORTED, "ConvexTotalSplitter on the device needs a cost model obeying the quadrangle inequality (work / connectivity / monotonized-symmetric, beta >= 0)");
   if (con && con->enabled) {  // ConvexTotalChunker.jl:167-209
+    const Windows win = windows_affine(*f.A, con);
     oracle_ensure_ranks(f);
-    if (f.dev.is_float) convex_constrained_T<double>(f, con, K, h_spl_out); else convex_constrained_T<i64>(f, con, K, h_spl_out);
+    if (f.dev.is_float) convex_constrained_T<double>(f, win, K, h_spl_out); else convex_constrained_T<i64>(f, win, K, h_spl_out);
     return;
   }
   if (K == 1) {  // :33-35
@@ -613,6 +554,17 @@ void solve_convex_splitter(Oracle& f, const cpb_constraint* con, i64 K, int64_t*
   }
   oracle_ensure_ranks(f);
   if (f.dev.is_float) dynamic_T<double, TIE_CONVEX>(f, true, K, h_spl_out); else dynamic_T<i64, TIE_CONVEX>(f, true, K, h_spl_out);
+}
+
+// ConvexTotalSplitter(ConstrainedCost(f, w, w_max)) with a count weight w
+void solve_convex_weighted(Oracle& f, Oracle& w, i64 w_max, i64 K, int64_t* h_spl_out) {
+  CPB_REQUIRE(K >= 1, "K must be >= 1");
+  bool convex = f.mdl.kind == CPB_MODEL_WORK || f.mdl.kind == CPB_MODEL_CONNECTIVITY || f.mdl.kind == CPB_MODEL_MONOSYM;
+  for (int t = 1; t <= 3; ++t) convex = convex && f.mdl.coef[t] >= 0;
+  if (!convex) throw Error(CPB_ERR_UNSUPPORTED, "ConvexTotalSplitter on the device needs a cost model obeying the quadrangle inequality (work / connectivity / monotonized-symmetric, beta >= 0)");
+  const Windows win = windows_weighted(w, w_max);
+  oracle_ensure_ranks(f);
+  if (f.dev.is_float) convex_constrained_T<double>(f, win, K, h_spl_out); else convex_constrained_T<i64>(f, win, K, h_spl_out);
 }
 
 }  // namespace cpb

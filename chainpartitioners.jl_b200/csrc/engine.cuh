@@ -145,9 +145,36 @@ void bisect_finish(BisectRun* run, int64_t* h_spl_out);
 void bisect_stats(double out[8]);
 void bisect_plan_nodes(double c_lo, double c_hi, double eps, int P, double c_lo0, double c_hi0, double ub, bool adaptive, int* ids_out);
 void bisect_prewalk(double c_lo, double c_hi, double eps, double ub, double* c_hi_out, int* probes_out);  // bisect.cu (host arithmetic)
+// A weight constraint as the constrained splitters consume it (weights.cu): an affine work weight w(j, j') = a + b_v (j' - j)
+// + b_p (pos[j'] - pos[j]) evaluated on the fly, or a count weight (AffineConnectivityModel / AffineMonotonizedSymmetric...
+// as the weight of ConstrainedCost) reduced to its window array first_fit (k_weight_windows).  Both are monotone in both
+// arguments, so `fits` answers every window test of the reference.
+struct Windows {
+  i64 a = 0, bv = 0, bp = 0;      // affine work weight
+  i64 w_max = 0, alpha = 0;       // alpha = w(j, j): above w_max no part is feasible
+  i64 W = 0;                      // widest part the windows allow (an upper bound for the affine weight with a pin term)
+  std::vector<u32> hpos;          // colptr on the host (affine weight with a pin term)
+  DBuf<u32> first_fit;            // count weight: [n + 2], first_fit[j'] (1-based); empty for the affine weight
+  std::vector<u32> h_first_fit;   // its host copy (4 bytes per column)
+  bool fits(i64 j, i64 jp) const;        // w(j, j') <= w_max or j == j', 1-based
+  i64 reach(i64 j, i64 limit) const;     // largest jp in [j + 1, limit] with fits(j, jp) (j + 1 if none)
+};
+Windows windows_affine(const Matrix& A, const cpb_constraint* con);
+Windows windows_weighted(Oracle& w, i64 w_max);
+bool column_constraints(const Windows& win, i64 n, i64 K, std::vector<i64>& lo, std::vector<i64>& hi);
+void degenerate_partition(i64 n, i64 K, int64_t* h_spl_out);
+void weight_check(const Oracle& w);  // CPB_ERR_UNSUPPORTED unless w is an accepted weight model
+// first_fit[j'] = smallest j in [1, j'] with j == j' or w(j, j') <= w_max; reach[j] = largest j' in [j, n+1] with j' == j or
+// w(j, j') <= w_max (both 1-based, n + 2 entries; reach may be nullptr)
+void weight_windows(Oracle& w, i64 w_max, DBuf<u32>& first_fit, DBuf<u32>* reach);
+
 void solve_dynamic(Oracle& f, bool total, const cpb_constraint* con, i64 K, int64_t* h_spl_out);
 void solve_convex_splitter(Oracle& f, const cpb_constraint* con, i64 K, int64_t* h_spl_out);
 void solve_concave_splitter(Oracle& f, const cpb_constraint* con, i64 K, int64_t* h_spl_out);               // concave.cu
+// the same three with a count weight: w an oracle over the same matrix (weights.cu builds its windows)
+void solve_dynamic_weighted(Oracle& f, bool total, Oracle& w, i64 w_max, i64 K, int64_t* h_spl_out);
+void solve_convex_weighted(Oracle& f, Oracle& w, i64 w_max, i64 K, int64_t* h_spl_out);
+void solve_concave_weighted(Oracle& f, Oracle& w, i64 w_max, i64 K, int64_t* h_spl_out);                    // concave.cu
 void solve_concave_chunker(Oracle& f, const cpb_constraint* con, int64_t* h_spl_out, int64_t* K_out);     // concave.cu
 void solve_pack(Matrix& A, Oracle* f, int method, const cpb_constraint* con, double rho, i64 w_max, int64_t* h_spl_out,
                 int64_t* K_out, int64_t* n_nets_out);

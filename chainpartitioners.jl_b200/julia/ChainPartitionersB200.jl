@@ -93,10 +93,18 @@ function cmodel(m::BlockComponentCostModel{Tv, R}, w_tab, u_tab) where {Tv, R}
     (CModel(8, isfloat(Tv), pad8(), R, w_tab, u_tab, 0, pointer(a), pointer(bc), pointer(br)), Any[a, bc, br])
 end
 
+# ConstrainedCost(f, w, w_max) with a count weight (src/Costs.jl:105-147): w gets an oracle of its own on the same resident
+# matrix and the solve goes through cpb_partition_stripe_weighted (Dynamic, Convex and Concave splitters)
+const CountWeighted = Union{ConstrainedCost{<:Any, <:AffineConnectivityModel{<:Integer}},
+                            ConstrainedCost{<:Any, <:AffineMonotonizedSymmetricConnectivityModel{<:Integer}}}
+
 constraint(::Any) = CConstraint(0, 0, (0, 0, 0), 0)
 constraint(c::ConstrainedCost{<:Any, VertexCount}) = CConstraint(1, 0, (0, 1, 0), Int64(c.w_max))
 constraint(c::ConstrainedCost{<:Any, <:AffineWorkModel{<:Integer}}) = CConstraint(1, 0, (Int64(c.w.α), Int64(c.w.β_vertex), Int64(c.w.β_pin)), Int64(c.w_max))
 constraint(c::ConstrainedCost{<:Any, FeasibleCost}) = CConstraint(0, 0, (0, 0, 0), 0)
+# count weights (AffineConnectivityModel / AffineMonotonizedSymmetricConnectivityModel) cannot be expressed here: stripe_solve
+# hands them to cpb_partition_stripe_weighted; pack_stripe has no count-weight form
+constraint(c::CountWeighted) = throw(ArgumentError("pack_stripe takes VertexCount() or an integer AffineWorkModel weight; count weights are not built for the chunkers"))
 basecost(f) = f
 basecost(c::ConstrainedCost) = c.f
 
@@ -252,14 +260,26 @@ split_code(::DynamicTotalChunker) = (11, 0.0)
 
 split_code(::ConcaveTotalSplitter) = (9, 0.0)
 
+function stripe_solve(dA::DeviceMatrix, K, code, ϵ, f, args...)
+    ocl = DeviceOracle(dA, f, args...)
+    spl = Vector{Int64}(undef, K + 1)
+    GC.@preserve ocl check(ccall((:cpb_partition_stripe, lib), Cint, (Ptr{Cvoid}, Cint, Ref{CConstraint}, Float64, Int64, Ptr{Int64}),
+                                 ocl.h, code, constraint(f), ϵ, K, spl))
+    return SplitPartition{Int64}(K, spl)
+end
+function stripe_solve(dA::DeviceMatrix, K, code, ϵ, f::CountWeighted, args...)
+    ocl = DeviceOracle(dA, f.f, args...)
+    wcl = DeviceOracle(dA, f.w)
+    spl = Vector{Int64}(undef, K + 1)
+    GC.@preserve ocl wcl check(ccall((:cpb_partition_stripe_weighted, lib), Cint, (Ptr{Cvoid}, Cint, Ptr{Cvoid}, Int64, Float64, Int64, Ptr{Int64}),
+                                     ocl.h, code, wcl.h, Int64(f.w_max), ϵ, K, spl))
+    return SplitPartition{Int64}(K, spl)
+end
+
 # The stripe solve on a pattern that is already resident (what partition_plaid below and repeated solves use: no upload)
 function partition_stripe(dA::DeviceMatrix, K, method::OnB200, args...; kwargs...)
     (code, ϵ) = split_code(method.mtd)
-    ocl = DeviceOracle(dA, method.mtd.f, args...)
-    spl = Vector{Int64}(undef, K + 1)
-    check(ccall((:cpb_partition_stripe, lib), Cint, (Ptr{Cvoid}, Cint, Ref{CConstraint}, Float64, Int64, Ptr{Int64}),
-                ocl.h, code, constraint(method.mtd.f), ϵ, K, spl))
-    return SplitPartition{Int64}(K, spl)
+    return stripe_solve(dA, K, code, ϵ, method.mtd.f, args...)
 end
 
 # partition_plaid(A, K, AlternatingPartitioner(OnB200(m1), OnB200(m2), ...)) (src/AlternatingPartitioner.jl:18-32): A is
@@ -377,11 +397,7 @@ end
 function partition_stripe(A::SparseMatrixCSC{Tv, Int64}, K, method::OnB200, args...; kwargs...) where {Tv}
     dA = DeviceMatrix(A)
     (code, ϵ) = split_code(method.mtd)
-    ocl = DeviceOracle(dA, method.mtd.f, args...)
-    spl = Vector{Int64}(undef, K + 1)
-    check(ccall((:cpb_partition_stripe, lib), Cint, (Ptr{Cvoid}, Cint, Ref{CConstraint}, Float64, Int64, Ptr{Int64}),
-                ocl.h, code, constraint(method.mtd.f), ϵ, K, spl))
-    return SplitPartition{Int64}(K, spl)
+    return stripe_solve(dA, K, code, ϵ, method.mtd.f, args...)
 end
 
 pack_code(m::DynamicTotalChunker) = (0, m.f, 0.0, 0)

@@ -430,12 +430,21 @@ class FeasibleCost:
 
 @dataclass
 class ConstrainedCost:
-    """Costs.jl:105-118: cost ``f`` if ``w(j,j') <= w_max`` else +inf.  ``w`` is ``VertexCount()``
-    or an integer ``AffineWorkModel`` (the only weights the reference's tests/benchmarks use)."""
+    """Costs.jl:105-147: cost ``f`` if ``w(j,j') <= w_max`` else +inf, ``w(j, j')`` being the weight model's own cost of
+    the columns ``j..j'-1``.  ``w`` is ``VertexCount()`` or an integer ``AffineWorkModel`` (an affine work weight, the form
+    every solver takes), or -- for ``partition_stripe`` with the Dynamic, Convex and Concave splitters -- an integer
+    ``AffineConnectivityModel`` or ``AffineMonotonizedSymmetricConnectivityModel`` with non-negative betas (a count
+    weight: distinct rows, i.e. a part's footprint).  The count weight gets an oracle of its own on the same matrix."""
 
     f: Any
     w: Any
     w_max: Any
+
+    def count_weight(self):
+        """The weight model if it is evaluated through an oracle of its own (anything but an affine work weight), else None."""
+        if isinstance(self.w, (FeasibleCost, VertexCount)) or (isinstance(self.w, AffineWorkModel) and not self.w.is_float):
+            return None
+        return self.w if isinstance(self.w, _AffineModel) else None
 
     def constraint(self) -> CConstraint:
         c = CConstraint()
@@ -446,6 +455,10 @@ class ConstrainedCost:
             coef = VertexCount.w_coef
         elif isinstance(self.w, AffineWorkModel) and not self.w.is_float:
             coef = self.w.coef
+        elif self.count_weight() is not None:
+            raise TypeError("a count weight (AffineConnectivityModel / AffineMonotonizedSymmetricConnectivityModel) is taken by "
+                            "partition_stripe's Dynamic, Convex and Concave splitters only; here the weight must be VertexCount() "
+                            "or an integer AffineWorkModel")
         else:
             raise TypeError("ConstrainedCost weight must be VertexCount() or an integer AffineWorkModel")
         c.enabled = 1

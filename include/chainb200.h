@@ -195,6 +195,23 @@ enum {
 /* -> spl_out[K+1] (SplitPartition{Int64}(K, spl), Partitions.jl:3-6); con may be NULL. */
 int cpb_partition_stripe(cpb_oracle* f, int method, const cpb_constraint* con, double eps, int64_t K, int64_t* spl_out);
 
+/* partition_stripe(A, K, method(ConstrainedCost(f, w, w_max))) with the weight given as a cost model of its own
+ * (Costs.jl:105-147: the reference turns w into an oracle and tests w(j, j') > w_max for the windows of every constrained
+ * solver, column_constraints DynamicSplitter.jl:144-173).  w is a cpb_oracle created by cpb_oracle_create over the SAME
+ * cpb_matrix as f (else CPB_ERR_ARG); w(j, j') is its Int64 cost of columns j..j'-1.  Accepted weights: integer
+ * AffineWorkModel, AffineConnectivityModel and AffineMonotonizedSymmetricConnectivityModel (square A) with
+ * beta_vertex, beta_pin / beta_over_pin, beta_net / beta_dia_net >= 0 (delta_pins is free) -- they cannot shrink when the
+ * range grows, so the windows are monotone.  An AffineWorkModel weight takes the cpb_constraint path.  Float64 weights,
+ * negative betas and every other model return CPB_ERR_UNSUPPORTED, as do the Bisect, Flip and Equi methods.  Methods:
+ * CPB_SPLIT_DYNAMIC_BOTTLENECK / _TOTAL (and their _CHUNKER forms), CPB_SPLIT_CONVEX_TOTAL, CPB_SPLIT_CONCAVE_TOTAL.
+ * w_max below w(j, j) makes every part infeasible; an infeasible chain returns [1, 1, ..., 1, n+1]. */
+int cpb_partition_stripe_weighted(cpb_oracle* f, int method, cpb_oracle* w, int64_t w_max, double eps, int64_t K, int64_t* spl_out);
+/* The windows of such a weight, 1-based, n + 1 entries each (index c - 1 holds column c = 1..n+1):
+ *   first_fit_out[j' - 1] = the smallest j in [1, j'] with j == j' or w(j, j') <= w_max,
+ *   reach_out[j - 1]      = the largest j' in [j, n+1] with j' == j or w(j, j') <= w_max.
+ * Builds w's dominance index on first use (a second wavelet index when f and w are different oracles). */
+int cpb_weight_windows(cpb_oracle* w, int64_t w_max, int64_t* first_fit_out, int64_t* reach_out);
+
 /* Link construction sharded by row blocks (the sweep of SparseColorArrays.jl:103-118 / :72-99 touches every row
  * independently): cpb_links_partial builds the links of the nonzeros whose row lies in [row_lo, row_hi) (1-based,
  * half-open) into d_prev_out (DEVICE buffer with room for nnz + n uint32; *ne_out <= nnz + n entries are written,
