@@ -22,7 +22,7 @@ __all__ = [
     "dianetcount", "selfnetcount", "selfpincount", "PrefixMatrix", "dominancecount", "dominancesum", "rookcount", "rooksum", "profile_enable", "profile_reset", "profile_get",
     "Communicator", "ShardedMatrix", "partition_stripe_sharded", "partition_stripe_sharded_emulated", "sharded_stats", "shard_range",
     "partition_plaid_sharded", "partition_plaid_sharded_emulated", "adjointpattern_sharded_emulated",
-    "weight_windows", "launch_count", "probe_cluster_capacity", "bisect_stats", "bisect_plan", "bisect_prewalk", "timer_start", "timer_stop", "StepwiseBisection", "StripeOracle", "init", "synchronize", "trim_memory", "library_path", "load_library", "CpbError",
+    "weight_windows", "launch_count", "bisect_stats", "bisect_plan", "bisect_prewalk", "timer_start", "timer_stop", "StripeOracle", "init", "synchronize", "trim_memory", "library_path", "load_library", "CpbError",
 ]
 
 I64 = np.int64
@@ -36,11 +36,11 @@ ABI_SYMBOLS = [
     "cpb_oracle_create", "cpb_oracle_destroy", "cpb_oracle_query", "cpb_oracle_query_device", "cpb_count_query",
     "cpb_bound_stripe", "cpb_objective", "cpb_partition_stripe", "cpb_pack_stripe", "cpb_profile_enable",
     "cpb_profile_reset", "cpb_profile_get", "cpb_launch_count", "cpb_timer_start", "cpb_timer_stop",
-    "cpb_bisect_begin", "cpb_bisect_probe", "cpb_bisect_advance", "cpb_bisect_finish", "cpb_bisect_stats", "cpb_bisect_plan", "cpb_bisect_prewalk", "cpb_probe_cluster_capacity",
+    "cpb_bisect_stats", "cpb_bisect_plan", "cpb_bisect_prewalk",
     "cpb_comm_unique_id", "cpb_comm_init", "cpb_comm_destroy", "cpb_comm_info", "cpb_shard_range", "cpb_sharded_matrix_create", "cpb_sharded_matrix_destroy",
     "cpb_partition_stripe_sharded", "cpb_partition_stripe_sharded_emulated", "cpb_sharded_stats",
     "cpb_sharded_adjointpattern", "cpb_adjointpattern_sharded_emulated", "cpb_sharded_matrix_get",
-    "cpb_links_partial", "cpb_oracle_set_links", "cpb_prefix_create", "cpb_prefix_query", "cpb_prefix_destroy", "cpb_matrix_permute", "cpb_trim_memory", "cpb_matrix_create_i32",
+    "cpb_prefix_create", "cpb_prefix_query", "cpb_prefix_destroy", "cpb_matrix_permute", "cpb_trim_memory", "cpb_matrix_create_i32",
     "cpb_partition_stripe_weighted", "cpb_weight_windows",
 ]
 
@@ -88,12 +88,6 @@ def load_library():
         lib.cpb_weight_windows.argtypes = [vp, i64, vp, vp]
         lib.cpb_pack_stripe.argtypes = [vp, vp, i32, ctypes.POINTER(T.CConstraint), dbl, i64, vp, ctypes.POINTER(i64), vp]
         lib.cpb_profile_get.argtypes = [i32, vp, vp, vp, vp]
-        lib.cpb_bisect_begin.argtypes = [vp, i32, dbl, i64, i32, vp, vp, vp, ctypes.POINTER(vp)]
-        lib.cpb_bisect_probe.argtypes = [vp, i32, i32]
-        lib.cpb_bisect_advance.argtypes = [vp, ctypes.POINTER(i32)]
-        lib.cpb_bisect_finish.argtypes = [vp, vp]
-        lib.cpb_links_partial.argtypes = [vp, i64, i64, vp, ctypes.POINTER(i64)]
-        lib.cpb_oracle_set_links.argtypes = [vp, vp, i64]
         lib.cpb_comm_unique_id.argtypes = [vp]
         lib.cpb_comm_init.argtypes = [vp, i32, i32]
         lib.cpb_comm_info.argtypes = [ctypes.POINTER(i32), ctypes.POINTER(i32)]
@@ -403,16 +397,6 @@ class StripeOracle:
         if self.weight is None:
             raise TypeError("weight_windows needs a ConstrainedCost with a count weight")
         return weight_windows(self.weight, self.w_max)
-
-    def links_partial(self, row_lo: int, row_hi: int, d_prev: int) -> int:
-        """Multi-GPU link construction: links of the nonzeros with row in [row_lo, row_hi) into the device buffer
-        ``d_prev`` (room for nnz + n uint32); returns the number of link entries."""
-        ne = ctypes.c_int64()
-        _check(load_library().cpb_links_partial(self._h, int(row_lo), int(row_hi), ctypes.c_void_p(d_prev), ctypes.byref(ne)))
-        return ne.value
-
-    def set_links(self, d_prev: int, ne: int):
-        _check(load_library().cpb_oracle_set_links(self._h, ctypes.c_void_p(d_prev), int(ne)))
 
     def query_device(self, d_j: int, d_jp: int, d_out: int, Q: int):
         """Batched queries on device-resident Int64 arrays (raw device pointers), result Float64 on the device."""
@@ -924,39 +908,6 @@ def partition_plaid_sharded_emulated(A, K, method, world: int):
                 held["T"].close()
 
 
-class StepwiseBisection:
-    """One BisectCost / LazyBisectCost solve as explicit rounds (``cpb_bisect_*``): the speculative
-    thresholds of a round (the first ``nodes`` nodes of the bisection tree) may be probed by different GPUs; the caller exchanges the node
-    buffers (device pointers of caller-owned arrays, e.g. torch tensors) between ``probe`` and ``advance``."""
-
-    def __init__(self, ocl: StripeOracle, method, K: int, nodes: int, d_res: int = 0, d_c: int = 0, d_spl: int = 0):
-        code, _, eps = T.split_method_code(method)
-        self.K = int(K)
-        self.nodes = max(1, min(int(nodes), 255))
-        self._h = ctypes.c_void_p()
-        _check(load_library().cpb_bisect_begin(ocl._h, code, eps, self.K, self.nodes, ctypes.c_void_p(d_res), ctypes.c_void_p(d_c),
-                                               ctypes.c_void_p(d_spl), ctypes.byref(self._h)))
-
-    def probe(self, node_lo: int, node_hi: int):
-        _check(load_library().cpb_bisect_probe(self._h, int(node_lo), int(node_hi)))
-
-    def advance(self) -> bool:
-        done = ctypes.c_int()
-        _check(load_library().cpb_bisect_advance(self._h, ctypes.byref(done)))
-        return bool(done.value)
-
-    def finish(self) -> T.SplitPartition:
-        spl = np.empty(self.K + 1, dtype=I64)
-        h, self._h = self._h, None
-        _check(load_library().cpb_bisect_finish(h, _p(spl)))
-        return T.SplitPartition(self.K, spl)
-
-    def __del__(self):
-        if getattr(self, "_h", None) is not None and _lib is not None:
-            _lib.cpb_bisect_finish(self._h, None)
-            self._h = None
-
-
 # ------------------------------------------------------------------------------- measurement hooks
 
 
@@ -1007,12 +958,6 @@ def bisect_stats() -> dict:
     _check(load_library().cpb_bisect_stats(out))
     return {"rounds": int(out[0]), "probes": int(out[1]), "speculated": int(out[2]), "c_lo": out[3], "c_hi": out[4], "plan_upper_bound": out[5],
             "c_lo_final": out[6], "c_hi_final": out[7]}
-
-
-def probe_cluster_capacity(streaming: bool = True) -> int:
-    out = ctypes.c_int()
-    _check(load_library().cpb_probe_cluster_capacity(int(streaming), ctypes.byref(out)))
-    return out.value
 
 
 def launch_count() -> int:

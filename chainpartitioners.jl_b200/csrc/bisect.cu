@@ -1225,7 +1225,7 @@ __global__ void k_ub_index(const __grid_constant__ DevOracle o, int K, double* _
 }
 
 // ---- one bisection as a sequence of steps, so that the nodes of a round can be probed by different
-//      ranks (chainb200.parallel.partition_stripe_sharded) ----
+//      ranks (the sharded solve, sharded.cu) ----
 struct BisectRun {
   Oracle* f = nullptr;
   bool stream = false;
@@ -1233,11 +1233,11 @@ struct BisectRun {
   double eps1 = 1;
   int P = 1;
   DBuf<BisectState> st;
-  DBuf<int> hint_lo, hint_hi, best, own_spl, own_res, ids;
-  DBuf<double> own_c;
-  int* node_spl = nullptr;
-  int* node_res = nullptr;
-  double* node_c = nullptr;
+  DBuf<int> hint_lo, hint_hi, best, ids;
+  // per node of the round: 1-based split points ((K+2) each), result (0 = loop condition already false, 1 = infeasible,
+  // 2 = feasible), threshold
+  DBuf<int> node_spl, node_res;
+  DBuf<double> node_c;
   DevStream ds{};
   bool done = false;
   double c_lo0 = 0, c_hi0 = 0, eps = 0;
@@ -1416,13 +1416,15 @@ void bisect_prewalk(double c_lo, double c_hi, double eps, double ub, double* c_h
   *probes_out = probes;
 }
 
-BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int* d_node_res, double* d_node_c, int* d_node_spl) {
+void BisectRunDelete::operator()(BisectRun* run) const { delete run; }
+
+BisectRunPtr bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes) {
   CPB_REQUIRE(K >= 1, "K must be >= 1");
   CPB_REQUIRE(f.dev.kind != CPB_MODEL_BLOCK, "bisection needs a random-access oracle");
   require_monotone_cost(f);
   const Matrix& A = *f.A;
   CPB_REQUIRE(A.n + 1 < ((i64)1 << 31) && K + 2 < ((i64)1 << 30), "problem too large for 32-bit split points");
-  auto run = std::make_unique<BisectRun>();
+  BisectRunPtr run(new BisectRun);
   run->f = &f;
   run->K = K;
   run->adaptive = env_int("CPB_BISECT_PLAN", 1) != 0;
@@ -1432,13 +1434,12 @@ BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int*
     // Everything the host needs before the first round -- the row-degree check of the link construction, nets(1, n+1)
     // or the over-pin total for bound_stripe, the planner's upper bound -- is produced without waiting and read back
     // with ONE synchronisation.
-    CPB_REQUIRE(f.ls_complete, "partial links were built but never completed (cpb_oracle_set_links)");
     const bool dia = f.dev.kind == CPB_MODEL_MONOSYM;
     if (!f.ls) {
       ProfScope prof("oracle_stripe");
       // (large patterns: check the row degree first -- a wasted gigabyte-sized segment allocation costs far more than
       //  the ~20 us round trip the deferred check saves)
-      f.ls = build_link_stream(A, dia, 0, (i64)1 << 62, /*defer_check=*/A.N < ((i64)1 << 25), false, /*as_pos=*/true);
+      f.ls = build_link_stream(A, dia, /*defer_check=*/A.N < ((i64)1 << 25), false, /*as_pos=*/true);
     }
     trace_mark("links");
     const bool want_ub = run->adaptive && K >= 2 && K <= 65535 && A.n >= 1;  // (K is the y extent of the counting grid)
@@ -1457,7 +1458,7 @@ BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int*
       if (f.ls->speculative && !dia) A.max_row_deg = (i64)info[1];
       if (f.ls->speculative && info[1] > LT_MAX_DEG) {  // a heavy row: the row-segment kernels did nothing -> stable sort
         ProfScope prof("oracle_stripe");
-        f.ls = build_link_stream(A, dia, 0, (i64)1 << 62, false, /*force_sort=*/true, /*as_pos=*/true);
+        f.ls = build_link_stream(A, dia, false, /*force_sort=*/true, /*as_pos=*/true);
         continue;
       }
       trace_mark("plan_bound");
@@ -1512,15 +1513,10 @@ BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int*
   run->hint_hi.alloc(K + 2);
   run->best.alloc(K + 2);
   run->h_best.assign(K + 2, 0);
-  if (d_node_res && d_node_c && d_node_spl) {
-    run->node_res = d_node_res; run->node_c = d_node_c; run->node_spl = d_node_spl;
-  } else {
-    run->own_spl.alloc((size_t)P * (K + 2));
-    run->own_res.alloc(P);
-    run->own_c.alloc(P);
-    run->own_spl.zero();
-    run->node_res = run->own_res.get(); run->node_c = run->own_c.get(); run->node_spl = run->own_spl.get();
-  }
+  run->node_spl.alloc((size_t)P * (K + 2));
+  run->node_res.alloc(P);
+  run->node_c.alloc(P);
+  run->node_spl.zero();
   BisectState h{};
   h.c_lo = bnd[0];
   h.c_hi = bnd[1];
@@ -1547,7 +1543,7 @@ BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int*
     CPB_CUDA(cudaMemcpyAsync(run->h_best.data(), run->best.get(), (K + 2) * sizeof(int), cudaMemcpyDeviceToHost, ctx().stream));
     CPB_CUDA(cudaStreamSynchronize(ctx().stream));
   }
-  return run.release();
+  return run;
 }
 
 static unsigned long long* g_probe_dbg_host = nullptr;
@@ -1588,13 +1584,13 @@ void bisect_probe(BisectRun& run, int node_lo, int node_hi) {
       ProfScope pk("k_probe_stream", (double)(f.ls->Ne + f.A->n + 1) * 4.0 + (double)cnt * (K + 1) * 8.0);
       probe_debug_arm();
       if (f.dev.is_float)
-        CPB_LAUNCH(k_probe_stream<double>, cnt * BS_CLUSTER, SP_THREADS, 0, run.ds, K, run.eps1, run.st.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
+        CPB_LAUNCH(k_probe_stream<double>, cnt * BS_CLUSTER, SP_THREADS, 0, run.ds, K, run.eps1, run.st.get(), run.node_spl.get(), run.node_res.get(), run.node_c.get(), run.ids.get(), base);
       else
-        CPB_LAUNCH(k_probe_stream<i64>, cnt * BS_CLUSTER, SP_THREADS, 0, run.ds, K, run.eps1, run.st.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
+        CPB_LAUNCH(k_probe_stream<i64>, cnt * BS_CLUSTER, SP_THREADS, 0, run.ds, K, run.eps1, run.st.get(), run.node_spl.get(), run.node_res.get(), run.node_c.get(), run.ids.get(), base);
     } else if (f.dev.is_float) {
-      CPB_LAUNCH(k_bisect_round<double>, cnt * BS_CLUSTER, BS_THREADS, 0, f.dev, K, run.eps1, run.st.get(), run.hint_lo.get(), run.hint_hi.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
+      CPB_LAUNCH(k_bisect_round<double>, cnt * BS_CLUSTER, BS_THREADS, 0, f.dev, K, run.eps1, run.st.get(), run.hint_lo.get(), run.hint_hi.get(), run.node_spl.get(), run.node_res.get(), run.node_c.get(), run.ids.get(), base);
     } else {
-      CPB_LAUNCH(k_bisect_round<i64>, cnt * BS_CLUSTER, BS_THREADS, 0, f.dev, K, run.eps1, run.st.get(), run.hint_lo.get(), run.hint_hi.get(), run.node_spl, run.node_res, run.node_c, run.ids.get(), base);
+      CPB_LAUNCH(k_bisect_round<i64>, cnt * BS_CLUSTER, BS_THREADS, 0, f.dev, K, run.eps1, run.st.get(), run.hint_lo.get(), run.hint_hi.get(), run.node_spl.get(), run.node_res.get(), run.node_c.get(), run.ids.get(), base);
     }
   }
 }
@@ -1603,7 +1599,7 @@ void bisect_probe(BisectRun& run, int node_lo, int node_hi) {
 bool bisect_advance(BisectRun& run, bool sync) {
   if (!run.planned) plan_round(run);  // (advance without a probe: the walk stops at the root)
   CPB_LAUNCH(k_bisect_advance, 1, 256, 0, (int)run.K, run.P, run.eps1, run.st.get(), run.hint_lo.get(), run.hint_hi.get(), run.best.get(),
-             run.node_spl, run.node_res, run.node_c, run.ids.get());
+             run.node_spl.get(), run.node_res.get(), run.node_c.get(), run.ids.get());
   if (sync) {
     check_probes(cudaMemcpyAsync(&run.h_st, run.st.get(), sizeof(BisectState), cudaMemcpyDeviceToHost, ctx().stream));
     check_probes(cudaMemcpyAsync(run.h_best.data(), run.best.get(), (run.K + 2) * sizeof(int), cudaMemcpyDeviceToHost, ctx().stream));
@@ -1615,7 +1611,7 @@ bool bisect_advance(BisectRun& run, bool sync) {
 }
 
 void bisect_node_buffers(BisectRun& run, int** res, double** c, int** spl, int* P) {
-  *res = run.node_res; *c = run.node_c; *spl = run.node_spl; *P = run.P;
+  *res = run.node_res.get(); *c = run.node_c.get(); *spl = run.node_spl.get(); *P = run.P;
 }
 bool bisect_is_done(BisectRun& run) { return run.done; }
 
@@ -1624,15 +1620,13 @@ void bisect_stats(double out[8]) {
   for (int t = 0; t < 8; ++t) out[t] = g_bisect_stats[t];
 }
 
-void bisect_finish(BisectRun* run_ptr, int64_t* h_spl_out) {
-  std::unique_ptr<BisectRun> run(run_ptr);
-  if (!h_spl_out) return;
-  CPB_REQUIRE(run->done, "bisection has not finished");
-  const i64 K = run->K;
-  g_bisect_stats[0] = run->h_st.rounds; g_bisect_stats[1] = run->h_st.probes; g_bisect_stats[2] = (double)run->speculated;
-  g_bisect_stats[3] = run->c_lo0; g_bisect_stats[4] = run->c_hi0; g_bisect_stats[5] = run->ub;
-  g_bisect_stats[6] = run->h_st.c_lo; g_bisect_stats[7] = run->h_st.c_hi;
-  for (i64 k = 1; k <= K + 1; ++k) h_spl_out[k - 1] = run->h_best[k];  // read back by the last advance
+void bisect_finish(const BisectRun& run, int64_t* h_spl_out) {
+  CPB_REQUIRE(run.done, "bisection has not finished");
+  const i64 K = run.K;
+  g_bisect_stats[0] = run.h_st.rounds; g_bisect_stats[1] = run.h_st.probes; g_bisect_stats[2] = (double)run.speculated;
+  g_bisect_stats[3] = run.c_lo0; g_bisect_stats[4] = run.c_hi0; g_bisect_stats[5] = run.ub;
+  g_bisect_stats[6] = run.h_st.c_lo; g_bisect_stats[7] = run.h_st.c_hi;
+  for (i64 k = 1; k <= K + 1; ++k) h_spl_out[k - 1] = run.h_best[k];  // read back by the last advance
 }
 
 #ifdef CPB_PROBE_TIMING
@@ -1735,9 +1729,9 @@ void solve_flip(Oracle& f, int method, double eps, i64 K, int64_t* h_spl_out) {
 
 void solve_bisect(Oracle& f, bool lazy, double eps, i64 K, int64_t* h_spl_out) {
   const int depth = std::min(std::max(env_int("CPB_BISECT_DEPTH", BS_LOCAL_DEPTH), 1), BS_LOCAL_DEPTH);
-  BisectRun* run = bisect_begin(f, lazy, eps, K, (1 << depth) - 1, nullptr, nullptr, nullptr);
+  BisectRunPtr run = bisect_begin(f, lazy, eps, K, (1 << depth) - 1);
   trace_mark("begin");
-  try {
+  {
     ProfScope prof("probe");
     // The gap c_hi - c_lo halves with every probe and the loop stops once it is <= eps * c_lo, so the number
     // of rounds is bounded from the initial bounds: queue them all without host round trips (rounds past
@@ -1757,11 +1751,8 @@ void solve_bisect(Oracle& f, bool lazy, double eps, i64 K, int64_t* h_spl_out) {
       trace_mark("advance");
     }
     CPB_REQUIRE(run->done, "bisection did not terminate (eps too small for Float64?)");
-  } catch (...) {
-    delete run;
-    throw;
   }
-  bisect_finish(run, h_spl_out);
+  bisect_finish(*run, h_spl_out);
   trace_mark("finish");
 #ifdef CPB_PROBE_TIMING
   if (env_int("CPB_PROBE_TIMING_DUMP", 0)) probe_timing_dump();

@@ -187,7 +187,7 @@ static void resolve_pending() {
 extern "C" {
 
 const char* cpb_last_error(void) { return cpb::g_err.c_str(); }
-int cpb_version(void) { return 100; }
+int cpb_version(void) { return 101; }
 
 int cpb_init(int device) {
   CPB_API_BEGIN
@@ -667,61 +667,6 @@ int cpb_weight_windows(cpb_oracle* w, int64_t w_max, int64_t* first_fit_out, int
     first_fit_out[c] = h[c];
     reach_out[c] = h[n1 + c];
   }
-  CPB_API_END
-}
-
-// ---- multi-GPU link construction ----
-int cpb_links_partial(cpb_oracle* f, int64_t row_lo, int64_t row_hi, uint32_t* d_prev_out, int64_t* ne_out) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(f && ne_out, "NULL argument");
-  *ne_out = oracle_links_partial(*f->O, row_lo, row_hi, d_prev_out);
-  CPB_API_END
-}
-int cpb_oracle_set_links(cpb_oracle* f, const uint32_t* d_prev, int64_t ne) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(f && (d_prev || ne == 0), "NULL argument");
-  oracle_set_links(*f->O, d_prev, ne);
-  CPB_API_END
-}
-
-// ---- stepwise bisection (multi-GPU threshold sharding) ----
-int cpb_bisect_begin(cpb_oracle* f, int method, double eps, int64_t K, int nodes, int32_t* d_node_res, double* d_node_c,
-                     int32_t* d_node_spl, cpb_bisect** out) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(f && out, "NULL argument");
-  CPB_REQUIRE(method == CPB_SPLIT_BISECT_COST || method == CPB_SPLIT_LAZY_BISECT_COST, "stepwise bisection: bisect methods only");
-  *out = reinterpret_cast<cpb_bisect*>(bisect_begin(*f->O, method == CPB_SPLIT_LAZY_BISECT_COST, eps, K, nodes, d_node_res, d_node_c, d_node_spl));
-  CPB_API_END
-}
-int cpb_probe_cluster_capacity(int streaming, int* out) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(out, "NULL argument");
-  *out = probe_cluster_capacity(streaming != 0);
-  CPB_API_END
-}
-int cpb_bisect_probe(cpb_bisect* b, int node_lo, int node_hi) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(b, "NULL argument");
-  bisect_probe(*reinterpret_cast<BisectRun*>(b), node_lo, node_hi);
-  CPB_API_END
-}
-int cpb_bisect_advance(cpb_bisect* b, int* done_out) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(b && done_out, "NULL argument");
-  *done_out = bisect_advance(*reinterpret_cast<BisectRun*>(b), true) ? 1 : 0;
-  CPB_API_END
-}
-int cpb_bisect_finish(cpb_bisect* b, int64_t* spl_out) {
-  CPB_API_BEGIN
-  ensure_context();
-  CPB_REQUIRE(b, "NULL argument");
-  bisect_finish(reinterpret_cast<BisectRun*>(b), spl_out);
   CPB_API_END
 }
 

@@ -54,8 +54,7 @@ struct LinkStream {
 struct Matrix;
 static constexpr u32 LS_COLQ = 128;     // granularity of LinkStream::colq: 128 elements rarely span more than 32 columns
 static constexpr u32 LT_MAX_DEG = 128;  // largest row degree handled by the row-segment link construction (links.cu)
-std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row_lo = 0, i64 row_hi = ((i64)1 << 62), bool defer_check = false,
-                                              bool force_sort = false, bool as_pos = false);
+std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, bool defer_check = false, bool force_sort = false, bool as_pos = false);
 void fill_colq(LinkStream& ls, u32 n);  // LinkStream::colq from P and Ne
 
 // SparseColorArrays.jl: NetCount :103-118, dianetcount! :72-99, SelfNetCount :177-229, SelfPinCount :281-318
@@ -65,8 +64,7 @@ std::unique_ptr<RankStruct> build_partwise_rank(const Matrix& A, const u32* asg,
 void build_partwise_columns(const Matrix& A, const u32* asg, u32 K, DBuf<u32>& part_col, DBuf<u32>& part_start, DBuf<u32>& part_head);
 // prev[q] = 1-based previous column holding the same row (0 if none); colidx[q] = 0-based column of q
 bool compute_prev_links(const u32* pos, const u32* row, u32 nrow, u32 ncol, size_t N, u32* prev, u32* colidx, u32* first_count = nullptr,
-                        i64 row_lo = 0, i64 row_hi = ((i64)1 << 62), bool defer_check = false, bool force_sort = false, bool as_pos = false,
-                        i64* max_deg_cache = nullptr);
+                        bool defer_check = false, bool force_sort = false, bool as_pos = false, i64* max_deg_cache = nullptr);
 // For the diagonal-augmented structure the pin prefix (pos') differs from A.pos; it is RankStruct::P.
 
 // ---- device-side oracle ------------------------------------------------------------------------
@@ -118,12 +116,9 @@ struct Oracle {
   std::vector<i64> h_pi_spl;
   i64 pi_K = 0;
   bool ranks_built = false;
-  bool ls_complete = true;  // false between cpb_links_partial and cpb_oracle_set_links
   DevOracle dev{};
 };
 void oracle_ensure_ranks(Oracle& f);
-i64 oracle_links_partial(Oracle& f, i64 row_lo, i64 row_hi, u32* d_prev_out);
-void oracle_set_links(Oracle& f, const u32* d_prev, i64 Ne);
 i64 count_first_occurrences(const LinkStream& ls);
 
 std::unique_ptr<Oracle> oracle_create(Matrix& A, const cpb_model* mdl, const int64_t* pi_spl, i64 pi_K);
@@ -137,11 +132,14 @@ void solve_bisect(Oracle& f, bool lazy, double eps, i64 K, int64_t* h_spl_out);
 void solve_bisect_index(Oracle& f, i64 K, int64_t* h_spl_out);
 void solve_flip(Oracle& f, int method, double eps, i64 K, int64_t* h_spl_out);
 int probe_cluster_capacity(bool stream);
+// one bisection as steps (bisect.cu); the run owns its node buffers
 struct BisectRun;
-BisectRun* bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes, int* d_node_res, double* d_node_c, int* d_node_spl);
+struct BisectRunDelete { void operator()(BisectRun* run) const; };
+using BisectRunPtr = std::unique_ptr<BisectRun, BisectRunDelete>;
+BisectRunPtr bisect_begin(Oracle& f, bool lazy, double eps, i64 K, int nodes);
 void bisect_probe(BisectRun& run, int node_lo, int node_hi);
 bool bisect_advance(BisectRun& run, bool sync);
-void bisect_finish(BisectRun* run, int64_t* h_spl_out);
+void bisect_finish(const BisectRun& run, int64_t* h_spl_out);  // copies spl_hi[1..K+1] out once the run is done
 void bisect_stats(double out[8]);
 void bisect_plan_nodes(double c_lo, double c_hi, double eps, int P, double c_lo0, double c_hi0, double ub, bool adaptive, int* ids_out);
 void bisect_prewalk(double c_lo, double c_hi, double eps, double ub, double* c_hi_out, int* probes_out);  // bisect.cu (host arithmetic)

@@ -28,18 +28,6 @@ static void transpose_order(const u32* row, size_t N, u64 max_row, TransposeOrde
 
 static unsigned grid_for(size_t n) { return (unsigned)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, (size_t)ctx().sm_count * 32)); }
 
-// (row, q) pairs of the nonzeros whose row lies in [lo, hi)
-__global__ void k_row_flags(const u32* __restrict__ row, size_t N, u32 lo, u32 hi, u32* __restrict__ flags) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q <= N; q += stride) flags[q] = (q < N && row[q] >= lo && row[q] < hi) ? 1u : 0u;
-}
-__global__ void k_row_compact(const u32* __restrict__ row, const u32* __restrict__ flags, const u32* __restrict__ scan, size_t N,
-                              u32* __restrict__ keys, u32* __restrict__ vals) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < N; q += stride)
-    if (flags[q]) { keys[scan[q]] = row[q]; vals[scan[q]] = (u32)q; }
-}
-
 // prev[q] = 1-based previous column holding the same row, 0 if none; as_pos: 1 + CSC position of that previous nonzero
 // instead (what the streaming probes compare against the part's first position -- no column lookup at all)
 __global__ void k_link_prev(const u32* __restrict__ sk, const u32* __restrict__ sq, const u32* __restrict__ colidx,
@@ -246,14 +234,12 @@ static u32 read_u32(const u32* d) {
 }
 
 // prev[q] = 1-based previous column holding the same row (0 if none); colidx[q] = 0-based column of q
-// row_lo/row_hi (0-based, half-open) restrict the construction to the nonzeros of a row block: prev[] is
-// written for those nonzeros only and is zero elsewhere (multi-GPU: ranks combine with an element-wise MAX).
 // info[0] receives the number of links equal to 0 (= non-empty rows), info[1] the maximal row degree when the row-segment
 // form was tried (0 otherwise).  defer_check: do not wait for that degree -- launch the row-segment kernels at once (they
 // do nothing if the degree is too large) and return true; the caller inspects info[1] later and calls again with
 // CPB_NO_ROW_SEGMENTS semantics (force_sort) if it exceeds LT_MAX_DEG.
 bool compute_prev_links(const u32* pos, const u32* row, u32 nrow, u32 ncol, size_t N, u32* prev, u32* colidx, u32* first_count,
-                        i64 row_lo, i64 row_hi, bool defer_check, bool force_sort, bool as_pos, i64* max_deg_cache) {
+                        bool defer_check, bool force_sort, bool as_pos, i64* max_deg_cache) {
   ProfScope prof("build_links", (double)(2 * N + ncol + 1) * 4.0);
   CPB_REQUIRE(colidx || as_pos, "column-valued links need the column array");
   if (colidx) {
@@ -266,7 +252,7 @@ bool compute_prev_links(const u32* pos, const u32* row, u32 nrow, u32 ncol, size
   // a row known to be too heavy (an earlier construction on the same resident matrix saw it): straight to the sort
   const bool known_heavy = max_deg_cache && *max_deg_cache > (i64)LT_MAX_DEG;
   const bool no_lt = force_sort || known_heavy || std::getenv("CPB_NO_ROW_SEGMENTS") != nullptr;  // (tests: force the radix-sort path)
-  if (row_lo <= 0 && row_hi >= (i64)nrow && N && nrow && !no_lt) {
+  if (N && nrow && !no_lt) {
     DBuf<u32> cur((size_t)nrow + 1);  // per-row counts -> segment starts -> (after the fill) segment ends; [nrow] = max degree
     CPB_CUDA(cudaMemsetAsync(cur.get(), 0, ((size_t)nrow + 1) * sizeof(u32), ctx().stream));
     u32 seen_deg = 0;
@@ -306,55 +292,42 @@ bool compute_prev_links(const u32* pos, const u32* row, u32 nrow, u32 ncol, size
       return defer_check;
     }
   }
-  if (row_lo <= 0 && row_hi >= (i64)nrow) {
-    trace_mark("degree_check");
-    const char* wmin_env0 = std::getenv("CPB_WINDOWED_SCATTER_MIN");  // (tests force the windowed form on small inputs; 0 = never)
-    const size_t wmin0 = wmin_env0 ? (size_t)std::atoll(wmin_env0) : ((size_t)1 << 25);
-    const char* os_env = std::getenv("CPB_ONESWEEP");  // 0: the tile-histogram sort of round 1 (kept for comparison)
-    if (onesweep_supported(N) && !(os_env && os_env[0] == '0')) {
-      // one-read-one-write radix passes on packed (row, position) pairs; the window pass forms the links while loading
-      DBuf<u64> a(N), b(N);
-      onesweep_links(row, N, bits_for(nrow ? nrow - 1 : 0), colidx, as_pos, 0u, prev, first_count, nullptr, wmin0, a.get(), b.get());
-      return false;
-    }
-    TransposeOrder t;
-    transpose_order(row, N, nrow ? nrow - 1 : 0, t);
-    trace_mark("sort");
-    const char* wmin_env = std::getenv("CPB_WINDOWED_SCATTER_MIN");  // (tests force the windowed form on small inputs; 0 = never)
-    const size_t wmin = wmin_env ? (size_t)std::atoll(wmin_env) : ((size_t)1 << 25);
-    if (wmin > 0 && N >= wmin) {
-      // the link array no longer fits L2: a scatter in row order touches one HBM sector per 4-byte link (measured 10.9 ms
-      // at N = 2.6e8).  One more partition pass groups the (position, link) pairs by 2^20-position windows (4 MB of `prev`
-      // each), and the scatter of each window stays in L2.
-      ProfScope pk("k_link_prev", (double)N * 12.0);
-      u32* const other_k = (t.keys == t.k0.get()) ? t.k1.get() : t.k0.get();  // the sort's scratch pair
-      u32* const other_v = (t.q == t.v0.get()) ? t.v1.get() : t.v0.get();
-      CPB_LAUNCH(k_link_values, grid_for(N), 256, 0, t.keys, t.q, colidx, other_k, N, first_count, as_pos ? 1 : 0);
-      const int shift = std::max(0, bits_for(N - 1) - 8);
-      radix_partition_pass(t.q, other_k, t.keys, other_v, N, shift);  // t.keys is free once the links are formed
-      CPB_LAUNCH(k_scatter_pairs, (unsigned)((N + 255) / 256), 256, 0, t.keys, other_v, prev, N);
-    } else if (N) {
-      ProfScope pk("k_link_prev", (double)N * 12.0);
-      CPB_LAUNCH(k_link_prev, grid_for(N), 256, 0, t.keys, t.q, colidx, prev, N, first_count, as_pos ? 1 : 0);
-    }
+  trace_mark("degree_check");
+  const char* wmin_env0 = std::getenv("CPB_WINDOWED_SCATTER_MIN");  // (tests force the windowed form on small inputs; 0 = never)
+  const size_t wmin0 = wmin_env0 ? (size_t)std::atoll(wmin_env0) : ((size_t)1 << 25);
+  const char* os_env = std::getenv("CPB_ONESWEEP");  // 0: the tile-histogram sort of round 1 (kept for comparison)
+  if (onesweep_supported(N) && !(os_env && os_env[0] == '0')) {
+    // one-read-one-write radix passes on packed (row, position) pairs; the window pass forms the links while loading
+    DBuf<u64> a(N), b(N);
+    onesweep_links(row, N, bits_for(nrow ? nrow - 1 : 0), colidx, as_pos, 0u, prev, first_count, nullptr, wmin0, a.get(), b.get());
     return false;
   }
-  if (N) CPB_CUDA(cudaMemsetAsync(prev, 0, N * sizeof(u32), ctx().stream));
-  DBuf<u32> flags(N + 1), scan(N + 1);
-  CPB_LAUNCH(k_row_flags, grid_for(N + 1), 256, 0, row, N, (u32)std::max<i64>(row_lo, 0), (u32)std::min<i64>(row_hi, nrow), flags.get());
-  exclusive_scan_u32(flags.get(), scan.get(), N + 1);
-  const size_t M = read_u32(scan.get() + N);
-  if (M == 0) return false;
-  DBuf<u32> k0(M), v0(M), k1(M), v1(M);
-  CPB_LAUNCH(k_row_compact, grid_for(N), 256, 0, row, flags.get(), scan.get(), N, k0.get(), v0.get());
-  const int which = radix_sort_pairs(k0.get(), v0.get(), k1.get(), v1.get(), M, bits_for(nrow ? nrow - 1 : 0));
-  CPB_LAUNCH(k_link_prev, grid_for(M), 256, 0, which ? k1.get() : k0.get(), which ? v1.get() : v0.get(), colidx, prev, M, first_count, as_pos ? 1 : 0);
+  TransposeOrder t;
+  transpose_order(row, N, nrow ? nrow - 1 : 0, t);
+  trace_mark("sort");
+  const char* wmin_env = std::getenv("CPB_WINDOWED_SCATTER_MIN");  // (tests force the windowed form on small inputs; 0 = never)
+  const size_t wmin = wmin_env ? (size_t)std::atoll(wmin_env) : ((size_t)1 << 25);
+  if (wmin > 0 && N >= wmin) {
+    // the link array no longer fits L2: a scatter in row order touches one HBM sector per 4-byte link (measured 10.9 ms
+    // at N = 2.6e8).  One more partition pass groups the (position, link) pairs by 2^20-position windows (4 MB of `prev`
+    // each), and the scatter of each window stays in L2.
+    ProfScope pk("k_link_prev", (double)N * 12.0);
+    u32* const other_k = (t.keys == t.k0.get()) ? t.k1.get() : t.k0.get();  // the sort's scratch pair
+    u32* const other_v = (t.q == t.v0.get()) ? t.v1.get() : t.v0.get();
+    CPB_LAUNCH(k_link_values, grid_for(N), 256, 0, t.keys, t.q, colidx, other_k, N, first_count, as_pos ? 1 : 0);
+    const int shift = std::max(0, bits_for(N - 1) - 8);
+    radix_partition_pass(t.q, other_k, t.keys, other_v, N, shift);  // t.keys is free once the links are formed
+    CPB_LAUNCH(k_scatter_pairs, (unsigned)((N + 255) / 256), 256, 0, t.keys, other_v, prev, N);
+  } else if (N) {
+    ProfScope pk("k_link_prev", (double)N * 12.0);
+    CPB_LAUNCH(k_link_prev, grid_for(N), 256, 0, t.keys, t.q, colidx, prev, N, first_count, as_pos ? 1 : 0);
+  }
   return false;
 }
 
 // The link array of A (dia = false) or of A + I (dia = true, SparseColorArrays.jl:72-99) in column order,
 // kept for the streaming probes; P[x] = #{elements in columns < x}.
-std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row_lo, i64 row_hi, bool defer_check, bool force_sort, bool as_pos) {
+std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, bool defer_check, bool force_sort, bool as_pos) {
   auto ls = std::make_unique<LinkStream>();
   ls->pos_links = as_pos;
   const size_t N = (size_t)A.N;
@@ -364,8 +337,8 @@ std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row
     ls->prev.alloc(N);
     if (!as_pos) ls->colidx.alloc(N);
     ls->first_count.alloc(2);
-    ls->speculative = compute_prev_links(A.pos.get(), A.row.get(), m, n, N, ls->prev.get(), as_pos ? nullptr : ls->colidx.get(), ls->first_count.get(), row_lo,
-                                         row_hi, defer_check, force_sort, as_pos, &A.max_row_deg);
+    ls->speculative = compute_prev_links(A.pos.get(), A.row.get(), m, n, N, ls->prev.get(), as_pos ? nullptr : ls->colidx.get(), ls->first_count.get(),
+                                         defer_check, force_sort, as_pos, &A.max_row_deg);
     ls->P = A.pos.get() - 1;  // P[x] = pos[x-1]
     fill_colq(*ls, n);
     return ls;
@@ -389,7 +362,7 @@ std::unique_ptr<LinkStream> build_link_stream(const Matrix& A, bool dia, i64 row
   ls->prev.alloc(N2);
   if (!as_pos) ls->colidx.alloc(N2);
   ls->first_count.alloc(2);
-  ls->speculative = compute_prev_links(pos2, row2.get(), m, n, N2, ls->prev.get(), as_pos ? nullptr : ls->colidx.get(), ls->first_count.get(), row_lo, row_hi,
+  ls->speculative = compute_prev_links(pos2, row2.get(), m, n, N2, ls->prev.get(), as_pos ? nullptr : ls->colidx.get(), ls->first_count.get(),
                                        defer_check, force_sort, as_pos, &heavy_hint);
   ls->P = ls->P_own.get();  // P[x] = pos2[x-1]
   fill_colq(*ls, n);

@@ -244,39 +244,6 @@ void oracle_ensure_ranks(Oracle& f) {
   f.ranks_built = true;
 }
 
-// ---- multi-GPU link construction --------------------------------------------------------------------
-__global__ void k_count_zero_u32(const u32* __restrict__ v, size_t n, u32* __restrict__ out) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  u32 c = 0;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) c += v[i] == 0u;
-  c = __reduce_add_sync(0xffffffffu, c);
-  if ((threadIdx.x & 31) == 0 && c) atomicAdd(out, c);
-}
-
-static bool model_uses_dia(int kind) { return kind == CPB_MODEL_MONOSYM; }
-
-// the links of the nonzeros whose row is in [row_lo, row_hi) (1-based, half-open); zero elsewhere
-i64 oracle_links_partial(Oracle& f, i64 row_lo, i64 row_hi, u32* d_prev_out) {
-  CPB_REQUIRE(f.dev.kind == CPB_MODEL_CONNECTIVITY || f.dev.kind == CPB_MODEL_MONOSYM, "streaming links exist for connectivity-type models only");
-  auto ls = build_link_stream(*f.A, model_uses_dia(f.dev.kind), row_lo - 1, row_hi - 1, false, false, /*as_pos=*/true);
-  if (d_prev_out && ls->Ne) CPB_CUDA(cudaMemcpyAsync(d_prev_out, ls->prev.get(), ls->Ne * sizeof(u32), cudaMemcpyDeviceToDevice, ctx().stream));
-  CPB_CUDA(cudaStreamSynchronize(ctx().stream));
-  const i64 Ne = (i64)ls->Ne;
-  f.ls = std::move(ls);  // keeps colidx / P; prev is replaced by oracle_set_links
-  f.ls_complete = false;
-  return Ne;
-}
-
-// adopts the combined link array (all ranks' partial arrays reduced with MAX)
-void oracle_set_links(Oracle& f, const u32* d_prev, i64 Ne) {
-  CPB_REQUIRE(f.ls && (i64)f.ls->Ne == Ne, "call cpb_links_partial first (sizes must agree)");
-  if (Ne) CPB_CUDA(cudaMemcpyAsync(f.ls->prev.get(), d_prev, (size_t)Ne * sizeof(u32), cudaMemcpyDeviceToDevice, ctx().stream));
-  CPB_CUDA(cudaMemsetAsync(f.ls->first_count.get(), 0, sizeof(u32), ctx().stream));
-  if (Ne) CPB_LAUNCH(k_count_zero_u32, grid_for((size_t)Ne), 256, 0, f.ls->prev.get(), (size_t)Ne, f.ls->first_count.get());
-  f.ls->h_first_count = -1;
-  f.ls_complete = true;
-}
-
 // ---- oracle_query_batch ---------------------------------------------------------------------------
 template <class T>
 __global__ void __launch_bounds__(256) k_oracle_query(const __grid_constant__ DevOracle o, i64 Q, const i64* __restrict__ qj,
@@ -335,7 +302,7 @@ template <class T> static void bound_T(Oracle& f, i64 K, double out[2]) {
       if (f.ranks_built) {
         c_hi = (T)query_one(f, 1, A.n + 1);
       } else {  // ocl(1, n+1) from the link array alone: nets(1, n+1) = number of non-empty rows
-        if (!f.ls) f.ls = build_link_stream(*f.A, false, 0, (i64)1 << 62, false, false, /*as_pos=*/true);
+        if (!f.ls) f.ls = build_link_stream(*f.A, false, false, false, /*as_pos=*/true);
         if (f.ls->h_first_count < 0) f.ls->h_first_count = count_first_occurrences(*f.ls);
         const i64 nets_all = f.ls->h_first_count;
         c_hi = c[0] + (T)A.n * c[1] + (T)A.N * c[2] + (T)nets_all * c[3];

@@ -579,15 +579,14 @@ void solve_sharded(ShardedMatrix& S, const cpb_model* mdl, int method, double ep
   auto f = oracle_create(S.M, mdl, nullptr, 0);  // (the monotonized symmetric model checks that A is square, on every rank alike)
   const bool dia = mdl->kind == CPB_MODEL_MONOSYM;
   f->ls = sharded_link_stream(S, dia);
-  f->ls_complete = true;
   const double t1 = now_ms();
   const int cap = std::min(probe_cluster_capacity(true), 15);
   const int per = std::max(1, std::min(cap, 255 / S.world));
   const int nodes = per * S.world;
-  BisectRun* run = bisect_begin(*f, method == CPB_SPLIT_LAZY_BISECT_COST, eps, K, nodes, nullptr, nullptr, nullptr);
+  BisectRunPtr run = bisect_begin(*f, method == CPB_SPLIT_LAZY_BISECT_COST, eps, K, nodes);
   int rounds = 0;
   double coll_bytes = 0;
-  try {
+  {
     ProfScope prof("probe");
     int* res = nullptr;
     double* c = nullptr;
@@ -612,11 +611,8 @@ void solve_sharded(ShardedMatrix& S, const cpb_model* mdl, int method, double ep
       if (bisect_advance(*run, true)) { done = true; break; }
     }
     CPB_REQUIRE(done, "bisection did not terminate (eps too small for Float64?)");
-  } catch (...) {
-    bisect_finish(run, nullptr);
-    throw;
   }
-  bisect_finish(run, h_spl_out);
+  bisect_finish(*run, h_spl_out);
   const double t2 = now_ms();
   g_shard_stats[0] = S.world;
   g_shard_stats[1] = t1 - t0;                      // link construction incl. carry + all-gather, host clock (asynchronous part excluded)
@@ -635,22 +631,16 @@ void solve_sharded_emulated(Matrix& A, const cpb_model* mdl, int method, double 
   CPB_REQUIRE(world >= 1 && world <= 16, "1..16 emulated ranks");
   auto f = oracle_create(A, mdl, nullptr, 0);
   f->ls = emulated_sharded_link_stream(A, world, mdl->kind == CPB_MODEL_MONOSYM);
-  f->ls_complete = true;
   const int cap = std::min(probe_cluster_capacity(true), 15);
   const int per = std::max(1, std::min(cap, 255 / world));
-  BisectRun* run = bisect_begin(*f, method == CPB_SPLIT_LAZY_BISECT_COST, eps, K, per * world, nullptr, nullptr, nullptr);
-  try {
-    bool done = false;
-    for (int guard = 0; guard < 4096 && !done; ++guard) {
-      if (bisect_is_done(*run)) break;
-      for (int r = 0; r < world; ++r) bisect_probe(*run, r * per, (r + 1) * per);
-      done = bisect_advance(*run, true);
-    }
-  } catch (...) {
-    bisect_finish(run, nullptr);
-    throw;
+  BisectRunPtr run = bisect_begin(*f, method == CPB_SPLIT_LAZY_BISECT_COST, eps, K, per * world);
+  bool done = false;
+  for (int guard = 0; guard < 4096 && !done; ++guard) {
+    if (bisect_is_done(*run)) break;
+    for (int r = 0; r < world; ++r) bisect_probe(*run, r * per, (r + 1) * per);
+    done = bisect_advance(*run, true);
   }
-  bisect_finish(run, h_spl_out);
+  bisect_finish(*run, h_spl_out);
 }
 
 // ---- adjointpattern of a sharded matrix ---------------------------------------------------------------------------------

@@ -1,7 +1,9 @@
-"""Multi-GPU plumbing: one process per GPU over ``torch.distributed`` (NCCL on the GPU box, gloo in the
-CPU tests).  The path shards by INDEPENDENT problems (SURVEY.md section 8e: stripe solves on different
-matrices / the two sides of a plaid alternation share nothing), so there is no data-path collective:
-ranks take problems round-robin, results and device timings are combined with one small collective.
+"""Multi-GPU plumbing around ``torch.distributed``, one process per GPU (NCCL on a GPU machine, gloo in the CPU tests).
+
+- Independent problems (SURVEY.md section 8e: stripe solves on different matrices / the two sides of a plaid alternation
+  share nothing) are dealt to the ranks round-robin; results and device timings are combined with one small collective.
+- ONE stripe solve over several GPUs runs inside the library (``cp.partition_stripe_sharded``, NCCL owned by the
+  library); ``library_communicator`` creates that communicator from the host framework's process group.
 """
 from __future__ import annotations
 
@@ -33,107 +35,6 @@ def gather_split_vectors(local: dict, n_problems: int, K: int, device="cpu") -> 
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         dist.all_reduce(table, op=dist.ReduceOp.SUM)  # disjoint rows: SUM == gather
     return table.cpu().numpy()
-
-
-# ---------------------------------------------------------------------------------------------------
-# Sharding ONE bisection across ranks (BASELINE.json north_star: "candidate-threshold sets of the
-# bisection ... NCCL carries only the exchange of feasible thresholds").  Every rank holds the matrix
-# and builds the link array; per round the 2^depth - 1 thresholds of the speculation tree are split
-# into contiguous node ranges, one per rank; the per-node results (feasible?, threshold, split
-# vector) are exchanged with one all-gather; every rank then walks the same tree, so all ranks hold
-# the same state and the same final split vector.  The threshold sequence is the reference's, so the
-# result is identical to the single-GPU (and the CPU) one.
-# ---------------------------------------------------------------------------------------------------
-
-
-def node_slots(world: int, capacity: int = 15):
-    """-> (nodes of the round's speculation tree, nodes per rank).  ``capacity`` = probe clusters one GPU keeps
-    resident (``cpb_probe_cluster_capacity``: 15 on B200 for the streaming probes); the tree is the first
-    world * capacity nodes of the bisection tree in heap order (at most 255)."""
-    per = max(1, min(capacity, 255 // max(world, 1)))
-    return per * world, per
-
-
-def row_block(m: int, rank: int, world: int):
-    """1-based half-open row range of ``rank``: [lo, hi)."""
-    return 1 + (m * rank) // world, 1 + (m * (rank + 1)) // world
-
-
-def build_links_sharded(ocl, m: int, n: int, nnz: int, rank: int, world: int, emulate_ranks: bool = False):
-    """Link construction by row blocks (north_star: "column blocks of the oracle-construction sweep" -- the sweep
-    is independent per ROW, so rows are the natural shard): every rank sorts only the nonzeros of its rows, the
-    partial link arrays (zero outside the block) are combined with one element-wise MAX all-reduce."""
-    from . import api
-
-    dev = torch.device("cuda", torch.cuda.current_device())
-    prev = torch.zeros(nnz + n, dtype=torch.int32, device=dev)
-    torch.cuda.synchronize()
-    if emulate_ranks:
-        acc = torch.zeros_like(prev)
-        ne = 0
-        for r in range(world):
-            lo, hi = row_block(m, r, world)
-            ne = ocl.links_partial(lo, hi, prev.data_ptr())
-            api.synchronize()
-            acc = torch.maximum(acc, prev)
-            torch.cuda.synchronize()
-        prev = acc
-    else:
-        lo, hi = row_block(m, rank, world)
-        ne = ocl.links_partial(lo, hi, prev.data_ptr())
-        api.synchronize()
-        if world > 1:
-            dist.all_reduce(prev, op=dist.ReduceOp.MAX)
-            torch.cuda.synchronize()
-    ocl.set_links(prev.data_ptr(), ne)
-    return prev
-
-
-def partition_stripe_sharded(A, K, method, rank: int = 0, world: int = 1, emulate_ranks: bool = False, shard_links: bool = True):
-    """``partition_stripe(A, K, BisectCost/LazyBisectCost...)`` with the threshold tree of every round
-    sharded over ``world`` ranks (torch.distributed must be initialised with a CUDA-capable backend when
-    world > 1).  ``emulate_ranks`` probes all node ranges from this one process (single-GPU test of the
-    sharding logic)."""
-    from . import api
-
-    streaming = getattr(api.T.split_constrained(api.T.split_method_code(method)[1])[0], "kind", -1) in (api.T.MODEL_CONNECTIVITY, api.T.MODEL_MONOSYM)
-    nodes, per = node_slots(world, min(api.probe_cluster_capacity(streaming), 15))
-    slots = per * world
-    K = int(K)
-    dev = torch.device("cuda", torch.cuda.current_device())
-    res = torch.zeros(slots, dtype=torch.int32, device=dev)
-    thr = torch.zeros(slots, dtype=torch.float64, device=dev)
-    spl = torch.zeros((slots, K + 2), dtype=torch.int32, device=dev)
-    torch.cuda.synchronize()
-    _, spec, _ = api.T.split_method_code(method)
-    ocl = api.StripeOracle(spec, A)
-    try:
-        if streaming and shard_links and world > 1:
-            build_links_sharded(ocl, ocl.dm.m, ocl.dm.n, ocl.dm.nnz, rank, world, emulate_ranks)
-        run = api.StepwiseBisection(ocl, method, K, nodes, res.data_ptr(), thr.data_ptr(), spl.data_ptr())
-        nodes = run.nodes
-        done = nodes == 0
-        guard = 0
-        while True:
-            if emulate_ranks:
-                for r in range(world):
-                    run.probe(r * per, min((r + 1) * per, nodes))
-            else:
-                run.probe(rank * per, min((rank + 1) * per, nodes))
-            api.synchronize()
-            if world > 1 and not emulate_ranks:
-                lo, hi = rank * per, (rank + 1) * per
-                dist.all_gather_into_tensor(res, res[lo:hi].clone())
-                dist.all_gather_into_tensor(thr, thr[lo:hi].clone())
-                dist.all_gather_into_tensor(spl, spl[lo:hi].clone())
-                torch.cuda.synchronize()
-            done = run.advance()
-            guard += 1
-            if done or guard > 4096:
-                break
-        return run.finish()
-    finally:
-        ocl.close()
 
 
 def library_communicator(cp, dist_mod, rank: int, world: int):

@@ -28,8 +28,7 @@
  * Streams
  *   - entry points that take HOST arrays return when their results are in those arrays.
  *   - entry points that take or fill DEVICE arrays (cpb_matrix_create_device,
- *     cpb_oracle_query_device, cpb_links_partial, cpb_oracle_set_links, cpb_bisect_probe and the
- *     other stepwise bisection calls) ENQUEUE work on the library's own non-blocking stream and may
+ *     cpb_oracle_query_device) ENQUEUE work on the library's own non-blocking stream and may
  *     return before it has run: arrays produced on another stream (torch's, the caller's) must be
  *     complete before the call, and cpb_synchronize() must return before another stream reads
  *     what the call wrote.
@@ -212,36 +211,6 @@ int cpb_partition_stripe_weighted(cpb_oracle* f, int method, cpb_oracle* w, int6
  * Builds w's dominance index on first use (a second wavelet index when f and w are different oracles). */
 int cpb_weight_windows(cpb_oracle* w, int64_t w_max, int64_t* first_fit_out, int64_t* reach_out);
 
-/* Link construction sharded by row blocks (the sweep of SparseColorArrays.jl:103-118 / :72-99 touches every row
- * independently): cpb_links_partial builds the links of the nonzeros whose row lies in [row_lo, row_hi) (1-based,
- * half-open) into d_prev_out (DEVICE buffer with room for nnz + n uint32; *ne_out <= nnz + n entries are written,
- * zero for all nonzeros outside the row block); the ranks combine their arrays with an element-wise MAX all-reduce and hand the result back with
- * cpb_oracle_set_links.  Connectivity-type models only (their probes stream this array). */
-int cpb_links_partial(cpb_oracle* f, int64_t row_lo, int64_t row_hi, uint32_t* d_prev_out, int64_t* ne_out);
-int cpb_oracle_set_links(cpb_oracle* f, const uint32_t* d_prev, int64_t ne);
-
-/* The same bisection (BisectCostBottleneckSplitter.jl:41-60 / LazyBisect...:237-255) as explicit steps, so that
- * the speculative thresholds of a round -- `nodes` (<= 255) nodes of the bisection tree, slot t holding the t-th
- * node of the round's plan (the subtree the sequential loop is most likely to visit; every rank derives the same
- * plan from the same state; CPB_BISECT_PLAN=0 selects the complete tree in heap order) -- can be probed by
- * different GPUs (one process per GPU):
- *   begin   builds what the probes need, computes bound_stripe, sets up the round state.  d_node_res (int32
- *           per node: 0 = loop condition already false, 1 = infeasible, 2 = feasible), d_node_c (double per
- *           node), d_node_spl ((K+2) int32 per node, 1-based split points in [1..K+1]) are DEVICE buffers for
- *           `nodes` nodes in heap order; pass NULL for library-owned buffers.
- *   probe   launches the probes of nodes [node_lo, node_hi) of the current round (asynchronous).
- *   advance walks the tree by feasibility; every node of the round must be present in the buffers (after the
- *           caller's all-gather).  done_out = 1 when c_lo (1 + eps) >= c_hi.
- *   finish  copies spl_hi[K+1] out (spl_out may be NULL to abandon) and frees the handle. */
-typedef struct cpb_bisect cpb_bisect;
-int cpb_bisect_begin(cpb_oracle* f, int method, double eps, int64_t K, int nodes, int32_t* d_node_res, double* d_node_c,
-                     int32_t* d_node_spl, cpb_bisect** out);
-int cpb_bisect_probe(cpb_bisect* b, int node_lo, int node_hi);
-/* Number of 8-CTA probe clusters (= thresholds) this GPU keeps resident at once; streaming = 1 for the
- * link-array probes, 0 for the dominance-index probes.  Sizes the per-rank node ranges. */
-int cpb_probe_cluster_capacity(int streaming, int* out);
-int cpb_bisect_advance(cpb_bisect* b, int* done_out);
-int cpb_bisect_finish(cpb_bisect* b, int64_t* spl_out);
 /* The speculation plan of one round, as a pure host computation (no device needed): the `nodes` nodes (heap indices in
  * the bisection tree, root = 0, left child 2i+1 = "probe i was feasible"; -1 = unused slot) that are probed concurrently
  * when the bracket is (c_lo, c_hi], the initial bracket was (c_lo0, c_hi0] and `upper_bound` (0 = unknown) bounds the

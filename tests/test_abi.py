@@ -24,7 +24,7 @@ def test_library_exports_every_declared_symbol():
     for s in syms:
         assert hasattr(lib, s), f"libchainb200.so does not export {s}"
     assert sorted(cp.api.ABI_SYMBOLS) == syms
-    assert lib.cpb_version() == 100
+    assert lib.cpb_version() == 101
 
 
 def test_model_struct_layout_matches_header():

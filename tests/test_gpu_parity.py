@@ -915,49 +915,30 @@ def test_degenerate_inputs(ref):
         assert np.array_equal(B.colptr, Br.colptr) and np.array_equal(B.rowval, Br.rowval)
 
 
-def test_sharded_bisection_emulated_ranks(ref):
-    """The multi-GPU threshold sharding with all node ranges probed from one process: begin / probe(range) /
-    advance / finish through the C ABI with caller-owned (torch) node buffers."""
-    import torch
-
-    from chainb200 import parallel
-
-    torch.cuda.set_device(0)
-    A = synth.erdos_renyi(30000, 10)
-    G = synth.random_geometric(20000)
-    sym = cp.AffineMonotonizedSymmetricConnectivityModel(0, 0, 1, 100, 4)
-    for M, K, mtd in [(A, 16, cp.BisectCostBottleneckSplitter(AFF, 0.01)), (A, 64, cp.LazyBisectCostBottleneckSplitter(AFF, 0.001)),
-                      (G, 32, cp.LazyBisectCostBottleneckSplitter(sym, 0.1)), (A, 8, cp.BisectCostBottleneckSplitter(cp.AffineWorkModel(0, 10, 1), 0.01))]:
-        exp = ref.partition_stripe(M, K, mtd).spl
-        for world in (1, 2, 4, 8):
-            got = parallel.partition_stripe_sharded(M, K, mtd, world=world, emulate_ranks=True)
-            assert np.array_equal(got.spl, exp), (type(mtd).__name__, K, world)
-
-
 def test_sharded_solve_emulated_ranks_and_single_rank(ref):
     """csrc/sharded.cu on one GPU: the block-wise link construction with the carried "last position" array and rounds of
     world x 15 thresholds, the ranks played one after the other (cpb_partition_stripe_sharded_emulated), and the real entry
     point with a world of one (no communicator)."""
-    cases = [(synth.erdos_renyi(30000, 10), 16, 0.01), (synth.rmat(14, 16 << 14), 128, 0.01), (synth.laplacian5(40), 7, 0.001),
+    A = synth.erdos_renyi(30000, 10)
+    cases = [(A, 16, 0.01), (synth.rmat(14, 16 << 14), 128, 0.01), (synth.laplacian5(40), 7, 0.001),
              (synth.banded(3000, 20), 5, 0.05), (cp.SparseMatrixCSC(4, 3, [1, 1, 1, 1], np.zeros(0, dtype=np.int64)), 2, 0.1)]
-    for A, K, eps in cases:
-        for mtd in (cp.LazyBisectCostBottleneckSplitter(AFF, eps), cp.BisectCostBottleneckSplitter(cp.AffineConnectivityModel(0.0, 3.0, 1.0, 7.0), eps)):
-            exp = ref.partition_stripe(A, K, mtd).spl
-            for world in (1, 2, 3, 8):
-                got = cp.partition_stripe_sharded_emulated(A, K, mtd, world).spl
-                assert np.array_equal(got, exp), (A.n, K, world)
-            assert np.array_equal(cp.partition_stripe_sharded(A, K, mtd).spl, exp), (A.n, K, "world of one")
-    with pytest.raises(cp.CpbError):
-        cp.partition_stripe_sharded(cases[0][0], 4, cp.LazyBisectCostBottleneckSplitter(cp.AffineWorkModel(0, 1, 1), 0.1))
-
-
-def test_node_slots():
-    from chainb200 import parallel
-
-    assert parallel.node_slots(1) == (15, 15)
-    assert parallel.node_slots(2) == (30, 15)
-    assert parallel.node_slots(8) == (120, 15)
-    assert parallel.node_slots(32) == (224, 7)
+    runs = [(M, K, mtd) for M, K, eps in cases
+            for mtd in (cp.LazyBisectCostBottleneckSplitter(AFF, eps), cp.BisectCostBottleneckSplitter(cp.AffineConnectivityModel(0.0, 3.0, 1.0, 7.0), eps))]
+    sym = cp.AffineMonotonizedSymmetricConnectivityModel(0, 0, 1, 100, 4)
+    runs += [(A, 16, cp.BisectCostBottleneckSplitter(AFF, 0.01)), (A, 64, cp.LazyBisectCostBottleneckSplitter(AFF, 0.001)),
+             (synth.random_geometric(20000), 32, cp.LazyBisectCostBottleneckSplitter(sym, 0.1))]
+    for M, K, mtd in runs:
+        exp = ref.partition_stripe(M, K, mtd).spl
+        for world in (1, 2, 3, 4, 8):
+            got = cp.partition_stripe_sharded_emulated(M, K, mtd, world).spl
+            assert np.array_equal(got, exp), (M.n, K, type(mtd).__name__, world)
+        assert np.array_equal(cp.partition_stripe_sharded(M, K, mtd).spl, exp), (M.n, K, type(mtd).__name__, "world of one")
+    # the sharded solve streams links: a work model (bisection on the dominance index) is refused, emulated or not
+    for K, work in ((4, cp.LazyBisectCostBottleneckSplitter(cp.AffineWorkModel(0, 1, 1), 0.1)), (8, cp.BisectCostBottleneckSplitter(cp.AffineWorkModel(0, 10, 1), 0.01))):
+        with pytest.raises(cp.CpbError):
+            cp.partition_stripe_sharded(A, K, work)
+        with pytest.raises(cp.CpbError):
+            cp.partition_stripe_sharded_emulated(A, K, work, 2)
 
 
 def test_c_abi_example_binary(ref):

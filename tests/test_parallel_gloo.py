@@ -59,21 +59,6 @@ def test_two_rank_sharding_gloo():
         assert table[i] == exp.tolist()
 
 
-def test_row_blocks_cover_all_rows():
-    import sys
-
-    for p in (ROOT,):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    from chainb200 import parallel
-
-    for m in (1, 7, 100, 1000003):
-        for world in (1, 2, 3, 8):
-            blocks = [parallel.row_block(m, r, world) for r in range(world)]
-            assert blocks[0][0] == 1 and blocks[-1][1] == m + 1
-            assert all(blocks[i][1] == blocks[i + 1][0] for i in range(world - 1))
-
-
 # ---------------------------------------------------------------------------------------------------
 # The sharded link construction of csrc/sharded.cu as a host model over gloo: every rank owns the block of CSC positions
 # cpb_shard_range gives it, links inside the block come from the block alone, the per-row "last position" array travels
