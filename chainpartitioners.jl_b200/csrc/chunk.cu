@@ -18,6 +18,7 @@
 //   chain unravel      the pointer chain (bounded jumps) is marked block-wise the same way and
 //                      compacted with a scan.
 #include <algorithm>
+#include <type_traits>
 #include "engine.cuh"
 #include "primitives.cuh"
 
@@ -351,14 +352,24 @@ __global__ void k_chunk_seq_f64(const double* __restrict__ C, u32 n, int W, doub
 }
 
 // ConvexTotalChunker{ConstrainedCost} pointer rule (SURVEY App. B; ConvexTotalChunker.jl:211-265):
-// windows B_t = (1 + t W, 1 + (t+1) W]; within the current window the leftmost argmin, unless the
-// previous window is strictly better -- then its rightmost argmin.
+// windows B_t = (b_t, b_t+1]; within the current window the leftmost argmin, unless the
+// previous window is strictly better -- then its rightmost argmin.  The window ends b_t come from
+// k_convex_bounds (bnd, nb of them); bnd == nullptr: a vertex-count weight, b_t = 1 + t W.
 template <class T>
-__global__ void k_convex_ptr(const T* __restrict__ C, const T* __restrict__ cst, u32 n, int W, u32* __restrict__ ptr) {
+__global__ void k_convex_ptr(const T* __restrict__ C, const T* __restrict__ cst, u32 n, int W, const u32* __restrict__ bnd, const u32* __restrict__ nb,
+                             u32* __restrict__ ptr) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     const u32 jp = (u32)i + 2;
-    const u32 j0 = 1 + ((jp - 2) / W) * W;
+    u32 j0 = 1 + ((jp - 2) / W) * W;
+    if (bnd) {  // the last window end before jp (bnd[0] = 1 < jp)
+      u32 lo = 0, hi = *nb - 1;
+      while (lo < hi) {
+        const u32 mid = (lo + hi + 1) >> 1;
+        if (bnd[mid] < jp) lo = mid; else hi = mid - 1;
+      }
+      j0 = bnd[lo];
+    }
     const T* row = C + (size_t)(jp - 1) * W;
     bool has_in = false, has_pr = false;
     T vin = 0, vpr = 0;
@@ -374,6 +385,26 @@ __global__ void k_convex_ptr(const T* __restrict__ C, const T* __restrict__ cst,
     }
     ptr[jp] = (!has_pr || (has_in && vin <= vpr)) ? ain : apr;
   }
+}
+
+// Window ends of a pin-weighted constraint: the reference moves from window to window by the weight's reach
+// (ConvexTotalChunker.jl:211-265) -- b_0 = 1, b_t+1 = the last j' with w(b_t, j') <= w_max (at least b_t + 1) -- and a pin
+// term makes that reach depend on the column lengths.  One thread walks the chain with binary searches on pos.
+__global__ void k_convex_bounds(const u32* __restrict__ pos, u32 n, int W, i64 wa, i64 wbv, i64 wbp, i64 w_max, u32* __restrict__ bnd,
+                                u32* __restrict__ nb) {
+  if (blockIdx.x || threadIdx.x) return;
+  u32 b = 1, k = 0;
+  bnd[k++] = 1;
+  while (b < n + 1) {
+    u32 lo = b + 1, hi = min(b + (u32)W, n + 1);
+    while (lo < hi) {
+      const u32 mid = (lo + hi + 1) >> 1;
+      if (wa + (i64)(mid - b) * wbv + ((i64)pos[mid - 1] - (i64)pos[b - 1]) * wbp <= w_max) lo = mid; else hi = mid - 1;
+    }
+    b = lo;
+    bnd[k++] = b;
+  }
+  *nb = k;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -685,6 +716,16 @@ static void pack_dynamic(Matrix& A, Oracle& f, int method, const cpb_constraint*
   trace_mark("window_hist");
   const size_t cells = ((size_t)n + 1) * W;
   DBuf<u32> ptr((size_t)n + 3);
+  auto convex_ptr = [&](const auto* C, const auto* cst) {
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(C)>>;
+    DBuf<u32> bnd, nb;
+    if (tm.wbp != 0) {  // pin-weighted windows: their ends follow the column lengths
+      bnd.alloc((size_t)n + 2);
+      nb.alloc(1);
+      CPB_LAUNCH(k_convex_bounds, 1, 32, 0, A.pos.get(), n, W, tm.wa, tm.wbv, tm.wbp, tm.w_max, bnd.get(), nb.get());
+    }
+    CPB_LAUNCH(k_convex_ptr<T>, grid_for(n), 256, 0, C, cst, n, W, (const u32*)bnd.get(), (const u32*)nb.get(), ptr.get());
+  };
   if (!is_f) {
     DBuf<i64> C(cells), cst((size_t)n + 2);
     {
@@ -702,7 +743,7 @@ static void pack_dynamic(Matrix& A, Oracle& f, int method, const cpb_constraint*
       CPB_CUDA(cudaMemcpyAsync(&last, cst.get() + n + 1, sizeof(i64), cudaMemcpyDeviceToHost, ctx().stream));
       CPB_CUDA(cudaStreamSynchronize(ctx().stream));
       if (last >= CH_INF) throw Error(CPB_ERR_INFEASIBLE, "width constraint cannot be met (reference: @assert j0 < j')");
-      if (method == CPB_PACK_CONVEX_TOTAL) CPB_LAUNCH(k_convex_ptr<i64>, grid_for(n), 256, 0, C.get(), cst.get(), n, W, ptr.get());
+      if (method == CPB_PACK_CONVEX_TOTAL) convex_ptr(C.get(), cst.get());
     }
   } else {
     DBuf<double> C(cells), cst((size_t)n + 2);
@@ -716,7 +757,7 @@ static void pack_dynamic(Matrix& A, Oracle& f, int method, const cpb_constraint*
     CPB_CUDA(cudaMemcpyAsync(&last, cst.get() + n + 1, sizeof(double), cudaMemcpyDeviceToHost, ctx().stream));
     CPB_CUDA(cudaStreamSynchronize(ctx().stream));
     if (!(last < INFINITY)) throw Error(CPB_ERR_INFEASIBLE, "width constraint cannot be met (reference: @assert j0 < j')");
-    if (method == CPB_PACK_CONVEX_TOTAL) CPB_LAUNCH(k_convex_ptr<double>, grid_for(n), 256, 0, C.get(), cst.get(), n, W, ptr.get());
+    if (method == CPB_PACK_CONVEX_TOTAL) convex_ptr(C.get(), cst.get());
   }
   trace_mark("chunk_dp");
   ProfScope prof("unravel_chunks");

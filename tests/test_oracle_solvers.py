@@ -577,6 +577,7 @@ def test_dynamic_total_chunker(ref, fixtures):
     """test_Partitioners.jl:225-248: width <= w_max, optimal total; App. B: leftmost argmin."""
     rng = np.random.default_rng(16)
     mats = [fixtures["LPnetlib/lpi_itest6"]] + [sprand(rng, m, n, 0.3) for m in [2, 5, 9] for n in [1, 2, 5, 11, 17]]
+    mats += [sprand(rng, m, n, p) for m, n, p in [(6, 90, 0.15), (20, 130, 0.05)]]  # the device's wide window templates
     for A in mats:
         Pi = ref.pack_stripe(ref.adjointpattern(A), cp.EquiChunker(2))
         for mdl in [cp.AffineConnectivityModel(0, 3, 1, 3), cp.AffineConnectivityModel(0, 0, 0, 1),
@@ -584,7 +585,7 @@ def test_dynamic_total_chunker(ref, fixtures):
                     cp.BlockComponentCostModel(int, 1, 3, (1, cp.identity), (1, cp.identity)),
                     cp.ColumnBlockComponentCostModel(int, 3, lambda w: 1 + w)]:
             C = cost_matrix(mdl, A, Pi)
-            for w_max in [1, 2, 4, 8]:
+            for w_max in [1, 2, 4, 8, 16, 17, 32, 33, 64]:
                 Phi = ref.pack_stripe(A, cp.DynamicTotalChunker(cp.ConstrainedCost(mdl, cp.VertexCount(), w_max)), Pi)
                 check_split(Phi.spl, A.n)
                 assert np.all(np.diff(Phi.spl) <= w_max)
@@ -625,6 +626,7 @@ def test_convex_chunkers(ref, fixtures):
     """test_Partitioners.jl:250-275 (optimal value); SURVEY E5/E6 tie rules for convex costs."""
     rng = np.random.default_rng(17)
     mats = [fixtures["LPnetlib/lpi_itest6"]] + [sprand(rng, m, n, 0.3) for m in [2, 5, 9] for n in [1, 2, 5, 11, 17, 30]]
+    mats += [sprand(rng, m, n, p) for m, n, p in [(6, 90, 0.15), (20, 130, 0.05)]]  # the device's wide window templates
     for A in mats:
         for mdl in [cp.AffineConnectivityModel(0, 0, 0, 1), cp.AffineConnectivityModel(0, 3, 1, 3), cp.AffineConnectivityModel(1, 0, 0, 1),
                     cp.AffineConnectivityModel(-0.5, 0.0, 0.0, 1.0)]:
@@ -633,7 +635,7 @@ def test_convex_chunkers(ref, fixtures):
             check_split(Phi.spl, A.n)
             assert objective(C, Phi.spl, True) == brute_chunk_optimum(C, A.n, None)
             assert Phi.spl.tolist() == leftmost_chunk_dp(C, A.n, None)[0]
-            for w_max in [1, 2, 3, 4, 8]:
+            for w_max in [1, 2, 3, 4, 8, 16, 17, 32, 33, 64]:
                 Phi = ref.pack_stripe(A, cp.ConvexTotalChunker(cp.ConstrainedCost(mdl, cp.VertexCount(), w_max)))
                 check_split(Phi.spl, A.n)
                 assert np.all(np.diff(Phi.spl) <= w_max)
@@ -686,8 +688,9 @@ def strict_definition(A, w_max):
 def test_overlap_and_strict(ref, fixtures):
     rng = np.random.default_rng(19)
     mats = [fixtures["LPnetlib/lpi_itest6"], fixtures["Pajek/GD99_c"]] + [sprand(rng, m, n, p) for m in [3, 6] for n in [1, 2, 9, 25] for p in [0.3, 0.8]]
+    mats += [sprand(rng, m, n, p) for m, n, p in [(2, 100, 0.9), (3, 120, 0.8), (6, 70, 0.5)]]  # runs of identical / overlapping columns
     for A in mats:
-        for w_max in [1, 2, 4, 8]:
+        for w_max in [1, 2, 4, 8, 16, 17, 32, 33, 64]:
             for rho in [0.9, 0.8, 0.7, 0.3]:
                 box = [None]
                 Phi = ref.pack_stripe(A, cp.OverlapChunker(rho, w_max), n_nets=box)
