@@ -932,7 +932,7 @@ static int env_int(const char* name, int dflt) {
 
 // nets(1, n+1) = number of non-empty rows = links equal to 0 (ConnectivityCosts.jl:32 needs ocl(1, n+1))
 i64 count_first_occurrences(const LinkStream& ls) {
-  // counted by k_link_prev while it wrote the links
+  // counted while the links were written (k_lt_link, or the one-sweep link kernels of the k_link_prev phase)
   u32 h = 0;
   CPB_CUDA(cudaMemcpyAsync(&h, ls.first_count.get(), sizeof(u32), cudaMemcpyDeviceToHost, ctx().stream));
   CPB_CUDA(cudaStreamSynchronize(ctx().stream));

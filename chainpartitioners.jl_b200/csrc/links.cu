@@ -12,74 +12,27 @@
 
 namespace cpb {
 
-// sorted (row, q) pairs of a matrix: the transpose order
-struct TransposeOrder {
-  DBuf<u32> k0, v0, k1, v1;
-  u32* keys = nullptr;  // rows, ascending; ties keep CSC order (ascending column)
-  u32* q = nullptr;     // CSC position of each entry
-};
-
-static void transpose_order(const u32* row, size_t N, u64 max_row, TransposeOrder& t) {
-  t.k0.alloc(N); t.v0.alloc(N); t.k1.alloc(N); t.v1.alloc(N);
-  const int which = radix_sort_pairs_iota(row, t.k0.get(), t.v0.get(), t.k1.get(), t.v1.get(), N, bits_for(max_row));
-  t.keys = which ? t.k1.get() : t.k0.get();
-  t.q = which ? t.v1.get() : t.v0.get();
-}
-
 static unsigned grid_for(size_t n) { return (unsigned)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, (size_t)ctx().sm_count * 32)); }
 
-// prev[q] = 1-based previous column holding the same row, 0 if none; as_pos: 1 + CSC position of that previous nonzero
-// instead (what the streaming probes compare against the part's first position -- no column lookup at all)
-__global__ void k_link_prev(const u32* __restrict__ sk, const u32* __restrict__ sq, const u32* __restrict__ colidx,
-                            u32* __restrict__ prev, size_t N, u32* __restrict__ first_count, int as_pos) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  u32 firsts = 0;  // links equal to 0 = first occurrence of a row = number of non-empty rows
-  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += stride) {
-    u32 link = 0;
-    if (p > 0 && sk[p - 1] == sk[p]) link = as_pos ? sq[p - 1] + 1u : __ldg(colidx + sq[p - 1]) + 1u;
-    prev[sq[p]] = link;
-    firsts += link == 0u;
-  }
-  firsts = __reduce_add_sync(0xffffffffu, firsts);
-  if ((threadIdx.x & 31) == 0 && firsts) atomicAdd(first_count, firsts);
-}
-
-// The same links as values in sorted order (no scatter yet): lv[p] = link of the nonzero sq[p]
-__global__ void k_link_values(const u32* __restrict__ sk, const u32* __restrict__ sq, const u32* __restrict__ colidx, u32* __restrict__ lv, size_t N,
-                              u32* __restrict__ first_count, int as_pos) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  u32 firsts = 0;
-  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += stride) {
-    u32 link = 0;
-    if (p > 0 && sk[p - 1] == sk[p]) link = as_pos ? sq[p - 1] + 1u : __ldg(colidx + sq[p - 1]) + 1u;
-    lv[p] = link;
-    firsts += link == 0u;
-  }
-  firsts = __reduce_add_sync(0xffffffffu, firsts);
-  if ((threadIdx.x & 31) == 0 && firsts) atomicAdd(first_count, firsts);
-}
-// prev[q[p]] = v[p], pairs grouped by destination window: consecutive CTAs write into the same few megabytes
-__global__ void k_scatter_pairs(const u32* __restrict__ q, const u32* __restrict__ v, u32* __restrict__ prev, size_t N) {
-  const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (p < N) prev[q[p]] = v[p];
-}
-
-__global__ void k_head_flags(const u32* __restrict__ sk, size_t N, u32* __restrict__ flags) {
+// flags[p] = 1 iff the sorted (row << 32 | position) pair p starts a row run; flags[N] = 0
+__global__ void k_head_flags(const u64* __restrict__ sorted, size_t N, u32* __restrict__ flags) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p <= N; p += stride)
-    flags[p] = (p < N && (p == 0 || sk[p - 1] != sk[p])) ? 1u : 0u;
+    flags[p] = (p < N && (p == 0 || (u32)(sorted[p - 1] >> 32) != (u32)(sorted[p] >> 32))) ? 1u : 0u;
 }
 
 // one point per non-empty row: x = last column, val = first column (both 1-based)
-__global__ void k_selfnet_points(const u32* __restrict__ sk, const u32* __restrict__ sq, const u32* __restrict__ colidx,
-                                 const u32* __restrict__ headscan, size_t N, u32* __restrict__ x, u32* __restrict__ val) {
+__global__ void k_selfnet_points(const u64* __restrict__ sorted, const u32* __restrict__ colidx, const u32* __restrict__ headscan, size_t N,
+                                 u32* __restrict__ x, u32* __restrict__ val) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += stride) {
-    const bool head = (p == 0) || (sk[p - 1] != sk[p]);
-    const bool tail = (p + 1 == N) || (sk[p + 1] != sk[p]);
+    const u64 cur = sorted[p];
+    const u32 r = (u32)(cur >> 32);
+    const bool head = (p == 0) || ((u32)(sorted[p - 1] >> 32) != r);
+    const bool tail = (p + 1 == N) || ((u32)(sorted[p + 1] >> 32) != r);
     if (head | tail) {
       const u32 run = headscan[p] - (head ? 0u : 1u);
-      const u32 c = __ldg(colidx + sq[p]) + 1u;
+      const u32 c = __ldg(colidx + (u32)cur) + 1u;
       if (head) val[run] = c;
       if (tail) x[run] = c;
     }
@@ -135,7 +88,7 @@ __global__ void k_aug_diag(const u32* __restrict__ pos2, const u32* __restrict__
 // When no row holds more than LT_MAX_DEG nonzeros the stable sort is unnecessary: the nonzeros are dropped into their
 // row's segment in arbitrary order (one atomic cursor per row) and every entry finds its predecessor -- the largest
 // CSC position below its own -- by scanning its row's short segment.  The result does not depend on the
-// order inside the segments.  Heavier rows (power-law matrices) take the radix-sort path below.
+// order inside the segments.  Heavier rows (power-law matrices) take the one-sweep sort (onesweep_links).
 __global__ void k_lt_count(const u32* __restrict__ row, size_t N, u32* __restrict__ cnt) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < N; q += stride) atomicAdd(&cnt[row[q]], 1u);
@@ -293,35 +246,12 @@ bool compute_prev_links(const u32* pos, const u32* row, u32 nrow, u32 ncol, size
     }
   }
   trace_mark("degree_check");
-  const char* wmin_env0 = std::getenv("CPB_WINDOWED_SCATTER_MIN");  // (tests force the windowed form on small inputs; 0 = never)
-  const size_t wmin0 = wmin_env0 ? (size_t)std::atoll(wmin_env0) : ((size_t)1 << 25);
-  const char* os_env = std::getenv("CPB_ONESWEEP");  // 0: the tile-histogram sort of round 1 (kept for comparison)
-  if (onesweep_supported(N) && !(os_env && os_env[0] == '0')) {
-    // one-read-one-write radix passes on packed (row, position) pairs; the window pass forms the links while loading
-    DBuf<u64> a(N), b(N);
-    onesweep_links(row, N, bits_for(nrow ? nrow - 1 : 0), colidx, as_pos, 0u, prev, first_count, nullptr, wmin0, a.get(), b.get());
-    return false;
-  }
-  TransposeOrder t;
-  transpose_order(row, N, nrow ? nrow - 1 : 0, t);
-  trace_mark("sort");
+  if (!N) return false;
   const char* wmin_env = std::getenv("CPB_WINDOWED_SCATTER_MIN");  // (tests force the windowed form on small inputs; 0 = never)
   const size_t wmin = wmin_env ? (size_t)std::atoll(wmin_env) : ((size_t)1 << 25);
-  if (wmin > 0 && N >= wmin) {
-    // the link array no longer fits L2: a scatter in row order touches one HBM sector per 4-byte link (measured 10.9 ms
-    // at N = 2.6e8).  One more partition pass groups the (position, link) pairs by 2^20-position windows (4 MB of `prev`
-    // each), and the scatter of each window stays in L2.
-    ProfScope pk("k_link_prev", (double)N * 12.0);
-    u32* const other_k = (t.keys == t.k0.get()) ? t.k1.get() : t.k0.get();  // the sort's scratch pair
-    u32* const other_v = (t.q == t.v0.get()) ? t.v1.get() : t.v0.get();
-    CPB_LAUNCH(k_link_values, grid_for(N), 256, 0, t.keys, t.q, colidx, other_k, N, first_count, as_pos ? 1 : 0);
-    const int shift = std::max(0, bits_for(N - 1) - 8);
-    radix_partition_pass(t.q, other_k, t.keys, other_v, N, shift);  // t.keys is free once the links are formed
-    CPB_LAUNCH(k_scatter_pairs, (unsigned)((N + 255) / 256), 256, 0, t.keys, other_v, prev, N);
-  } else if (N) {
-    ProfScope pk("k_link_prev", (double)N * 12.0);
-    CPB_LAUNCH(k_link_prev, grid_for(N), 256, 0, t.keys, t.q, colidx, prev, N, first_count, as_pos ? 1 : 0);
-  }
+  // one-read-one-write radix passes on packed (row, position) pairs; the window pass forms the links while loading
+  DBuf<u64> a(N), b(N);
+  onesweep_links(row, N, bits_for(nrow ? nrow - 1 : 0), colidx, as_pos, 0u, prev, first_count, nullptr, wmin, a.get(), b.get());
   return false;
 }
 
@@ -397,15 +327,15 @@ std::unique_ptr<RankStruct> build_rank(const Matrix& A, int which) {
       break;
     }
     case RANK_SELFNET: {
-      TransposeOrder t;
-      transpose_order(A.row.get(), N, m ? m - 1 : 0, t);
+      DBuf<u64> a(N), b(N);
+      const u64* sorted = N ? onesweep_sort_iota(A.row.get(), N, bits_for(m ? m - 1 : 0), a.get(), b.get()) : nullptr;
       DBuf<u32> colidx(N), flags(N + 1), headscan(N + 1);
       expand_columns(A.pos.get(), n, colidx.get(), N);
-      CPB_LAUNCH(k_head_flags, grid_for(N + 1), 256, 0, t.keys, N, flags.get());
+      CPB_LAUNCH(k_head_flags, grid_for(N + 1), 256, 0, sorted, N, flags.get());
       exclusive_scan_u32(flags.get(), headscan.get(), N + 1);
       const size_t R = read_u32(headscan.get() + N);
       DBuf<u32> x(R), val(R);
-      if (N) CPB_LAUNCH(k_selfnet_points, grid_for(N), 256, 0, t.keys, t.q, colidx.get(), headscan.get(), N, x.get(), val.get());
+      if (N) CPB_LAUNCH(k_selfnet_points, grid_for(N), 256, 0, sorted, colidx.get(), headscan.get(), N, x.get(), val.get());
       build_from_points(x, val, R, n, *rs);
       break;
     }
@@ -483,13 +413,8 @@ void build_partwise_columns(const Matrix& A, const u32* asg, u32 K, DBuf<u32>& p
   exclusive_scan_u32(flags.get(), part_head.get(), N + 1);
 }
 
-// adjointpattern(A) (util.jl:67-95): stable sort by row = CSC of the transpose
-__global__ void k_gather_cols(const u32* __restrict__ sq, const u32* __restrict__ colidx, size_t N, u32* __restrict__ out) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += stride) out[p] = colidx[sq[p]];
-}
-
-// the same from packed (row << 32 | position) pairs (one-sweep sort)
+// adjointpattern(A) (util.jl:67-95): stable sort by row = CSC of the transpose; row'[p] = column of the p-th sorted
+// (row << 32 | position) pair, pos'[i] = first sorted index with row >= i, i = 0..m
 __global__ void k_gather_cols_pairs(const u64* __restrict__ sorted, const u32* __restrict__ colidx, size_t N, u32* __restrict__ out) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += stride) out[p] = colidx[(u32)sorted[p]];
@@ -508,28 +433,15 @@ std::unique_ptr<Matrix> adjoint_pattern(const Matrix& A) {
   B->m = A.n; B->n = A.m; B->N = A.N;
   const size_t N = (size_t)A.N;
   ProfScope prof("adjointpattern", (double)(2 * N + A.n + A.m + 2) * 4.0);
-  const char* os_env = std::getenv("CPB_ONESWEEP");
-  if (onesweep_supported(N) && !(os_env && os_env[0] == '0')) {
-    DBuf<u64> a(N), b(N);
-    const u64* sorted = onesweep_sort_iota(A.row.get(), N, bits_for(A.m ? A.m - 1 : 0), a.get(), b.get());
-    DBuf<u32> colidx(N);
-    expand_columns(A.pos.get(), (u32)A.n, colidx.get(), N);
-    B->row.alloc(N);
-    CPB_LAUNCH(k_gather_cols_pairs, grid_for(N), 256, 0, sorted, colidx.get(), N, B->row.get());
-    B->pos.alloc((size_t)A.m + 1);
-    const unsigned grid = (unsigned)std::min<size_t>((N + 1 + 255) / 256, (size_t)ctx().sm_count * 16);
-    CPB_LAUNCH(k_segment_starts_pairs, grid, 256, 0, sorted, N, B->pos.get(), (u32)A.m);
-    return B;
-  }
-  TransposeOrder t;
-  transpose_order(A.row.get(), N, A.m ? A.m - 1 : 0, t);
+  DBuf<u64> a(N), b(N);
+  const u64* sorted = N ? onesweep_sort_iota(A.row.get(), N, bits_for(A.m ? A.m - 1 : 0), a.get(), b.get()) : nullptr;
   DBuf<u32> colidx(N);
   expand_columns(A.pos.get(), (u32)A.n, colidx.get(), N);
   B->row.alloc(N);
-  if (N) CPB_LAUNCH(k_gather_cols, grid_for(N), 256, 0, t.q, colidx.get(), N, B->row.get());
+  if (N) CPB_LAUNCH(k_gather_cols_pairs, grid_for(N), 256, 0, sorted, colidx.get(), N, B->row.get());
   B->pos.alloc((size_t)A.m + 1);
-  // pos'[i] = first sorted index with row >= i, i = 0..m
-  segment_starts(t.keys, N, B->pos.get(), (u32)A.m);
+  const unsigned grid = (unsigned)std::min<size_t>((N + 1 + 255) / 256, (size_t)ctx().sm_count * 16);
+  CPB_LAUNCH(k_segment_starts_pairs, grid, 256, 0, sorted, N, B->pos.get(), (u32)A.m);  // (N = 0: pos' = 0, sorted unread)
   return B;
 }
 

@@ -1,10 +1,9 @@
 // onesweep.cu -- stable LSD radix sort of packed (key << 32 | payload) pairs with ONE read and ONE write of the pairs per
 // 8-bit pass (sm_100a), and the link construction that sits on top of it (links.cu, sharded.cu).
 //
-// The tile-histogram sort in primitives.cu reads the keys twice per pass (histogram table + scatter) and keeps a
-// digit-major table of every tile's counts.  Here the digit histograms of ALL passes come from one sweep over the keys
-// (k_os_hist), and a tile learns how many equal digits precede it from its predecessors' published counts (chained scan
-// with decoupled look-back: every tile publishes its per-digit count as soon as it is known, then the inclusive prefix):
+// The digit histograms of ALL passes come from one sweep over the keys (k_os_hist), and a tile learns how many equal
+// digits precede it from its predecessors' published counts (chained scan with decoupled look-back: every tile publishes
+// its per-digit count as soon as it is known, then the inclusive prefix), so no pass reads the keys twice:
 //   k_os_pass<MODE>   MODE 0: first pass, pairs formed on the fly from a u32 key array (payload = element index)
 //                     MODE 1: pair -> pair
 //                     MODE 2: the pairs arrive sorted by (row, position); the pass forms every nonzero's link from its left
@@ -21,7 +20,9 @@ static constexpr int OS_THREADS = 256;
 static constexpr int OS_IPT = 16;
 static constexpr int OS_WARPS = OS_THREADS / 32;
 static constexpr int OS_TILE = OS_THREADS * OS_IPT;  // 4096 pairs per CTA
-static constexpr u32 OS_AGG = 1u << 30, OS_INC = 2u << 30, OS_VAL = (1u << 30) - 1u;
+// look-back state word: 0 = not yet published, count + 1 = the tile's own count (<= OS_TILE + 1), OS_INC | prefix = the
+// inclusive prefix (< 2^31: every index the library accepts)
+static constexpr u32 OS_INC = 1u << 31, OS_VAL = OS_INC - 1u;
 static constexpr int OS_LOOKBACK = 4;  // predecessors inspected per round trip
 
 // digit histograms of up to four 8-bit passes in one sweep over the keys: ghist[pass * 256 + digit]
@@ -180,7 +181,7 @@ __device__ __forceinline__ void os_tile_body(const u32* __restrict__ keys32, con
 #pragma unroll
   for (int k = 0; k < OS_WARPS; ++k) total += s_cur[k][tid];
   u32* const my_state = state + (size_t)tile * 256 + tid;
-  st_state(my_state, (tile == 0 ? OS_INC : OS_AGG) | total);
+  st_state(my_state, tile == 0 ? (OS_INC | total) : total + 1u);
   const u32 lbase = os_block_scan(total, s_scan);  // first staged slot of the digit
   {
     u32 run = lbase;
@@ -204,16 +205,20 @@ __device__ __forceinline__ void os_tile_body(const u32* __restrict__ keys32, con
 #pragma unroll
       for (int j = 0; j < OS_LOOKBACK; ++j) {
         if (done) break;
-        while ((v[j] & ~OS_VAL) == 0u) {
+        while (v[j] == 0u) {
           v[j] = ld_state(state + (size_t)(t - j) * 256 + tid);
           if (clock64() - t_start > (4ll << 30)) __trap();  // (a predecessor never published: fail loudly instead of hanging)
         }
-        excl += v[j] & OS_VAL;
-        if (v[j] & OS_INC) done = true;
+        if (v[j] & OS_INC) {
+          excl += v[j] & OS_VAL;
+          done = true;
+        } else {
+          excl += v[j] - 1u;
+        }
       }
       t -= OS_LOOKBACK;
     }
-    st_state(my_state, OS_INC | ((excl + total) & OS_VAL));
+    st_state(my_state, OS_INC | (excl + total));
   }
   s_gbase[tid] = dstart + excl - lbase;
   __syncthreads();
@@ -278,8 +283,6 @@ k_os_pass(const u32* __restrict__ keys32, const u64* __restrict__ in, u64* __res
 
 static size_t os_tiles(size_t n) { return (n + OS_TILE - 1) / OS_TILE; }
 
-bool onesweep_supported(size_t n) { return n > 0 && n < ((size_t)1 << 30); }
-
 struct OsWork {
   DBuf<u32> ghist, state, counters;
   size_t tiles = 0;
@@ -327,7 +330,7 @@ static u64* os_sort_passes(OsWork& wk, const u32* keys, size_t n, int passes, u6
 }
 
 u64* onesweep_sort_iota(const u32* keys, size_t n, int bits, u64* a, u64* b) {
-  CPB_REQUIRE(onesweep_supported(n), "onesweep: unsupported size");
+  CPB_REQUIRE(n > 0 && n < ((size_t)1 << 31), "onesweep: 0 < n < 2^31 pairs");
   const int passes = std::max(1, (bits + 7) / 8);
   OsWork wk;
   wk.init(n, passes);
@@ -371,7 +374,7 @@ __global__ void __launch_bounds__(256) k_os_link_scatter(const u64* __restrict__
 
 u64* onesweep_links(const u32* row, size_t N, int row_bits, const u32* colidx, bool as_pos, u32 q_off, u32* prev, u32* first_count, u32* last_local,
                     size_t window_min, u64* a, u64* b) {
-  CPB_REQUIRE(onesweep_supported(N), "onesweep: unsupported size");
+  CPB_REQUIRE(N > 0 && N < ((size_t)1 << 31), "onesweep: 0 < N < 2^31 pairs");
   const int passes = std::max(1, (row_bits + 7) / 8);
   const bool windowed = window_min > 0 && N >= window_min;
   OsWork wk;
@@ -380,8 +383,9 @@ u64* onesweep_links(const u32* row, size_t N, int row_bits, const u32* colidx, b
   const OsLinkArgs la{colidx, as_pos ? 1 : 0, q_off, first_count, last_local};
   ProfScope pk("k_link_prev", (double)N * 12.0);
   if (windowed) {
-    // the link array does not fit L2: one more pass groups (link, position) by 2^shift-position windows of `prev`, then the
-    // scatter of a window stays in L2 (see links.cu)
+    // the link array does not fit L2, and a scatter in row order touches one HBM sector per 4-byte link (10.9 ms at
+    // N = 2.6e8 on B200): one more pass groups (link, position) by 2^shift-position windows of `prev`, then the scatter
+    // of a window stays in L2
     u64* other = (sorted == a) ? b : a;
     const int shift = std::max(0, bits_for(N - 1) - 8);
     os_launch<2>(wk, nullptr, sorted, other, N, shift, nullptr, la);

@@ -285,23 +285,6 @@ static int radix_sort_impl(u32* keys, u32* vals, u32* keys_tmp, u32* vals_tmp, s
   return radix_sort_passes<8>(keys, vals, keys_tmp, vals_tmp, n, p8, iota_payload, first_keys);
 }
 
-// ONE stable partition pass by the 8 key bits [shift, shift + 8): (keys_in, vals_in) -> (keys_out, vals_out).  Used to
-// group scattered writes by destination window (links.cu) so that they land in L2 instead of touching HBM one sector each.
-void radix_partition_pass(const u32* keys_in, const u32* vals_in, u32* keys_out, u32* vals_out, size_t n, int shift) {
-  if (n == 0) return;
-  constexpr int DB = 8, NB = 1 << DB;
-  static bool attr_set = false;
-  if (!attr_set) {
-    CPB_CUDA(cudaFuncSetAttribute(k_rs_scatter<DB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem<DB>()));
-    attr_set = true;
-  }
-  const u32 tiles = (u32)((n + RS_TILE - 1) / RS_TILE);
-  DBuf<u32> hist((size_t)NB * tiles);
-  CPB_LAUNCH(k_rs_hist<DB>, tiles, 256, 0, keys_in, n, shift, hist.get(), tiles);
-  exclusive_scan_u32(hist.get(), hist.get(), (size_t)NB * tiles);
-  CPB_LAUNCH(k_rs_scatter<DB>, tiles, RS_THREADS, rs_smem<DB>(), keys_in, vals_in, keys_out, vals_out, n, shift, hist.get(), tiles, 0);
-}
-
 int radix_sort_pairs(u32* keys, u32* vals, u32* keys_tmp, u32* vals_tmp, size_t n, int bits) {
   return radix_sort_impl(keys, vals, keys_tmp, vals_tmp, n, bits, false, nullptr);
 }

@@ -15,9 +15,6 @@ int radix_sort_pairs(u32* keys, u32* vals, u32* keys_tmp, u32* vals_tmp, size_t 
 // read-only keys_src in the first pass (keys is scratch and need not be initialised either)
 int radix_sort_pairs_iota(const u32* keys_src, u32* keys, u32* vals, u32* keys_tmp, u32* vals_tmp, size_t n, int bits);
 
-// one stable partition pass by key bits [shift, shift + 8)
-void radix_partition_pass(const u32* keys_in, const u32* vals_in, u32* keys_out, u32* vals_out, size_t n, int shift);
-
 // dst[i] = (u32)(src[i] - 1); flags[0] |= 1 if any src[i] outside [lo, hi]
 void narrow_minus1(const i64* src, u32* dst, size_t n, i64 lo, i64 hi, u32* flags);
 void narrow32_minus1(const int* src, u32* dst, size_t n, i64 lo, i64 hi, u32* flags);  // the same from Int32 indices

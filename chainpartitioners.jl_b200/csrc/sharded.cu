@@ -136,39 +136,6 @@ struct ShardedMatrix {
 
 static unsigned grid_for(size_t n) { return (unsigned)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, (size_t)ctx().sm_count * 32)); }
 
-// sorted (row, local position) pairs of the block -> link of every pair in sorted order (run heads: 0 for now) and the
-// last position (+1) of every row of the block
-__global__ void k_shard_link_values(const u32* __restrict__ sk, const u32* __restrict__ sq, size_t cnt, u32 q_lo, u32* __restrict__ lv,
-                                    u32* __restrict__ last_local) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cnt; p += stride) {
-    const u32 r = sk[p];
-    const bool head = p == 0 || sk[p - 1] != r;
-    const bool tail = p + 1 == cnt || sk[p + 1] != r;
-    lv[p] = head ? 0u : q_lo + sq[p - 1] + 1u;
-    if (tail) last_local[r] = q_lo + sq[p] + 1u;
-  }
-}
-__global__ void k_shard_scatter(const u32* __restrict__ sq, const u32* __restrict__ lv, size_t cnt, u32* __restrict__ prev_blk) {
-  const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (p < cnt) prev_blk[sq[p]] = lv[p];
-}
-// run heads: the predecessor is the last position of the row in the earlier blocks (carry), none if the carry is 0
-__global__ void k_shard_heads(const u32* __restrict__ sk, const u32* __restrict__ sq, size_t cnt, const u32* __restrict__ carry,
-                              u32* __restrict__ prev_blk, u32* __restrict__ first_count) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  u32 firsts = 0;
-  for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cnt; p += stride) {
-    const u32 r = sk[p];
-    if (p == 0 || sk[p - 1] != r) {
-      const u32 c = carry ? carry[r] : 0u;
-      if (c) prev_blk[sq[p]] = c;
-      firsts += c == 0u;
-    }
-  }
-  firsts = __reduce_add_sync(0xffffffffu, firsts);
-  if ((threadIdx.x & 31) == 0 && firsts) atomicAdd(first_count, firsts);
-}
 __global__ void k_carry_merge(const u32* __restrict__ last_local, const u32* __restrict__ carry_in, u32* __restrict__ out, size_t m) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride) {
@@ -189,7 +156,8 @@ __global__ void k_carry_pick(const u32* __restrict__ all, size_t m, int rank, u3
 
 static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-// run heads of the packed (row << 32 | local position) pairs: as k_shard_heads
+// run heads of the sorted (row << 32 | local position) pairs of a block: the predecessor is the last position (+1) of the row
+// in the earlier blocks (carry), none if the carry is 0
 __global__ void k_shard_heads_pairs(const u64* __restrict__ sorted, size_t cnt, const u32* __restrict__ carry, u32* __restrict__ prev_blk,
                                     u32* __restrict__ first_count) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
@@ -209,10 +177,9 @@ __global__ void k_shard_heads_pairs(const u64* __restrict__ sorted, size_t cnt, 
 
 // one block's share of the construction: sort, in-block links, last positions
 struct BlockWork {
-  DBuf<u32> k0, v0, k1, v1, last_local;
-  DBuf<u64> pa, pb;      // one-sweep form: packed pairs
-  u64* sorted = nullptr;  // (row << 32 | local position), sorted
-  u32 *sk = nullptr, *sq = nullptr;
+  DBuf<u32> last_local;
+  DBuf<u64> pa, pb;
+  u64* sorted = nullptr;  // (row << 32 | local position), sorted (in pa or pb)
   size_t cntL = 0;
 };
 static void block_local_links(const u32* row_blk, size_t cntL, u32 q_lo, size_t m, u32* prev_full, BlockWork& w) {
@@ -223,37 +190,15 @@ static void block_local_links(const u32* row_blk, size_t cntL, u32 q_lo, size_t 
   if (!cntL) return;
   const char* wmin_env = std::getenv("CPB_WINDOWED_SCATTER_MIN");
   const size_t wmin = wmin_env ? (size_t)std::atoll(wmin_env) : ((size_t)1 << 25);
-  u32* const prev_blk = prev_full + q_lo;
-  const char* os_env = std::getenv("CPB_ONESWEEP");
-  if (onesweep_supported(cntL) && !(os_env && os_env[0] == '0')) {
-    // one-sweep radix passes on packed pairs (onesweep.cu): in-block links (run heads: 0 for now) and last positions
-    w.pa.alloc(cntL);
-    w.pb.alloc(cntL);
-    w.sorted = onesweep_links(row_blk, cntL, bits_for(m ? m - 1 : 0), nullptr, /*as_pos=*/true, q_lo, prev_blk, nullptr, w.last_local.get(), wmin, w.pa.get(),
-                              w.pb.get());
-    return;
-  }
-  w.k0.alloc(cntL); w.v0.alloc(cntL); w.k1.alloc(cntL); w.v1.alloc(cntL);
-  const int which = radix_sort_pairs_iota(row_blk, w.k0.get(), w.v0.get(), w.k1.get(), w.v1.get(), cntL, bits_for(m ? m - 1 : 0));
-  w.sk = which ? w.k1.get() : w.k0.get();
-  w.sq = which ? w.v1.get() : w.v0.get();
-  u32* const other_k = which ? w.k0.get() : w.k1.get();
-  u32* const other_v = which ? w.v0.get() : w.v1.get();
-  CPB_LAUNCH(k_shard_link_values, grid_for(cntL), 256, 0, w.sk, w.sq, cntL, q_lo, other_k, w.last_local.get());
-  if (wmin > 0 && cntL >= wmin) {
-    // the block's links no longer fit L2: group the (position, link) pairs by windows of the link array first (see links.cu)
-    DBuf<u32> pk2(cntL);
-    const int shift = std::max(0, bits_for(cntL - 1) - 8);
-    radix_partition_pass(w.sq, other_k, pk2.get(), other_v, cntL, shift);
-    CPB_LAUNCH(k_shard_scatter, (unsigned)((cntL + 255) / 256), 256, 0, pk2.get(), other_v, cntL, prev_blk);
-  } else {
-    CPB_LAUNCH(k_shard_scatter, (unsigned)((cntL + 255) / 256), 256, 0, w.sq, other_k, cntL, prev_blk);
-  }
+  // one-sweep radix passes on packed pairs (onesweep.cu): in-block links (run heads: 0 for now) and last positions
+  w.pa.alloc(cntL);
+  w.pb.alloc(cntL);
+  w.sorted = onesweep_links(row_blk, cntL, bits_for(m ? m - 1 : 0), nullptr, /*as_pos=*/true, q_lo, prev_full + q_lo, nullptr, w.last_local.get(), wmin,
+                            w.pa.get(), w.pb.get());
 }
 static void block_heads(const BlockWork& w, const u32* carry_in, u32 q_lo, u32* prev_full, u32* first_count) {
   if (!w.cntL) return;
-  if (w.sorted) CPB_LAUNCH(k_shard_heads_pairs, grid_for(w.cntL), 256, 0, w.sorted, w.cntL, carry_in, prev_full + q_lo, first_count);
-  else CPB_LAUNCH(k_shard_heads, grid_for(w.cntL), 256, 0, w.sk, w.sq, w.cntL, carry_in, prev_full + q_lo, first_count);
+  CPB_LAUNCH(k_shard_heads_pairs, grid_for(w.cntL), 256, 0, w.sorted, w.cntL, carry_in, prev_full + q_lo, first_count);
 }
 
 // ---- A + I: the monotonized symmetric model streams the links of A + I (links.cu, build_link_stream(dia = true)) ----------
@@ -666,21 +611,13 @@ __global__ void k_tr_combine(const u32* __restrict__ all, size_t m, int world, i
     below[i] = b;
   }
 }
-// the sorted block (packed pairs of the one-sweep sort, or keys / values) -> (column << 32 | Aᵀ position) in sorted order
-__global__ void k_tr_pairs(const u64* __restrict__ sorted, const u32* __restrict__ sk, const u32* __restrict__ sq, size_t cntL, u32 q_lo,
-                           const u32* __restrict__ pos, u32 n, const u32* __restrict__ colptrT, const u32* __restrict__ below,
-                           const u32* __restrict__ lstart, u64* __restrict__ out) {
+// the sorted (row << 32 | local position) pairs of the block -> (column << 32 | Aᵀ position) in sorted order
+__global__ void k_tr_pairs(const u64* __restrict__ sorted, size_t cntL, u32 q_lo, const u32* __restrict__ pos, u32 n, const u32* __restrict__ colptrT,
+                           const u32* __restrict__ below, const u32* __restrict__ lstart, u64* __restrict__ out) {
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < cntL; p += stride) {
-    u32 i, lp;
-    if (sorted) {
-      const u64 v = sorted[p];
-      i = (u32)(v >> 32);
-      lp = (u32)v;
-    } else {
-      i = sk[p];
-      lp = sq[p];
-    }
+    const u64 v = sorted[p];
+    const u32 i = (u32)(v >> 32), lp = (u32)v;
     const u32 dst = colptrT[i] + below[i] + ((u32)p - lstart[i]);
     out[p] = ((u64)column_of(pos, n, q_lo + lp) << 32) | dst;
   }
@@ -710,29 +647,15 @@ __global__ void k_tr_scatter(const u64* __restrict__ pairs, size_t cnt, u32 q_lo
   }
 }
 
-struct TrBlock {
-  DBuf<u32> k0, v0, k1, v1;
-  DBuf<u64> a, b;
-  const u64* sorted = nullptr;
-  const u32 *sk = nullptr, *sq = nullptr;
-};
-// stable sort of a block by row: the one-sweep passes block_local_links runs, or the tile-histogram sort
-static void tr_sort(const u32* rows, size_t cntL, size_t m, TrBlock& t) {
-  if (!cntL) return;
-  const char* os_env = std::getenv("CPB_ONESWEEP");
-  if (onesweep_supported(cntL) && !(os_env && os_env[0] == '0')) {
-    t.a.alloc(cntL);
-    t.b.alloc(cntL);
-    t.sorted = onesweep_sort_iota(rows, cntL, bits_for(m ? m - 1 : 0), t.a.get(), t.b.get());
-    return;
-  }
-  t.k0.alloc(cntL); t.v0.alloc(cntL); t.k1.alloc(cntL); t.v1.alloc(cntL);
-  const int which = radix_sort_pairs_iota(rows, t.k0.get(), t.v0.get(), t.k1.get(), t.v1.get(), cntL, bits_for(m ? m - 1 : 0));
-  t.sk = which ? t.k1.get() : t.k0.get();
-  t.sq = which ? t.v1.get() : t.v0.get();
+// stable sort of a block by row (the one-sweep passes block_local_links runs) into a or b; nullptr for an empty block
+static const u64* tr_sort(const u32* rows, size_t cntL, size_t m, DBuf<u64>& a, DBuf<u64>& b) {
+  if (!cntL) return nullptr;
+  a.alloc(cntL);
+  b.alloc(cntL);
+  return onesweep_sort_iota(rows, cntL, bits_for(m ? m - 1 : 0), a.get(), b.get());
 }
 // colptrᵀ (m + 1, 0-based) and the routed pairs of rank `rank`'s sorted block, from every rank's row histogram (all: world x m)
-static void tr_pairs(const Matrix& A, const u32* all, int world, int rank, const TrBlock& t, size_t cntL, u32 q_lo, u32* colptrT, DBuf<u64>& pairs) {
+static void tr_pairs(const Matrix& A, const u32* all, int world, int rank, const u64* sorted, size_t cntL, u32 q_lo, u32* colptrT, DBuf<u64>& pairs) {
   const size_t m = (size_t)A.m;
   DBuf<u32> tot(m + 1), below(std::max<size_t>(m, 1)), lstart(std::max<size_t>(m, 1));
   tot.zero();
@@ -742,7 +665,7 @@ static void tr_pairs(const Matrix& A, const u32* all, int world, int rank, const
   }
   exclusive_scan_u32(tot.get(), colptrT, m + 1);
   pairs.alloc(std::max<size_t>(cntL, 1));
-  if (cntL) CPB_LAUNCH(k_tr_pairs, grid_for(cntL), 256, 0, t.sorted, t.sk, t.sq, cntL, q_lo, A.pos.get(), (u32)A.n, colptrT, below.get(), lstart.get(), pairs.get());
+  if (cntL) CPB_LAUNCH(k_tr_pairs, grid_for(cntL), 256, 0, sorted, cntL, q_lo, A.pos.get(), (u32)A.n, colptrT, below.get(), lstart.get(), pairs.get());
 }
 
 ShardedMatrix* sharded_adjointpattern(const ShardedMatrix& S) {
@@ -763,10 +686,8 @@ ShardedMatrix* sharded_adjointpattern(const ShardedMatrix& S) {
   u32* const mine = all.get() + (size_t)rank * m;
   if (cntL) CPB_LAUNCH(k_tr_hist, grid_for(cntL), 256, 0, S.row_blk.get(), cntL, mine);
   if (world > 1 && m) CPB_NCCL(g_nccl.AllGather(mine, all.get(), m, ncclUint32, g_comm, ctx().stream));
-  TrBlock t;
-  tr_sort(S.row_blk.get(), cntL, m, t);
-  DBuf<u64> pairs;
-  tr_pairs(A, all.get(), world, rank, t, cntL, (u32)S.q_lo, T->M.pos.get(), pairs);
+  DBuf<u64> sa, sb, pairs;
+  tr_pairs(A, all.get(), world, rank, tr_sort(S.row_blk.get(), cntL, m, sa, sb), cntL, (u32)S.q_lo, T->M.pos.get(), pairs);
   if (world == 1) {
     if (cntL) CPB_LAUNCH(k_tr_scatter, grid_for(cntL), 256, 0, pairs.get(), cntL, 0u, T->row_blk.get());
     CPB_CUDA(cudaStreamSynchronize(ctx().stream));
@@ -829,10 +750,8 @@ std::unique_ptr<Matrix> adjoint_pattern_sharded_emulated(const Matrix& A, int wo
     i64 lo = 0, hi = 0;
     shard_range(A.N, r, world, nullptr, &lo, &hi);
     const size_t cntL = (size_t)(hi - lo);
-    TrBlock t;
-    tr_sort(A.row.get() + lo, cntL, m, t);
-    DBuf<u64> pairs;
-    tr_pairs(A, all.get(), world, r, t, cntL, (u32)lo, r == 0 ? B->pos.get() : colptrT.get(), pairs);
+    DBuf<u64> sa, sb, pairs;
+    tr_pairs(A, all.get(), world, r, tr_sort(A.row.get() + lo, cntL, m, sa, sb), cntL, (u32)lo, r == 0 ? B->pos.get() : colptrT.get(), pairs);
     // the slices as the destination ranks would receive them
     CPB_LAUNCH(k_tr_slices, 1, 32, 0, pairs.get(), cntL, (u64)cnt, (u64)N, world, off.get(), (u32*)nullptr);
     std::vector<u32> h_off((size_t)world + 1);

@@ -3,6 +3,7 @@ columns, warp and thread-per-block forms, several staged chunks), the one-sweep 
 tile edge and link-construction route, and the environment switches that select between forms which must give identical
 results.  Each check compares with an independent reference exactly: split vectors, K, n_nets, integer counts and patterns
 (scipy's transpose for adjointpattern, the CPU oracle for everything else)."""
+import ctypes
 import functools
 import json
 import os
@@ -19,7 +20,7 @@ AFF = cp.AffineConnectivityModel(0, 10, 1, 100)
 SYM = cp.AffineMonotonizedSymmetricConnectivityModel(0, 0, 1, 100, 4)
 TILE = 4096  # pairs per one-sweep tile (OS_TILE in onesweep.cu)
 
-LINK_SWITCHES = ("CPB_ONESWEEP", "CPB_NO_ROW_SEGMENTS", "CPB_WINDOWED_SCATTER_MIN", "CPB_CHUNK_THREAD_BLOCKS")
+LINK_SWITCHES = ("CPB_NO_ROW_SEGMENTS", "CPB_WINDOWED_SCATTER_MIN", "CPB_CHUNK_THREAD_BLOCKS")
 
 
 def set_env(monkeypatch, env):
@@ -282,8 +283,7 @@ def query_pairs(A, rng):
     return np.array(j, dtype=np.int64), np.array(jp, dtype=np.int64)
 
 
-LINK_CONFIGS = [dict(base, **os_) for os_ in ({}, {"CPB_ONESWEEP": "0"})
-                for base in ({}, {"CPB_NO_ROW_SEGMENTS": "1"}, {"CPB_NO_ROW_SEGMENTS": "1", "CPB_WINDOWED_SCATTER_MIN": "1"})]
+LINK_CONFIGS = [{}, {"CPB_NO_ROW_SEGMENTS": "1"}, {"CPB_NO_ROW_SEGMENTS": "1", "CPB_WINDOWED_SCATTER_MIN": "1"}]
 
 
 def scipy_transpose(A):
@@ -293,27 +293,25 @@ def scipy_transpose(A):
 
 
 @pytest.mark.parametrize("name", list(LINK_CASES) + list(DEGREE_CASES))
-def test_onesweep_adjointpattern(ref, monkeypatch, name):
-    """adjointpattern is a direct readout of the stable row sort: equal to scipy's transpose and to the oracle under both
-    sorts, and the one-sweep sort runs exactly ceil(bits(m - 1) / 8) passes."""
+def test_adjointpattern_row_sort(ref, monkeypatch, name):
+    """adjointpattern is a direct readout of the stable row sort: equal to scipy's transpose and to the oracle, and the
+    one-sweep sort runs exactly ceil(bits(m - 1) / 8) passes."""
     A = link_input(name)
     S = scipy_transpose(A)
     R = ref.adjointpattern(A)
     assert np.array_equal(R.colptr - 1, S.indptr) and np.array_equal(R.rowval - 1, S.indices)
-    for env in ({}, {"CPB_ONESWEEP": "0"}):
-        set_env(monkeypatch, env)
-        g, prof = profiled(lambda: cp.adjointpattern(A))
-        assert (g.m, g.n) == (A.n, A.m)
-        assert np.array_equal(g.colptr - 1, S.indptr) and np.array_equal(g.rowval - 1, S.indices), (name, env)
-        assert launches(prof, "k_os_pass") == (0 if env else os_passes(A.m)), (name, env, prof.get("k_os_pass"))
     set_env(monkeypatch, {})
+    g, prof = profiled(lambda: cp.adjointpattern(A))
+    assert (g.m, g.n) == (A.n, A.m)
+    assert np.array_equal(g.colptr - 1, S.indptr) and np.array_equal(g.rowval - 1, S.indices), name
+    assert launches(prof, "k_os_pass") == os_passes(A.m), (name, prof.get("k_os_pass"))
 
 
 @pytest.mark.parametrize("name", list(LINK_CASES) + list(DEGREE_CASES))
 def test_link_construction_forms(ref, monkeypatch, name):
     """netcount / dianetcount / selfnetcount queries and the streaming bisections against the oracle under every link
-    construction route: row segments (immediate degree check in the counts, deferred in LazyBisect), the sort with the
-    direct scatter and with the windowed MODE-2 pass, each through the one-sweep and the round-1 tile-histogram sort."""
+    construction route: row segments (immediate degree check in the counts, deferred in LazyBisect), the one-sweep sort
+    with the direct scatter and with the windowed MODE-2 pass.  selfnetcount sorts the rows with the same passes."""
     A = link_input(name)
     rng = np.random.default_rng(sum(map(ord, name)) + 1)
     j, jp = query_pairs(A, rng)
@@ -330,9 +328,11 @@ def test_link_construction_forms(ref, monkeypatch, name):
         set_env(monkeypatch, env)
         got, prof = profiled(lambda: cp.netcount(A).query(j, jp))
         assert np.array_equal(got, want["net"]), (name, env)
-        if env.get("CPB_NO_ROW_SEGMENTS") and "CPB_ONESWEEP" not in env:
+        if env.get("CPB_NO_ROW_SEGMENTS"):
             assert launches(prof, "k_os_pass") == os_passes(A.m), (name, env, prof.get("k_os_pass"))
-        assert np.array_equal(cp.selfnetcount(A).query(j, jp), want["selfnet"]), (name, env)
+        got, prof = profiled(lambda: cp.selfnetcount(A).query(j, jp))
+        assert np.array_equal(got, want["selfnet"]), (name, env)
+        assert launches(prof, "k_os_pass") == os_passes(A.m), (name, env, prof.get("k_os_pass"))
         if square:
             assert np.array_equal(cp.dianetcount(A).query(j, jp), want["dianet"]), (name, env)
         for mtd, spl in zip(mtds, want_spl):
@@ -394,15 +394,85 @@ def test_row_degree_prefix_count(ref, monkeypatch, heavy_in_prefix):
 @pytest.mark.parametrize("name", ["m2^24+1-uniform", "m65537-uniform-N12288", "m257-low-N12288"])
 def test_sharded_link_blocks(ref, monkeypatch, name):
     """The sharded construction sorts each rank's block of positions with the same passes: 4-pass and tile-edge inputs at
-    worlds 2 and 3, one-sweep on and off."""
+    worlds 2 and 3."""
     A = link_input(name)
     mtd = cp.LazyBisectCostBottleneckSplitter(AFF, 0.01)
     exp = ref.partition_stripe(A, 8, mtd).spl
-    for env in ({}, {"CPB_ONESWEEP": "0"}):
-        set_env(monkeypatch, env)
-        for world in (2, 3):
-            assert np.array_equal(cp.partition_stripe_sharded_emulated(A, 8, mtd, world).spl, exp), (name, env, world)
     set_env(monkeypatch, {})
+    for world in (2, 3):
+        assert np.array_equal(cp.partition_stripe_sharded_emulated(A, 8, mtd, world).spl, exp), (name, world)
+
+
+@pytest.mark.skipif(os.environ.get("CPB_SKIP_FULL_SIZE") == "1", reason="CPB_SKIP_FULL_SIZE=1")
+def test_row_sort_above_2_30_nonzeros(monkeypatch):
+    """m = n = 2^22 with 257 nonzeros per column, entry k of every column in the k-th band of rows (distinct and sorted,
+    about 257 per row: every row is too heavy for the row segments): 1.08e9 nonzeros, above the 2^30 that a 30-bit
+    look-back word could count.  The row sort runs 3 one-sweep passes and the windowed MODE-2 pass.  The pattern is built
+    on the device; adjointpattern must equal torch's stable sort by row, netcount the distinct rows of each column range
+    counted from that sort."""
+    import torch
+
+    set_env(monkeypatch, {})
+    dev = "cuda"
+    m = n = 1 << 22
+    d = 257
+    band = m // d
+    N = n * d
+    assert N > 1 << 30
+    gen = torch.Generator(device=dev).manual_seed(30)
+    rows = (torch.arange(d, dtype=torch.int32, device=dev) * band).repeat(n)  # 0-based, CSC order: column q // d
+    rows += torch.randint(0, band, (N,), dtype=torch.int32, device=dev, generator=gen)
+    rowval = rows.to(torch.int64) + 1
+    colptr = torch.arange(n + 1, dtype=torch.int64, device=dev) * d + 1
+    torch.cuda.synchronize()
+    h = ctypes.c_void_p()
+    cp.api._check(cp.load_library().cpb_matrix_create_device(m, n, N, colptr.data_ptr(), rowval.data_ptr(), ctypes.byref(h)))
+    dA = cp.api.DeviceMatrix(h, m, n, N)
+    del rowval, colptr
+
+    sr, perm = torch.sort(rows, stable=True)
+    del rows
+    B, prof = profiled(lambda: cp.adjointpattern(dA))
+    assert launches(prof, "k_os_pass") == os_passes(m), prof.get("k_os_pass")
+    Bh = B.to_host()
+    B.close()
+    exp_colptr = torch.zeros(m + 1, dtype=torch.int64, device=dev)
+    exp_colptr[1:] = torch.cumsum(torch.bincount(sr, minlength=m), 0)
+    assert torch.equal(torch.from_numpy(Bh.colptr).to(dev) - 1, exp_colptr)
+    got = torch.from_numpy(Bh.rowval).to(dev)
+    del Bh
+    assert torch.equal(got - 1, perm // d)
+    del got, exp_colptr
+
+    # prevpos[q] = the previous position of q's row (-1 if none): rows of positions [lo, hi) = #{q in [lo, hi): prevpos[q] < lo}
+    perm = perm.to(torch.int32)
+    head = torch.ones(N, dtype=torch.bool, device=dev)
+    head[1:] = sr[1:] != sr[:-1]
+    del sr
+    prevpos = torch.empty(N, dtype=torch.int32, device=dev)
+    prevpos[1:] = perm[:-1]
+    prevpos[head] = -1
+    del head
+    pp = torch.empty_like(prevpos)
+    pp[perm.to(torch.int64)] = prevpos
+    prevpos = pp
+    del perm, pp
+
+    rng = np.random.default_rng(31)
+    j = rng.integers(1, n + 1, 60)
+    jp = np.minimum(j + rng.integers(1, 3000, 60), n + 1)
+    edges = [TILE, 1 << 23, 1 << 29, 1 << 30, (1 << 30) + TILE, N // TILE * TILE, N - 1]  # tiles, MODE-2 windows, the end
+    for b in edges:
+        c = b // d + 1  # 1-based column of 0-based position b
+        for a, ap in ((c - 1, c), (c, c + 1), (c - 1, c + 2), (c, min(c + 40, n + 1))):
+            if 1 <= a < ap <= n + 1:
+                j, jp = np.append(j, a), np.append(jp, ap)
+    j, jp = np.append(j, [1, 1, n // 2]), np.append(jp, [n + 1, n // 2, n + 1])
+    exp = np.array([int((prevpos[(int(a) - 1) * d:(int(ap) - 1) * d] < (int(a) - 1) * d).sum()) for a, ap in zip(j, jp)], dtype=np.int64)
+    got, prof = profiled(lambda: cp.netcount(dA).query(j, jp))
+    assert launches(prof, "k_os_pass") == os_passes(m), prof.get("k_os_pass")
+    assert np.array_equal(got, exp), np.flatnonzero(got != exp)[:10]
+    dA.close()
 
 
 # ------------------------------------------------------------------------------------------ bisection and DP switches
