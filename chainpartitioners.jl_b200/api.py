@@ -18,7 +18,7 @@ from . import types as T
 
 __all__ = [
     "DeviceMatrix", "device_matrix", "device_matrix_i32", "adjointpattern", "permute", "oracle_stripe", "bound_stripe", "partition_stripe",
-    "pack_stripe", "partition_plaid", "pack_plaid", "bottleneck_value", "total_value", "pincount", "netcount",
+    "partition_stripe_batch", "partition_stripe_batch_capacity", "pack_stripe", "partition_plaid", "pack_plaid", "bottleneck_value", "total_value", "pincount", "netcount",
     "dianetcount", "selfnetcount", "selfpincount", "PrefixMatrix", "dominancecount", "dominancesum", "rookcount", "rooksum", "profile_enable", "profile_reset", "profile_get",
     "Communicator", "ShardedMatrix", "partition_stripe_sharded", "partition_stripe_sharded_emulated", "sharded_stats", "shard_range",
     "partition_plaid_sharded", "partition_plaid_sharded_emulated", "adjointpattern_sharded_emulated",
@@ -41,7 +41,7 @@ ABI_SYMBOLS = [
     "cpb_partition_stripe_sharded", "cpb_partition_stripe_sharded_emulated", "cpb_sharded_stats",
     "cpb_sharded_adjointpattern", "cpb_adjointpattern_sharded_emulated", "cpb_sharded_matrix_get",
     "cpb_prefix_create", "cpb_prefix_query", "cpb_prefix_destroy", "cpb_matrix_permute", "cpb_trim_memory", "cpb_matrix_create_i32",
-    "cpb_partition_stripe_weighted", "cpb_weight_windows",
+    "cpb_partition_stripe_weighted", "cpb_weight_windows", "cpb_partition_stripe_batch", "cpb_partition_stripe_batch_capacity",
 ]
 
 
@@ -85,6 +85,8 @@ def load_library():
         lib.cpb_objective.argtypes = [vp, i32, i64, vp, ctypes.POINTER(dbl)]
         lib.cpb_partition_stripe.argtypes = [vp, i32, ctypes.POINTER(T.CConstraint), dbl, i64, vp]
         lib.cpb_partition_stripe_weighted.argtypes = [vp, i32, vp, i64, dbl, i64, vp]
+        lib.cpb_partition_stripe_batch.argtypes = [i64, vp, vp, vp, vp, vp]
+        lib.cpb_partition_stripe_batch_capacity.argtypes = [ctypes.POINTER(i32)]
         lib.cpb_weight_windows.argtypes = [vp, i64, vp, vp]
         lib.cpb_pack_stripe.argtypes = [vp, vp, i32, ctypes.POINTER(T.CConstraint), dbl, i64, vp, ctypes.POINTER(i64), vp]
         lib.cpb_profile_get.argtypes = [i32, vp, vp, vp, vp]
@@ -562,6 +564,59 @@ def partition_stripe(A, K, method, Pi=None, **kwargs) -> T.SplitPartition:
         finally:
             ocl.close()
     return T.SplitPartition(K, spl)
+
+
+_BATCH_METHODS = (T.SPLIT_BISECT_INDEX, T.SPLIT_FLIP_BISECT_COST, T.SPLIT_LAZY_FLIP_BISECT_COST, T.SPLIT_FLIP_BISECT_INDEX)
+
+
+def partition_stripe_batch(problems) -> list:
+    """Many ``partition_stripe`` problems in one launch (``cpb_partition_stripe_batch``): ``problems`` is a list of
+    ``(A, K, method)`` or ``(A, K, method, Pi)`` with ``method`` a BisectIndex or Flip splitter; returns the list of
+    ``SplitPartition``s, each identical to ``partition_stripe(A, K, method[, Pi])``.  Entries with the same ``A``, model and
+    ``Pi`` objects share one oracle (a sweep over K builds it once); a host matrix is uploaded once per distinct object."""
+    specs = []
+    for p in problems:
+        if len(p) not in (3, 4):
+            raise TypeError("a batch problem is (A, K, method) or (A, K, method, Pi)")
+        A, K, method = p[0], int(p[1]), p[2]
+        Pi = p[3] if len(p) == 4 else None
+        code, spec, eps = T.split_method_code(method)
+        if code not in _BATCH_METHODS:
+            raise TypeError(f"partition_stripe_batch: unsupported method {type(method).__name__} (BisectIndex and the Flip splitters only)")
+        if isinstance(spec, T.ConstrainedCost) and spec.count_weight() is not None:
+            raise TypeError("partition_stripe_batch: a count-weight constraint is taken by the Dynamic, Convex and Concave splitters only")
+        specs.append((A, K, code, spec, eps, Pi))
+    if not specs:
+        return []
+    mats, oracles = {}, {}
+    try:
+        for A, _, _, spec, _, Pi in specs:
+            if id(A) not in mats:
+                mats[id(A)] = _Scoped(A)
+            key = (id(A), id(spec), id(Pi))
+            if key not in oracles:
+                oracles[key] = StripeOracle(spec, mats[id(A)].dm, Pi)
+        B = len(specs)
+        outs = [np.full(K + 1, -1, dtype=I64) for (_, K, *_) in specs]
+        f = (ctypes.c_void_p * B)(*[oracles[(id(A), id(spec), id(Pi))]._h.value for A, _, _, spec, _, Pi in specs])
+        method = np.array([s[2] for s in specs], dtype=np.int32)
+        eps = np.array([s[4] for s in specs], dtype=np.float64)
+        Ks = np.array([s[1] for s in specs], dtype=I64)
+        spl = (ctypes.c_void_p * B)(*[o.ctypes.data for o in outs])
+        _check(load_library().cpb_partition_stripe_batch(B, f, _p(method), _p(eps), _p(Ks), spl))
+    finally:
+        for o in oracles.values():
+            o.close()
+        for m in mats.values():
+            m.__exit__()
+    return [T.SplitPartition(s[1], o) for s, o in zip(specs, outs)]
+
+
+def partition_stripe_batch_capacity() -> int:
+    """Clusters of the batch kernel the device keeps resident at once (``cpb_partition_stripe_batch_capacity``)."""
+    n = ctypes.c_int()
+    _check(load_library().cpb_partition_stripe_batch_capacity(ctypes.byref(n)))
+    return n.value
 
 
 _SCRATCH = {}

@@ -150,10 +150,8 @@ __global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
 // k_bisect_round), the windows are hard limits exactly as in the reference, so the split vector is the reference's.
 // ------------------------------------------------------------------------------------------------
 template <class T>
-__global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
-    k_bisect_index(const __grid_constant__ DevOracle o, int K, double c_lo, double c_hi, int* __restrict__ spl, int* __restrict__ spl_lo,
-                   int* __restrict__ spl_hi, int* __restrict__ probes_out) {
-  __shared__ int s_cnt[2][BS_CLUSTER];
+__device__ __forceinline__ void bisect_index_body(const DevOracle& o, int (*s_cnt)[BS_CLUSTER], int K, double c_lo, double c_hi, int* __restrict__ spl,
+                                                  int* __restrict__ spl_lo, int* __restrict__ spl_hi, int* __restrict__ probes_out) {
   cg::cluster_group cluster = cg::this_cluster();
   const bool cta0 = cluster.block_rank() == 0;
   const bool writer = cta0 && threadIdx.x == 0;
@@ -261,10 +259,8 @@ struct FlipResult {
 
 // mode 0: FlipBisectCost (windows spl_lo / spl_hi, answer spl_lo); mode 1: LazyFlipBisectCost (no windows, answer spl_hi)
 template <class T>
-__global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
-    k_flip_bisect(const __grid_constant__ DevOracle o, int K, double eps1, double c_lo, double c_hi, int lazy, int* __restrict__ spl,
-                  int* __restrict__ spl_lo, int* __restrict__ spl_hi, int* __restrict__ probes_out) {
-  __shared__ int s_cnt[2][BS_CLUSTER];
+__device__ __forceinline__ void flip_bisect_body(const DevOracle& o, int (*s_cnt)[BS_CLUSTER], int K, double eps1, double c_lo, double c_hi, int lazy,
+                                                 int* __restrict__ spl, int* __restrict__ spl_lo, int* __restrict__ spl_hi, int* __restrict__ probes_out) {
   cg::cluster_group cluster = cg::this_cluster();
   const bool cta0 = cluster.block_rank() == 0;
   const bool writer = cta0 && threadIdx.x == 0;
@@ -329,10 +325,8 @@ __global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
 
 // FlipBisectIndexBottleneckSplitter (BisectIndex...:87-166)
 template <class T>
-__global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
-    k_flip_bisect_index(const __grid_constant__ DevOracle o, int K, double c_lo, double c_hi, int* __restrict__ spl, int* __restrict__ spl_lo,
-                        int* __restrict__ spl_hi, int* __restrict__ probes_out) {
-  __shared__ int s_cnt[2][BS_CLUSTER];
+__device__ __forceinline__ void flip_bisect_index_body(const DevOracle& o, int (*s_cnt)[BS_CLUSTER], int K, double c_lo, double c_hi, int* __restrict__ spl,
+                                                       int* __restrict__ spl_lo, int* __restrict__ spl_hi, int* __restrict__ probes_out) {
   cg::cluster_group cluster = cg::this_cluster();
   const bool cta0 = cluster.block_rank() == 0;
   const bool writer = cta0 && threadIdx.x == 0;
@@ -394,6 +388,37 @@ __global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
   }
   if (writer) *probes_out = probes;
   cluster.sync();
+}
+
+// ------------------------------------------------------------------------------------------------
+// Batched solves (kernel "stripe_batch"): B independent problems of the four splitters above in one launch, one 8-CTA
+// cluster per problem.  A solve is a latency chain of K part searches that occupies one cluster; a batch lets a K sweep,
+// many matrices or the secondary models of a 2-D alternation fill the GPU instead of queueing one cluster at a time.
+// ------------------------------------------------------------------------------------------------
+struct StripeJob {
+  int oracle;         // index into the batch's DevOracle table (one entry per distinct oracle)
+  int method;         // CPB_SPLIT_BISECT_INDEX, CPB_SPLIT_FLIP_BISECT_COST, CPB_SPLIT_LAZY_FLIP_BISECT_COST or CPB_SPLIT_FLIP_BISECT_INDEX
+  int K;
+  int lazy;           // LazyFlipBisectCost
+  double c_lo, c_hi;  // oracle_bound
+  double eps1;        // 1 + eps (the FlipBisectCost forms)
+  i64 spl, spl_lo, spl_hi, probes;  // offsets into the batch's int workspace
+};
+
+template <class T>
+__global__ void __cluster_dims__(BS_CLUSTER, 1, 1) __launch_bounds__(BS_THREADS)
+    k_stripe_batch(const DevOracle* __restrict__ oracles, const StripeJob* __restrict__ jobs, int* __restrict__ ws) {
+  __shared__ int s_cnt[2][BS_CLUSTER];
+  __shared__ DevOracle s_o;  // every cost evaluation reads the oracle's fields: keep them next to the SM, not in global memory
+  static_assert(sizeof(DevOracle) % sizeof(u64) == 0, "DevOracle is copied in 8-byte words");
+  const StripeJob jb = jobs[blockIdx.x / BS_CLUSTER];
+  const u64* src = reinterpret_cast<const u64*>(oracles + jb.oracle);
+  for (int t = threadIdx.x; t < (int)(sizeof(DevOracle) / sizeof(u64)); t += blockDim.x) reinterpret_cast<u64*>(&s_o)[t] = src[t];
+  __syncthreads();
+  int *spl = ws + jb.spl, *lo = ws + jb.spl_lo, *hi = ws + jb.spl_hi, *probes = ws + jb.probes;
+  if (jb.method == CPB_SPLIT_BISECT_INDEX) bisect_index_body<T>(s_o, s_cnt, jb.K, jb.c_lo, jb.c_hi, spl, lo, hi, probes);
+  else if (jb.method == CPB_SPLIT_FLIP_BISECT_INDEX) flip_bisect_index_body<T>(s_o, s_cnt, jb.K, jb.c_lo, jb.c_hi, spl, lo, hi, probes);
+  else flip_bisect_body<T>(s_o, s_cnt, jb.K, jb.eps1, jb.c_lo, jb.c_hi, jb.lazy, spl, lo, hi, probes);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1672,33 +1697,19 @@ int probe_cluster_capacity(bool stream) {
   return n;
 }
 
-void solve_bisect_index(Oracle& f, i64 K, int64_t* h_spl_out) {
+// The checks of a BisectIndex solve; leaves the oracle's bound (c_lo, c_hi) in bnd.
+static void bisect_index_prepare(Oracle& f, i64 K, double bnd[2]) {
   CPB_REQUIRE(K >= 1, "K must be >= 1");
   CPB_REQUIRE(f.dev.kind != CPB_MODEL_BLOCK, "bisection needs a random-access oracle");
   const Matrix& A = *f.A;
   CPB_REQUIRE(A.n + 1 < ((i64)1 << 31) && K + 2 < ((i64)1 << 30), "problem too large for 32-bit split points");
   require_monotone_cost(f);
   oracle_ensure_ranks(f);
-  double bnd[2];
   oracle_bound(f, K, bnd);  // (c_lo, c_hi) ./ 1 -- also checks beta >= 0, which the monotone part searches need
-  ProfScope prof("probe");
-  DBuf<int> spl(K + 2), spl_lo(K + 2), spl_hi(K + 2), probes(1);
-  if (f.dev.is_float)
-    CPB_LAUNCH(k_bisect_index<double>, BS_CLUSTER, BS_THREADS, 0, f.dev, (int)K, bnd[0], bnd[1], spl.get(), spl_lo.get(), spl_hi.get(), probes.get());
-  else
-    CPB_LAUNCH(k_bisect_index<i64>, BS_CLUSTER, BS_THREADS, 0, f.dev, (int)K, bnd[0], bnd[1], spl.get(), spl_lo.get(), spl_hi.get(), probes.get());
-  std::vector<int> h(K + 2);
-  int hp = 0;
-  CPB_CUDA(cudaMemcpyAsync(h.data(), spl_hi.get(), (K + 2) * sizeof(int), cudaMemcpyDeviceToHost, ctx().stream));
-  CPB_CUDA(cudaMemcpyAsync(&hp, probes.get(), sizeof(int), cudaMemcpyDeviceToHost, ctx().stream));
-  CPB_CUDA(cudaStreamSynchronize(ctx().stream));
-  for (i64 k = 1; k <= K + 1; ++k) h_spl_out[k - 1] = h[k];
-  g_bisect_stats[0] = 1; g_bisect_stats[1] = hp; g_bisect_stats[2] = hp;
-  g_bisect_stats[3] = bnd[0]; g_bisect_stats[4] = bnd[1]; g_bisect_stats[5] = 0; g_bisect_stats[6] = 0; g_bisect_stats[7] = 0;
 }
 
-// method: CPB_SPLIT_FLIP_BISECT_COST, CPB_SPLIT_LAZY_FLIP_BISECT_COST or CPB_SPLIT_FLIP_BISECT_INDEX
-void solve_flip(Oracle& f, int method, double eps, i64 K, int64_t* h_spl_out) {
+// The checks of a Flip solve (method: CPB_SPLIT_FLIP_BISECT_COST, CPB_SPLIT_LAZY_FLIP_BISECT_COST or CPB_SPLIT_FLIP_BISECT_INDEX).
+static void flip_prepare(Oracle& f, i64 K, double bnd[2]) {
   CPB_REQUIRE(K >= 1, "K must be >= 1");
   CPB_REQUIRE(f.dev.kind == CPB_MODEL_SECCONN || f.dev.kind == CPB_MODEL_SECEDGE, "the Flip splitters on the device serve the (decreasing) secondary models");
   if (f.dev.kind == CPB_MODEL_SECCONN)
@@ -1709,22 +1720,132 @@ void solve_flip(Oracle& f, int method, double eps, i64 K, int64_t* h_spl_out) {
   CPB_REQUIRE(A.n + 1 < ((i64)1 << 31) && K + 2 < ((i64)1 << 30), "problem too large for 32-bit split points");
   CPB_REQUIRE(K == f.pi_K, "the secondary model's row partition must have K parts");
   oracle_ensure_ranks(f);
-  double bnd[2];
   oracle_bound(f, K, bnd);
-  ProfScope prof("probe");
-  DBuf<int> spl(K + 2), spl_lo(K + 2), spl_hi(K + 2), probes(1);
-  const bool lazy = method == CPB_SPLIT_LAZY_FLIP_BISECT_COST;
-  if (method == CPB_SPLIT_FLIP_BISECT_INDEX) {
-    if (f.dev.is_float) CPB_LAUNCH(k_flip_bisect_index<double>, BS_CLUSTER, BS_THREADS, 0, f.dev, (int)K, bnd[0], bnd[1], spl.get(), spl_lo.get(), spl_hi.get(), probes.get());
-    else CPB_LAUNCH(k_flip_bisect_index<i64>, BS_CLUSTER, BS_THREADS, 0, f.dev, (int)K, bnd[0], bnd[1], spl.get(), spl_lo.get(), spl_hi.get(), probes.get());
-  } else {
-    if (f.dev.is_float) CPB_LAUNCH(k_flip_bisect<double>, BS_CLUSTER, BS_THREADS, 0, f.dev, (int)K, 1 + eps, bnd[0], bnd[1], lazy ? 1 : 0, spl.get(), spl_lo.get(), spl_hi.get(), probes.get());
-    else CPB_LAUNCH(k_flip_bisect<i64>, BS_CLUSTER, BS_THREADS, 0, f.dev, (int)K, 1 + eps, bnd[0], bnd[1], lazy ? 1 : 0, spl.get(), spl_lo.get(), spl_hi.get(), probes.get());
+}
+
+// One problem of k_stripe_batch, checked exactly as the single solvers check it (their messages).
+static StripeJob prepare_job(Oracle& f, int method, const double* eps, i64 K) {
+  if (method != CPB_SPLIT_BISECT_INDEX && method != CPB_SPLIT_FLIP_BISECT_COST && method != CPB_SPLIT_LAZY_FLIP_BISECT_COST && method != CPB_SPLIT_FLIP_BISECT_INDEX)
+    throw Error(CPB_ERR_UNSUPPORTED, "a batch takes the BisectIndex and Flip splitters only");
+  const bool cost = method == CPB_SPLIT_FLIP_BISECT_COST || method == CPB_SPLIT_LAZY_FLIP_BISECT_COST;
+  CPB_REQUIRE(eps || !cost, "eps is NULL but a FlipBisectCost method needs it");
+  double bnd[2];
+  if (method == CPB_SPLIT_BISECT_INDEX) bisect_index_prepare(f, K, bnd);
+  else flip_prepare(f, K, bnd);
+  StripeJob jb{};
+  jb.method = method;
+  jb.K = (int)K;
+  jb.lazy = method == CPB_SPLIT_LAZY_FLIP_BISECT_COST;
+  jb.c_lo = bnd[0];
+  jb.c_hi = bnd[1];
+  jb.eps1 = cost ? 1 + *eps : 1.0;
+  return jb;
+}
+
+// Launches checked jobs (one launch per cost type) and copies the split vectors out.  The workspace holds, per problem, the
+// vector the solve returns (spl_hi for BisectIndex and LazyFlipBisectCost, spl_lo for FlipBisectCost and FlipBisectIndex, as
+// in the reference) in one contiguous region, read back with one copy, and its two other vectors behind it.  The vectors
+// are 1-based: slot 0 of the returned one carries the problem's probe count.
+static void run_jobs(i64 B, Oracle* const* f, std::vector<StripeJob>& jobs, int64_t* const* h_spl_out, int* h_probes) {
+  std::vector<const Oracle*> distinct;
+  std::vector<i64> res_off(B);
+  i64 res_total = 0;
+  for (i64 b = 0; b < B; ++b) {
+    const auto it = std::find(distinct.begin(), distinct.end(), f[b]);
+    jobs[b].oracle = (int)(it - distinct.begin());
+    if (it == distinct.end()) distinct.push_back(f[b]);
+    res_off[b] = res_total;
+    res_total += jobs[b].K + 2;
   }
-  std::vector<int> h(K + 2);
-  CPB_CUDA(cudaMemcpyAsync(h.data(), (lazy ? spl_hi : spl_lo).get(), (K + 2) * sizeof(int), cudaMemcpyDeviceToHost, ctx().stream));
+  // Int64 problems first, then Float64
+  std::vector<StripeJob> sorted;
+  i64 other = res_total, n_int = 0;
+  for (int is_float = 0; is_float < 2; ++is_float)
+    for (i64 b = 0; b < B; ++b) {
+      if (f[b]->dev.is_float != is_float) continue;
+      StripeJob jb = jobs[b];
+      const i64 n = jb.K + 2;
+      const bool keep_hi = jb.method == CPB_SPLIT_BISECT_INDEX || jb.lazy;
+      jb.spl = other;
+      (keep_hi ? jb.spl_lo : jb.spl_hi) = other + n;
+      (keep_hi ? jb.spl_hi : jb.spl_lo) = res_off[b];
+      jb.probes = res_off[b];
+      other += 2 * n;
+      sorted.push_back(jb);
+      n_int += !is_float;
+    }
+  const size_t oracle_bytes = distinct.size() * sizeof(DevOracle);
+  std::vector<char> table(oracle_bytes + B * sizeof(StripeJob));
+  for (size_t i = 0; i < distinct.size(); ++i) std::memcpy(table.data() + i * sizeof(DevOracle), &distinct[i]->dev, sizeof(DevOracle));
+  std::memcpy(table.data() + oracle_bytes, sorted.data(), B * sizeof(StripeJob));
+  ProfScope prof("probe");
+  DBuf<char> d_table(table.size());
+  DBuf<int> ws((size_t)other);
+  CPB_CUDA(cudaMemcpyAsync(d_table.get(), table.data(), table.size(), cudaMemcpyHostToDevice, ctx().stream));
+  const DevOracle* d_or = reinterpret_cast<const DevOracle*>(d_table.get());
+  const StripeJob* d_jobs = reinterpret_cast<const StripeJob*>(d_table.get() + oracle_bytes);
+  if (n_int > 0) CPB_LAUNCH(k_stripe_batch<i64>, (unsigned)(n_int * BS_CLUSTER), BS_THREADS, 0, d_or, d_jobs, ws.get());
+  if (B > n_int) CPB_LAUNCH(k_stripe_batch<double>, (unsigned)((B - n_int) * BS_CLUSTER), BS_THREADS, 0, d_or, d_jobs + n_int, ws.get());
+  std::vector<int> h(res_total);
+  CPB_CUDA(cudaMemcpyAsync(h.data(), ws.get(), res_total * sizeof(int), cudaMemcpyDeviceToHost, ctx().stream));
   CPB_CUDA(cudaStreamSynchronize(ctx().stream));
-  for (i64 k = 1; k <= K + 1; ++k) h_spl_out[k - 1] = h[k];
+  for (i64 b = 0; b < B; ++b) {
+    const int* r = h.data() + res_off[b];
+    for (i64 k = 1; k <= jobs[b].K + 1; ++k) h_spl_out[b][k - 1] = r[k];
+    if (h_probes) h_probes[b] = r[0];
+  }
+}
+
+// The single solves are batches of one: the batch kernel reads the oracle into shared memory, which measured faster than
+// the kernel-parameter oracle of a one-problem kernel (DESIGN section 4).
+void solve_bisect_index(Oracle& f, i64 K, int64_t* h_spl_out) {
+  std::vector<StripeJob> jobs{prepare_job(f, CPB_SPLIT_BISECT_INDEX, nullptr, K)};
+  Oracle* fp = &f;
+  int hp = 0;
+  run_jobs(1, &fp, jobs, &h_spl_out, &hp);
+  g_bisect_stats[0] = 1; g_bisect_stats[1] = hp; g_bisect_stats[2] = hp;
+  g_bisect_stats[3] = jobs[0].c_lo; g_bisect_stats[4] = jobs[0].c_hi; g_bisect_stats[5] = 0; g_bisect_stats[6] = 0; g_bisect_stats[7] = 0;
+}
+
+// method: CPB_SPLIT_FLIP_BISECT_COST, CPB_SPLIT_LAZY_FLIP_BISECT_COST or CPB_SPLIT_FLIP_BISECT_INDEX
+void solve_flip(Oracle& f, int method, double eps, i64 K, int64_t* h_spl_out) {
+  std::vector<StripeJob> jobs{prepare_job(f, method, &eps, K)};
+  Oracle* fp = &f;
+  run_jobs(1, &fp, jobs, &h_spl_out, nullptr);
+}
+
+// Every problem is checked first -- a failure names the problem, and nothing is launched or written.  cpb_bisect_stats is
+// not updated.
+void solve_stripe_batch(i64 B, Oracle* const* f, const int* method, const double* eps, const i64* K, int64_t* const* h_spl_out) {
+  if (B <= 0) return;
+  std::vector<StripeJob> jobs(B);
+  for (i64 b = 0; b < B; ++b) {
+    try {
+      CPB_REQUIRE(f[b] && h_spl_out[b], "NULL argument");
+      jobs[b] = prepare_job(*f[b], method[b], eps ? eps + b : nullptr, K[b]);
+    } catch (const Error& e) {
+      throw Error(e.code, "problem " + std::to_string(b) + ": " + e.what());
+    }
+  }
+  run_jobs(B, f, jobs, h_spl_out, nullptr);
+}
+
+// how many stripe_batch clusters the device keeps resident at once
+int stripe_batch_capacity() {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(BS_CLUSTER * 1024, 1, 1);
+  cfg.blockDim = dim3(BS_THREADS, 1, 1);
+  cfg.dynamicSmemBytes = 0;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = BS_CLUSTER;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  int n = 0;
+  CPB_CUDA(cudaOccupancyMaxActiveClusters(&n, k_stripe_batch<i64>, &cfg));
+  return n;
 }
 
 void solve_bisect(Oracle& f, bool lazy, double eps, i64 K, int64_t* h_spl_out) {

@@ -619,6 +619,31 @@ int cpb_partition_stripe(cpb_oracle* f, int method, const cpb_constraint* con, d
   CPB_API_END
 }
 
+int cpb_partition_stripe_batch(int64_t B, cpb_oracle* const* f, const int* method, const double* eps, const int64_t* K, int64_t* const* spl_out) {
+  CPB_API_BEGIN
+  CPB_REQUIRE(B >= 0, "B must be >= 0");
+  if (B == 0) return CPB_OK;
+  ensure_context();
+  CPB_REQUIRE(f && method && K && spl_out, "NULL argument");
+  std::vector<Oracle*> O(B);
+  for (int64_t b = 0; b < B; ++b) {
+    if (!f[b]) throw Error(CPB_ERR_ARG, "problem " + std::to_string(b) + ": NULL argument");
+    O[b] = f[b]->O.get();
+  }
+  trace_mark("enter");
+  struct TraceEnd { ~TraceEnd() { trace_mark("exit"); trace_flush("partition_stripe_batch"); } } trace_end;
+  solve_stripe_batch(B, O.data(), method, eps, (const i64*)K, spl_out);
+  CPB_API_END
+}
+
+int cpb_partition_stripe_batch_capacity(int* clusters_out) {
+  CPB_API_BEGIN
+  ensure_context();
+  CPB_REQUIRE(clusters_out, "NULL argument");
+  *clusters_out = stripe_batch_capacity();
+  CPB_API_END
+}
+
 int cpb_partition_stripe_weighted(cpb_oracle* f, int method, cpb_oracle* w, int64_t w_max, double eps, int64_t K, int64_t* spl_out) {
   CPB_API_BEGIN
   ensure_context();

@@ -106,6 +106,10 @@ struct Oracle {
   std::unique_ptr<LinkStream> ls;  // links for the streaming probes (net or dia-net, by model)
   DBuf<u32> overpos;
   i64 h_n_over = -1;  // host copy of overpos[n] once it has been read
+  // ocl(1, n+1) once bound_stripe has queried it (connectivity, envelope; nets(1, n+1) for primary connectivity): the matrix
+  // never changes, and a batch of many K on one oracle asks for it once instead of once per problem
+  bool has_whole = false;
+  double h_whole = 0;
   DBuf<i64> env;
   int envH = 0;
   DBuf<double> tab_f;  // alpha_col | beta_col (double)
@@ -132,6 +136,9 @@ void solve_bisect(Oracle& f, bool lazy, double eps, i64 K, int64_t* h_spl_out);
 void solve_bisect_index(Oracle& f, i64 K, int64_t* h_spl_out);
 void solve_flip(Oracle& f, int method, double eps, i64 K, int64_t* h_spl_out);
 int probe_cluster_capacity(bool stream);
+// B problems of BisectIndex / the Flip splitters in one launch per cost type (eps may be nullptr without a FlipBisectCost problem)
+void solve_stripe_batch(i64 B, Oracle* const* f, const int* method, const double* eps, const i64* K, int64_t* const* h_spl_out);
+int stripe_batch_capacity();  // clusters of the batch kernel the device keeps resident at once
 // one bisection as steps (bisect.cu); the run owns its node buffers
 struct BisectRun;
 struct BisectRunDelete { void operator()(BisectRun* run) const; };

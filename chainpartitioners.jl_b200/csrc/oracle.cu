@@ -282,6 +282,14 @@ static double query_one(Oracle& f, i64 j, i64 jp) {
   return r;
 }
 
+static double query_whole(Oracle& f) {
+  if (!f.has_whole) {
+    f.h_whole = query_one(f, 1, f.A->n + 1);
+    f.has_whole = true;
+  }
+  return f.h_whole;
+}
+
 // bound_stripe: WorkCosts.jl:37-51, ConnectivityCosts.jl:25-35, Monotonized...:94-105, EnvelopeCosts.jl:44-54
 template <class T> static void bound_T(Oracle& f, i64 K, double out[2]) {
   const Matrix& A = *f.A;
@@ -300,7 +308,7 @@ template <class T> static void bound_T(Oracle& f, i64 K, double out[2]) {
     case CPB_MODEL_CONNECTIVITY: {
       CPB_REQUIRE(c[1] >= 0 && c[2] >= 0 && c[3] >= 0, "negative beta (ConnectivityCosts.jl:29-31)");
       if (f.ranks_built) {
-        c_hi = (T)query_one(f, 1, A.n + 1);
+        c_hi = (T)query_whole(f);
       } else {  // ocl(1, n+1) from the link array alone: nets(1, n+1) = number of non-empty rows
         if (!f.ls) f.ls = build_link_stream(*f.A, false, false, false, /*as_pos=*/true);
         if (f.ls->h_first_count < 0) f.ls->h_first_count = count_first_occurrences(*f.ls);
@@ -357,7 +365,7 @@ template <class T> static void bound_T(Oracle& f, i64 K, double out[2]) {
       f.dev.kind = CPB_MODEL_CONNECTIVITY;
       f.dev.cf[0] = f.dev.cf[1] = f.dev.cf[2] = 0; f.dev.cf[3] = 1;
       f.dev.ci[0] = f.dev.ci[1] = f.dev.ci[2] = 0; f.dev.ci[3] = 1;
-      const double nets_all = query_one(f, 1, A.n + 1);
+      const double nets_all = query_whole(f);
       f.dev = saved;
       (void)conn;
       c_hi = c[0] + c[1] * (T)A.n + c[2] * (T)A.N + std::max(c[3], c[4]) * (T)nets_all;
@@ -381,7 +389,7 @@ template <class T> static void bound_T(Oracle& f, i64 K, double out[2]) {
       // the oracle form (EnvelopeCosts.jl:30-42), the one partition_stripe(Bisect*) reaches: c_hi = ocl(1, n + 1) with the
       // oracle's own left-to-right sum, c_lo = alpha + fld(c_hi - alpha, K); an empty pattern is fine (envelope width 0)
       CPB_REQUIRE(c[1] >= 0 && c[2] >= 0 && c[3] >= 0, "negative beta (EnvelopeCosts.jl:34-36)");
-      c_hi = (T)query_one(f, 1, A.n + 1);
+      c_hi = (T)query_whole(f);
       c_lo = c[0] + jl_fld(c_hi - c[0], (T)K);
       break;
     }

@@ -282,6 +282,29 @@ function partition_stripe(dA::DeviceMatrix, K, method::OnB200, args...; kwargs..
     return stripe_solve(dA, K, code, ϵ, method.mtd.f, args...)
 end
 
+# Many BisectIndex / Flip problems in one launch, one cluster each (cpb_partition_stripe_batch): problems is a vector of
+# (A, K, OnB200(method)) or (A, K, OnB200(method), Π); each result is identical to partition_stripe(A, K, OnB200(method)[, Π]).
+# Problems with the same A, model and Π objects share one oracle (a sweep over K builds it once); a host matrix is uploaded once.
+function partition_stripe_batch(problems)
+    mats = IdDict{Any, DeviceMatrix}()
+    ocls = Dict{Tuple{UInt, UInt, UInt}, DeviceOracle}()
+    hs, codes, epss, Ks, outs = Ptr{Cvoid}[], Cint[], Float64[], Int64[], Vector{Int64}[]
+    for p in problems
+        A, K, method = p[1], Int64(p[2]), p[3]
+        Π = length(p) >= 4 ? p[4] : nothing
+        (code, ϵ) = split_code(method.mtd)
+        code in (12, 6, 7, 13) || throw(ArgumentError("partition_stripe_batch takes the BisectIndex and Flip splitters only"))
+        dA = get!(() -> device_matrix(A), mats, A)
+        ocl = get!(() -> DeviceOracle(dA, method.mtd.f, Π), ocls, (objectid(A), objectid(method.mtd.f), objectid(Π)))
+        push!(hs, ocl.h); push!(codes, code); push!(epss, ϵ); push!(Ks, K); push!(outs, Vector{Int64}(undef, K + 1))
+    end
+    ptrs = [pointer(o) for o in outs]
+    GC.@preserve mats ocls outs check(ccall((:cpb_partition_stripe_batch, lib), Cint,
+                                            (Int64, Ptr{Ptr{Cvoid}}, Ptr{Cint}, Ptr{Float64}, Ptr{Int64}, Ptr{Ptr{Int64}}),
+                                            length(hs), hs, codes, epss, Ks, ptrs))
+    return [SplitPartition{Int64}(K, o) for (K, o) in zip(Ks, outs)]
+end
+
 # partition_plaid(A, K, AlternatingPartitioner(OnB200(m1), OnB200(m2), ...)) (src/AlternatingPartitioner.jl:18-32): A is
 # uploaded ONCE, adjointpattern runs on the device, every stripe solve takes the resident handles -- the reference's
 # `adj_A = adjointpattern(A)` reuse seam, kept on the device.  A caller-supplied adj_A (host or device) is honoured.

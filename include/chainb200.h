@@ -193,6 +193,16 @@ enum {
 };
 /* -> spl_out[K+1] (SplitPartition{Int64}(K, spl), Partitions.jl:3-6); con may be NULL. */
 int cpb_partition_stripe(cpb_oracle* f, int method, const cpb_constraint* con, double eps, int64_t K, int64_t* spl_out);
+/* B independent partition_stripe problems in one launch, one cluster each.  Every result is identical to
+ * cpb_partition_stripe(f[b], method[b], NULL, eps[b], K[b], spl_out[b]).  Methods: CPB_SPLIT_BISECT_INDEX,
+ * CPB_SPLIT_FLIP_BISECT_COST, CPB_SPLIT_LAZY_FLIP_BISECT_COST, CPB_SPLIT_FLIP_BISECT_INDEX (else CPB_ERR_UNSUPPORTED).
+ * Oracles may repeat and may belong to different matrices of this device; eps may be NULL when no Flip-cost method is
+ * present; spl_out[b] holds K[b] + 1 entries.  Any invalid problem fails the whole call before any launch (the message
+ * names the problem) and no spl_out is written.  B = 0 returns CPB_OK; a batch does not update cpb_bisect_stats. */
+int cpb_partition_stripe_batch(int64_t B, cpb_oracle* const* f, const int* method, const double* eps, const int64_t* K,
+                               int64_t* const* spl_out);
+/* Clusters of the batch kernel the device keeps resident at once (cudaOccupancyMaxActiveClusters): larger batches queue. */
+int cpb_partition_stripe_batch_capacity(int* clusters_out);
 
 /* partition_stripe(A, K, method(ConstrainedCost(f, w, w_max))) with the weight given as a cost model of its own
  * (Costs.jl:105-147: the reference turns w into an oracle and tests w(j, j') > w_max for the windows of every constrained
